@@ -23,6 +23,11 @@ section 8d) of every EMAT of the forest; K steps are enqueued back to back betwe
 `--impl reference` times the reference's CPU implementation (oracle/_ref) on the same workload and prints the same keys; it
 loads no product code (inputs come from libdphy_synth.so).
 
+`--dump-outputs DIR` writes, after the timed steps, what the timed evaluation and SPR batch computed in their last step (log G
+terms and lambda_i of every chain, the batch's study summaries and regions; float64, a fixed seeded sample of any array larger
+than DUMP_MAX_ELEMS) as DIR/<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
+
 Multi-GPU (torchrun): the headline shards independent EMATs over ranks with no data-path collective (weak scaling); the
 `partitioned` section is the one place with a real exchange.
 """
@@ -70,7 +75,34 @@ def parse_args():
     ap.add_argument("--mcmc-tips", type=int, default=10000, help="tips of the second MCMC alignment (config 3 shape)")
     ap.add_argument("--mcmc-steps", type=int, default=200000)
     ap.add_argument("--mcmc-threads-per-gpu", type=int, default=1)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed log-G and SPR steps computed in their last step to DIR/<name>.npy (float64, rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+DUMP_MAX_ELEMS = 1 << 19      # per array: a fixed, seeded sample beyond this keeps a dump of ~30 MB at the default workload (<= 64 MB)
+
+
+def dump_sample(a):
+    """`a` as float64, or a fixed seeded sample of DUMP_MAX_ELEMS of its elements (in order) when it is larger."""
+    a = np.asarray(a, np.float64).ravel()
+    if a.size <= DUMP_MAX_ELEMS:
+        return a
+    idx = np.sort(np.random.default_rng(20251017).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+    return a[idx]
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"output dump of {total} bytes exceeds 64 MB"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def config_block(args):
@@ -447,8 +479,10 @@ def main():
         forest.eval_log_G()
         spr_reqs = db.spr_requests_for_attached(emats[0], 0, spr_xs, forest.lambda_i(0), infos[0]["t_max_tip"])
 
-    def spr_batch():
+    def spr_batch(keep=False):
         b = forest.spr_study_batch(spr_reqs)
+        if keep:
+            return b
         b.close()                    # stream-ordered free: the memory is reused by the next batch
 
     for _ in range(max(args.warmup, 3)):
@@ -463,7 +497,12 @@ def main():
     launches0 = ctx.launches
     logg_ms, host_enqueue_ms = time_evals(forest, args.steps, R)
     launches = ctx.launches - launches0
-    _, _, lg = forest.log_G()        # checksum of the timed work: log G of every chain
+    rp, br, lg = forest.log_G()      # checksum of the timed work: log G of every chain
+    dumped = {}
+    if args.dump_outputs:
+        # what a caller of the timed evaluation reads back: per chain the three log-G terms and lambda_i of every node
+        dumped.update(log_root_prior=rp, log_G_below_root=br, log_G=lg,
+                      lambda_i=dump_sample(np.concatenate([forest.lambda_i(k) for k in range(args.chains)])))
 
     spr_ms, spr_regions, spr_launches = None, 0, 0
     if spr_reqs is not None:
@@ -472,13 +511,23 @@ def main():
         a, b = ev(), ev()
         barrier()
         a.record(stream)
-        for _ in range(args.steps * SB):
-            spr_batch()
+        n_batches = args.steps * SB
+        for i in range(n_batches):
+            last = spr_batch(keep=bool(args.dump_outputs) and i == n_batches - 1)      # --dump-outputs reads the last timed batch back
         ctx.join_side_streams()       # the last batches' normalisation passes run on the library's tail stream: inside the timed region
         b.record(stream)
         barrier()
         spr_ms = a.elapsed_time(b) / (args.steps * SB)        # per batch
         spr_launches = ctx.launches - l0
+        if args.dump_outputs:
+            sm = last.summaries()
+            for k in ("mu", "log_Wmax", "sum_W_over_Wmax", "num_regions"):
+                dumped["spr_summary_" + k] = np.array([getattr(s, k) for s in sm], np.float64)
+            regs = last.regions()
+            for k in ("branch", "mut_idx", "min_muts", "t_min", "t_max", "log_W_over_Wmax", "W_over_Wmax"):
+                dumped["spr_region_" + k] = dump_sample(regs[k])
+            del regs
+            last.close()
         bt = forest.spr_study_batch(spr_reqs)
         spr_regions = bt.total_regions()
         bt.close()
@@ -489,6 +538,8 @@ def main():
         forest.eval_log_G()
     gen_ms, _ = time_evals(forest, args.steps, R)
     _, _, lg_gen = forest.log_G()
+    if args.dump_outputs:
+        dumped["log_G_general_schedule"] = lg_gen
     ctx.set_log_G_path("auto")
     assert np.allclose(lg_gen, lg, rtol=1e-11), "folded and general log-G schedules disagree"
     clocks = sampler.stop() if rank == 0 else None
@@ -785,6 +836,8 @@ def main():
         if world > 1:
             dist.barrier()
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dumped)
         emit_line(line)
     if world > 1:
         dist.destroy_process_group()

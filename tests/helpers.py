@@ -1,6 +1,7 @@
 """Shared helpers for the parity tests: synthetic EMATs (product-side generator) -> oracle structs."""
 from __future__ import annotations
 
+import copy
 import functools
 
 import numpy as np
@@ -27,9 +28,15 @@ def from_oracle(e: Emat, s: Sites):
 
 
 @functools.lru_cache(maxsize=32)
-def synth(config=0, **overrides):
+def _synth_cached(config=0, **overrides):
     p = db.synth_params(config, **overrides)
     return db.synth_generate(p)
+
+
+def synth(config=0, **overrides):
+    """(HostEmat, HostSites, info) of a synthetic shape.  Generated once, but every call gets its own copy: tests edit
+    trees and models in place, and must not change what a later test in the same process is given."""
+    return copy.deepcopy(_synth_cached(config, **overrides))
 
 
 def rel_err(a, b):
