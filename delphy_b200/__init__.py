@@ -75,6 +75,18 @@ class SprRequest(C.Structure):
     ]
 
 
+class SampleSet(C.Structure):
+    _fields_ = [("num_samples", C.c_int32), ("reserved", C.c_int32), ("delta_off", i32p), ("delta_site", i32p), ("delta_to", u8p),
+                ("miss_off", i32p), ("miss_start", i32p), ("miss_end", i32p)]
+
+
+class Placement(C.Structure):
+    _fields_ = [("min_muts", C.c_int32), ("num_best", C.c_int32), ("branch", C.c_int32), ("mut_idx", C.c_int32)]
+
+
+PLACEMENT_DTYPE = np.dtype([("min_muts", "<i4"), ("num_best", "<i4"), ("branch", "<i4"), ("mut_idx", "<i4")])
+
+
 class SprWeightParams(C.Structure):
     _fields_ = [("lambda_X", C.c_double), ("annealing_factor", C.c_double), ("t_max_tip", C.c_double)]
 
@@ -312,6 +324,8 @@ def lib() -> C.CDLL:
     L.dphy_forest_write_api_tree.argtypes = [vp, vp, C.c_int32, vp, C.c_size_t]; L.dphy_forest_write_api_tree.restype = C.c_int64
     L.dphy_forest_tree_counts.argtypes = [vp, vp, C.c_int32, C.POINTER(TreeCounts)]
     L.dphy_forest_download_tree.argtypes = [vp, vp, C.c_int32, C.POINTER(EmatHost)]
+    L.dphy_forest_place_samples.argtypes = [vp, vp, C.c_int32, C.POINTER(SampleSet), C.c_int32, C.c_int32, C.POINTER(Placement),
+                                            C.POINTER(CandidateRegion)]
     L.dphy_maple_parse.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(vp)]
     L.dphy_maple_get.argtypes = [vp, C.POINTER(MapleView)]
     L.dphy_maple_free.argtypes = [vp]; L.dphy_maple_free.restype = None
@@ -826,6 +840,27 @@ class Forest:
         nm = np.zeros((self.num_trees, ld), np.int32)
         self.ctx.check(lib().dphy_forest_calc_site_tallies(self.ctx._h, self._h, ld, _p(tw, f64p), _p(nm, i32p)))
         return tw, nm
+
+    # -- placement of new samples
+    def place_samples(self, samples, tree=0, can_change_root=True, max_best=0):
+        """dphy_forest_place_samples: maximum-parsimony placement of new sequences on tree `tree`.  `samples` is the dict maple_parse
+        returns, or any dict with its six arrays (delta_off / delta_site / delta_to, miss_off / miss_start / miss_end).  Returns a dict of
+        numpy arrays: min_muts, num_best, branch, mut_idx (one entry per sample) and best, a [S, max_best] REGION_DTYPE array of the
+        first max_best best regions in the study's emission order (unused slots: branch == -1)."""
+        a = dict(delta_off=np.ascontiguousarray(samples["delta_off"], np.int32), delta_site=np.ascontiguousarray(samples["delta_site"], np.int32),
+                 delta_to=np.ascontiguousarray(samples["delta_to"], np.uint8), miss_off=np.ascontiguousarray(samples["miss_off"], np.int32),
+                 miss_start=np.ascontiguousarray(samples["miss_start"], np.int32), miss_end=np.ascontiguousarray(samples["miss_end"], np.int32))
+        S = len(a["delta_off"]) - 1
+        if S < 0 or len(a["miss_off"]) != S + 1:
+            raise ValueError("place_samples: delta_off and miss_off must both have num_samples + 1 entries")
+        ss = SampleSet(S, 0, _p(a["delta_off"], i32p), _p(a["delta_site"], i32p), _p(a["delta_to"], u8p), _p(a["miss_off"], i32p),
+                       _p(a["miss_start"], i32p), _p(a["miss_end"], i32p))
+        out = np.zeros(max(S, 1), PLACEMENT_DTYPE)
+        best = np.zeros((max(S, 1), max_best), REGION_DTYPE)
+        self.ctx.check(lib().dphy_forest_place_samples(self.ctx._h, self._h, tree, C.byref(ss), int(bool(can_change_root)), max_best,
+                                                       _p(out, C.POINTER(Placement)), _p(best, C.POINTER(CandidateRegion)) if max_best > 0 else None))
+        return dict(min_muts=out["min_muts"][:S].copy(), num_best=out["num_best"][:S].copy(), branch=out["branch"][:S].copy(),
+                    mut_idx=out["mut_idx"][:S].copy(), best=best[:S])
 
     # -- SPR studies
     def spr_study_batch(self, requests):

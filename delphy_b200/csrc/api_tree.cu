@@ -383,6 +383,14 @@ int api_status_to_error(dphy_ctx* ctx, uint32_t bits) {
 }
 
 }  // namespace
+
+int launch_scan_i32(dphy_ctx* ctx, int32_t* v, int n, int32_t* tile_tot) {
+  const int nt = (n + kScanTile - 1) / kScanTile;
+  apitree_scan_tiles_kernel<<<nt, 1024, 0, ctx->stream>>>(v, n, tile_tot);
+  apitree_scan_fix_kernel<<<nt, 1024, 0, ctx->stream>>>(v, n, tile_tot);
+  ctx->launches += 2;
+  return check_cuda(ctx, cudaGetLastError(), "scan launch");
+}
 }  // namespace dphy
 
 using namespace dphy;

@@ -177,6 +177,16 @@ struct FlattenParams {
   const int32_t* old_parent_pos = nullptr;
 };
 
+// Per-tree index of dphy_forest_place_samples (kernels_place.cu), built by the first placement on the tree.
+struct PlaceIndex {
+  int32_t R = 0, P2 = 0, L = 0, pad = 0;   // regions of the unbounded study from the root; leaves of the segment tree (power of 2)
+  int32_t* site_off = nullptr;             // [L + 1] first record of every site
+  int4* rec = nullptr;                     // [M] per mutation, by site: (first region below it, end of those regions, from << 2 | to, dref)
+  int2* seg = nullptr;                     // [2 P2] (min, count) segment tree over Hr, leaves at P2 + region
+  size_t bytes = 0;                        // resident bytes
+  std::vector<int32_t> h_site_off;         // host copy of site_off (scratch bounds per sample)
+};
+
 }  // namespace dphy
 
 struct dphy_ctx {
@@ -272,6 +282,7 @@ struct dphy_forest {
   const int32_t* d_ctile_order = nullptr;   // [num_ctiles] launch order of the general log-G tile kernel (full tiles first)
   // study-independent tables of the event-scan SPR path (kernels_spr_group2.cuh), built by the first grouped batch on this forest
   int32_t* d_spr_eopen = nullptr; int32_t* d_spr_tnode = nullptr; int32_t* d_spr_ev = nullptr;
+  std::vector<dphy::PlaceIndex> place;   // per tree: the placement index (kernels_place.cu), empty until the first placement
   bool evaluated = false;
   bool struct_valid = false;    // nsmn / num_muts tallies (structure-only outputs of the general log-G pass) are current
   uint32_t epoch = 0;           // look-back flag value of the current launch (flag == epoch means "published")
@@ -312,6 +323,8 @@ int launch_flatten(dphy_ctx* ctx, const FlattenParams& P, int num_tiles, int max
 // stage 2 split per tree (direct uploads: each tree's lists are gathered as soon as its own arrays have landed)
 int launch_flatten_lists(dphy_ctx* ctx, FlattenParams P, int first_tile, int num_tiles);
 int launch_flatten_ctiles(dphy_ctx* ctx, const FlattenParams& P);
+// exclusive scan of n int32 in place (api_tree.cu); tile_tot holds (n + 8191) / 8192 ints
+int launch_scan_i32(dphy_ctx* ctx, int32_t* v, int n, int32_t* tile_tot);
 // many device-to-device array copies in one launch (16-byte aligned sources and destinations)
 struct DeviceCopyJob { char* dst; const char* src; size_t bytes; };
 int launch_device_copies(dphy_ctx* ctx, const DeviceCopyJob* d_jobs, int num_jobs, size_t max_bytes);

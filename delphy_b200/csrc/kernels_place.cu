@@ -1,0 +1,497 @@
+// kernels_place.cu -- batched maximum-parsimony placement of new samples on a device-resident tree (sm_100a).
+//
+// The question build_usher_like_tree asks per tip (core/phylo_tree.cpp:918-932) and UShER-style placement asks per new sequence:
+// over the regions of an unbounded study of the sample from the root (Spr_study_builder::seed_fill_from with X == k_no_node,
+// t_X == DBL_MAX, core/spr_study.cpp:9-128), the least min_muts, how many regions attain it and which is first in emission order --
+// without materialising the ~N + M regions of the study or an O(L) table of the sample.
+//
+// Regions are numbered in emission order: the root region (root, n_root) is 0, then every non-root node v in device order (the
+// builder's LIFO order, children[1] first) contributes (v, 0..n_v) at base(v) = (v - root) + mut_off[v] - mut_off[root + 1].  The
+// regions below v are the block [base(v), end(v)), end(v) = base(v + subtree_size(v)), and the k-th mutation of v lies above
+// [base(v) + k + 1, end(v)); the root's own list lies above every region.  With the Hamming-potential restatement (SURVEY.md
+// section 8a, a12), for a sample with deltas D from the reference and missing set Mx:
+//   min_muts(r) = B + Hr[r] + sum over m in A above r of c(m)
+//   Hr[r] = sum of dref(m) over the mutations above r,    dref(m) = [to != ref_l] - [from != ref_l]
+//   B = #{l in D \ Mx : x_l != ref_l},  A = mutations at sites in D u Mx,  c(m) = dx(m) - dref(m), dx(m) = 0 on Mx
+// (true when every mutation's `from` is the state above it, which the builder's delta arithmetic assumes as well).
+// Hr is study-independent: it lives in a min / count segment tree next to a site-sorted table of the mutations' region ranges (the
+// per-tree index, built once per forest).  A sample's correction is piecewise constant between the 2|A| range endpoints: sort them,
+// sweep, and ask the segment tree for (min, count) per piece -- O(|A| log R) per sample instead of O(R + L).
+#include "dphy_internal.h"
+#include "device_utils.cuh"
+
+#include <algorithm>
+#include <cfloat>
+#include <climits>
+#include <cstring>
+#include <new>
+#include <vector>
+
+namespace dphy {
+
+// ---- per-tree index --------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ int region_base(const ForestDev& f, int nb, int p) { return (p - nb) + f.mut_off[p] - f.mut_off[nb + 1]; }
+
+__global__ void place_site_hist_kernel(ForestDev f, int m0, int M, int32_t* __restrict__ site_off) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < M) atomicAdd(site_off + f.mut_site[m0 + i], 1);
+}
+
+// one thread per mutation: its node (binary search on the CSR offsets), its region range, its reference potential; scattered into
+// its site's run of the table and added to the difference array of Hr
+__global__ void place_site_scatter_kernel(ForestDev f, int nb, int N, int R, int m0, int M, const uint8_t* __restrict__ ref,
+                                          const int32_t* __restrict__ site_off, int32_t* __restrict__ fill, int4* __restrict__ rec,
+                                          int32_t* __restrict__ diff) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= M) return;
+  const int g = m0 + i;
+  int lo = nb, hi = nb + N - 1;                     // last node whose list starts at or before g
+  while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (f.mut_off[mid] <= g) lo = mid; else hi = mid - 1; }
+  const int p = lo;
+  int a = 0, b = R;
+  if (p != nb) { a = region_base(f, nb, p) + (g - f.mut_off[p]) + 1; b = region_base(f, nb, p + f.subtree_size[p]); }
+  const int site = f.mut_site[g], code = f.mut_code[g], from = (code >> 2) & 3, to = code & 3, rl = ref[site];
+  const int dref = (int)(to != rl) - (int)(from != rl);
+  const int slot = site_off[site] + atomicAdd(fill + site, 1);
+  rec[slot] = make_int4(a, b, (from << 2) | to, dref);
+  if (dref) { atomicAdd(diff + a, dref); atomicAdd(diff + b, -dref); }
+}
+
+__device__ __forceinline__ int2 seg_comb(int2 a, int2 b) {
+  const int m = min(a.x, b.x);
+  return make_int2(m, (a.x == m ? a.y : 0) + (b.x == m ? b.y : 0));
+}
+// leaves: Hr[r] = inclusive prefix of the difference array = the exclusive scan at r + 1; padding leaves never win
+__global__ void place_seg_leaves_kernel(const int32_t* __restrict__ scanned, int R, int P2, int2* __restrict__ seg) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < P2) seg[P2 + r] = r < R ? make_int2(scanned[r + 1], 1) : make_int2(INT_MAX, 0);
+}
+__global__ void place_seg_level_kernel(int2* __restrict__ seg, int lo) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < lo) { const int v = lo + i; seg[v] = seg_comb(seg[2 * v], seg[2 * v + 1]); }
+}
+
+// ---- segment tree queries ----------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ int2 seg_query(const int2* __restrict__ seg, int P2, int l, int r) {
+  int2 acc = make_int2(INT_MAX, 0);
+  for (l += P2, r += P2; l < r; l >>= 1, r >>= 1) {
+    if (l & 1) acc = seg_comb(acc, __ldg(seg + l++));
+    if (r & 1) acc = seg_comb(acc, __ldg(seg + --r));
+  }
+  return acc;
+}
+// first leaf at or after l whose Hr is <= target (the caller knows one exists before its segment ends): climb to the next subtree to
+// the right until one holds such a leaf, then descend to its leftmost
+__device__ __forceinline__ int seg_find_first(const int2* __restrict__ seg, int P2, int l, int target) {
+  int v = P2 + l;
+  while (__ldg(seg + v).x > target) {
+    while (v & 1) v >>= 1;
+    if (v == 0) return -1;
+    ++v;
+  }
+  while (v < P2) v = __ldg(seg + 2 * v).x <= target ? 2 * v : 2 * v + 1;
+  return v - P2;
+}
+
+// ---- stable warp-level LSD radix sort of (key, value) pairs in global scratch -----------------------------------------------------------
+// Sorts n pairs by key bits [0, bits), ping-ponging between (k0, v0) and (k1, v1); returns true if the result is in (k1, v1).  Equal
+// keys keep their order (a chunk of 32 is scattered in lane order: rank among the lanes of the same digit).
+__device__ bool warp_radix_sort(uint32_t* k0, uint32_t* v0, uint32_t* k1, uint32_t* v1, int n, int bits, int* cnt, int lane) {
+  bool alt = false;
+  if (n < 2) return alt;
+  for (int sh = 0; sh < bits; sh += 8) {
+    const uint32_t* ks = alt ? k1 : k0; const uint32_t* vs = alt ? v1 : v0;
+    uint32_t* kd = alt ? k0 : k1; uint32_t* vd = alt ? v0 : v1;
+    for (int d = lane; d < 256; d += 32) cnt[d] = 0;
+    __syncwarp();
+    for (int i = lane; i < n; i += 32) atomicAdd(cnt + ((ks[i] >> sh) & 255), 1);
+    __syncwarp();
+    int loc[8], s = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { loc[j] = cnt[lane * 8 + j]; s += loc[j]; }
+    int run = warp_scan_incl(s, lane) - s;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { cnt[lane * 8 + j] = run; run += loc[j]; }
+    __syncwarp();
+    for (int i0 = 0; i0 < n; i0 += 32) {
+      const int i = i0 + lane;
+      const bool act = i < n;
+      const uint32_t key = act ? ks[i] : 0u, val = act ? vs[i] : 0u;
+      const int d = act ? (int)((key >> sh) & 255) : 256 + lane;
+      const unsigned peers = __match_any_sync(0xffffffffu, d);
+      const int rank = __popc(peers & ((1u << lane) - 1u));
+      const int base = act ? cnt[d] : 0;
+      __syncwarp();
+      if (act && rank == 0) cnt[d] = base + __popc(peers);
+      __syncwarp();
+      if (act) { kd[base + rank] = key; vd[base + rank] = val; }
+    }
+    __syncwarp();
+    alt = !alt;
+  }
+  return alt;
+}
+
+__device__ __forceinline__ int warp_min(int v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+
+struct PlaceParams {
+  ForestDev f;
+  int32_t nb, N, R, P2, L, site_bits, pos_bits, can_change_root, max_best, s0, s1, pad;
+  const int32_t* site_off; const int4* rec; const int2* seg; const uint8_t* ref;
+  const int32_t* delta_off; const int32_t* delta_site; const uint8_t* delta_to;
+  const int32_t* miss_off; const int32_t* miss_start; const int32_t* miss_end;
+  const int64_t* scr_off;        // [S + 1] words of scratch per sample (prefix); a batch uses scratch + scr_off[k] - scr_off[s0]
+  uint32_t* scratch;
+  dphy_placement* out;
+  dphy_candidate_region* best;
+};
+
+// region index -> (device position, mut_idx) and the record the study would emit for it
+__device__ __forceinline__ dphy_candidate_region place_region_record(const PlaceParams& P, int r) {
+  const ForestDev& f = P.f;
+  dphy_candidate_region c;
+  if (r == 0) {
+    c.branch = f.node_id[P.nb]; c.mut_idx = f.mut_off[P.nb + 1] - f.mut_off[P.nb]; c.t_min = -DBL_MAX; c.t_max = f.t[P.nb];
+  } else {
+    int lo = P.nb + 1, hi = P.nb + P.N - 1;
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (region_base(f, P.nb, mid) <= r) lo = mid; else hi = mid - 1; }
+    const int j = r - region_base(f, P.nb, lo), m0 = f.mut_off[lo], n = f.mut_off[lo + 1] - m0;
+    c.branch = f.node_id[lo]; c.mut_idx = j;
+    c.t_min = j == 0 ? f.t[f.parent_pos[lo]] : f.mut_t[m0 + j - 1];
+    c.t_max = j == n ? f.t[lo] : f.mut_t[m0 + j];
+  }
+  c.min_muts = 0; c.pad_ = 0; c.log_W_over_Wmax = 0.0; c.W_over_Wmax = 0.0;
+  return c;
+}
+
+constexpr int kPlaceWarps = 8;
+
+// one warp per sample
+__global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(PlaceParams P) {
+  __shared__ int s_cnt[kPlaceWarps][256];
+  __shared__ int s_n[kPlaceWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int k = P.s0 + blockIdx.x * kPlaceWarps + warp;
+  if (k >= P.s1) return;
+  int* cnt = s_cnt[warp];
+  const int d0 = P.delta_off[k], nd = P.delta_off[k + 1] - d0;
+  const int i0 = P.miss_off[k], ni = P.miss_off[k + 1] - i0;
+  const int64_t words = P.scr_off[k + 1] - P.scr_off[k];
+  const int E = (int)(words / 4 - nd - ni);
+  uint32_t* ek0 = P.scratch + (P.scr_off[k] - P.scr_off[P.s0]);
+  uint32_t *ev0 = ek0 + E, *ek1 = ev0 + E, *ev1 = ek1 + E;
+  uint32_t *dk0 = ev1 + E, *dv0 = dk0 + nd, *dk1 = dv0 + nd, *dv1 = dk1 + nd;
+  uint32_t *ik0 = dv1 + nd, *iv0 = ik0 + ni, *ik1 = iv0 + ni, *iv1 = ik1 + ni;
+
+  // (1) missing intervals sorted by start, then cut to disjoint pieces: piece i = [max(start_i, max end before i), end_i)
+  // (empty pieces keep start == end; starts stay ascending, so a site's piece is found by one binary search)
+  for (int i = lane; i < ni; i += 32) { ik0[i] = (uint32_t)P.miss_start[i0 + i]; iv0[i] = (uint32_t)P.miss_end[i0 + i]; }
+  __syncwarp();
+  const bool ialt = warp_radix_sort(ik0, iv0, ik1, iv1, ni, P.site_bits, cnt, lane);
+  uint32_t* is = ialt ? ik1 : ik0;
+  uint32_t* ie = ialt ? iv1 : iv0;
+  int carry = 0;
+  for (int b0 = 0; b0 < ni; b0 += 32) {
+    const int i = b0 + lane;
+    const int s = i < ni ? (int)is[i] : 0, e = i < ni ? (int)ie[i] : 0;
+    int incl = e;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl = max(incl, u); }
+    int excl = __shfl_up_sync(0xffffffffu, incl, 1);
+    if (lane == 0) excl = 0;
+    const int s2 = max(s, max(excl, carry));
+    if (i < ni) { is[i] = (uint32_t)s2; ie[i] = (uint32_t)max(e, s2); }
+    carry = max(carry, __shfl_sync(0xffffffffu, incl, 31));
+  }
+  __syncwarp();
+
+  // (2) deltas sorted by site, stable: the last delta of a site in array order is the last of its run
+  for (int i = lane; i < nd; i += 32) { dk0[i] = (uint32_t)P.delta_site[d0 + i]; dv0[i] = P.delta_to[d0 + i]; }
+  __syncwarp();
+  const bool dalt = warp_radix_sort(dk0, dv0, dk1, dv1, nd, P.site_bits, cnt, lane);
+  const uint32_t* ds = dalt ? dk1 : dk0;
+  const uint32_t* dt = dalt ? dv1 : dv0;
+
+  // (3) the endpoints (position, +-c) of every mutation of A with c != 0
+  if (lane == 0) s_n[warp] = 0;
+  __syncwarp();
+  int B = 0;
+  for (int i = lane; i < nd; i += 32) {
+    const int l = (int)ds[i];
+    if (i + 1 < nd && (int)ds[i + 1] == l) continue;
+    int lo = 0, hi = ni;
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if ((int)is[mid] <= l) lo = mid + 1; else hi = mid; }
+    if (lo > 0 && l < (int)ie[lo - 1]) continue;
+    const int x = (int)dt[i];
+    B += x != (int)P.ref[l];
+    for (int j = P.site_off[l]; j < P.site_off[l + 1]; ++j) {
+      const int4 m = __ldg(P.rec + j);
+      const int c = (int)((m.z & 3) != x) - (int)((m.z >> 2) != x) - m.w;
+      if (c) { const int q = atomicAdd(&s_n[warp], 2); ek0[q] = (uint32_t)m.x; ev0[q] = (uint32_t)c; ek0[q + 1] = (uint32_t)m.y; ev0[q + 1] = (uint32_t)-c; }
+    }
+  }
+  constexpr int kLanePiece = 64;        // pieces with more mutations than this are spread over the warp
+  for (int i = lane; i < ni; i += 32) {
+    const int j0 = P.site_off[is[i]], j1 = P.site_off[ie[i]];
+    if (j1 - j0 > kLanePiece) continue;
+    for (int j = j0; j < j1; ++j) {
+      const int4 m = __ldg(P.rec + j);
+      if (m.w) { const int q = atomicAdd(&s_n[warp], 2); ek0[q] = (uint32_t)m.x; ev0[q] = (uint32_t)-m.w; ek0[q + 1] = (uint32_t)m.y; ev0[q + 1] = (uint32_t)m.w; }
+    }
+  }
+  for (int i = 0; i < ni; ++i) {
+    const int j0 = P.site_off[is[i]], j1 = P.site_off[ie[i]];
+    if (j1 - j0 <= kLanePiece) continue;
+    for (int j = j0 + lane; j < j1; j += 32) {
+      const int4 m = __ldg(P.rec + j);
+      if (m.w) { const int q = atomicAdd(&s_n[warp], 2); ek0[q] = (uint32_t)m.x; ev0[q] = (uint32_t)-m.w; ek0[q + 1] = (uint32_t)m.y; ev0[q + 1] = (uint32_t)m.w; }
+    }
+  }
+  B = warp_sum(B);
+  __syncwarp();
+  const int n = s_n[warp];
+  const bool ealt = warp_radix_sort(ek0, ev0, ek1, ev1, n, P.pos_bits, cnt, lane);
+  const uint32_t* ks = ealt ? ek1 : ek0;
+  const uint32_t* vs = ealt ? ev1 : ev0;
+
+  // (4) sweep: piece j in [-1, n) is [pos_j, pos_{j+1}) (pos_{-1} = first region, pos_n = R) with correction = prefix of c up to j
+  const int start0 = P.can_change_root ? 0 : 1;
+  int bv = INT_MAX, bc = 0, bl = 0, bm = 0;
+  carry = 0;
+  for (int b0 = -1; b0 < n; b0 += 32) {
+    const int j = b0 + lane;
+    const int c = (j >= 0 && j < n) ? (int)vs[j] : 0;
+    const int corr = warp_scan_incl(c, lane) + carry;
+    carry = __shfl_sync(0xffffffffu, corr, 31);
+    if (j < n) {
+      const int l = j < 0 ? start0 : max((int)ks[j], start0), r = j + 1 < n ? (int)ks[j + 1] : P.R;
+      if (l < r) {
+        const int2 q = seg_query(P.seg, P.P2, l, r);
+        const int v = q.x + corr;
+        if (v < bv) { bv = v; bc = q.y; bl = l; bm = q.x; }
+        else if (v == bv) bc += q.y;
+      }
+    }
+  }
+  const int best = warp_min(bv);
+  const int count = warp_sum(bv == best ? bc : 0);
+  const int first_l = warp_min(bv == best ? bl : INT_MAX);
+  int first = -1;
+  const unsigned owner = __ballot_sync(0xffffffffu, bv == best && bl == first_l && best != INT_MAX);
+  if (owner) {
+    const int ol = __ffs(owner) - 1;
+    if (lane == ol) first = seg_find_first(P.seg, P.P2, bl, bm);
+    first = __shfl_sync(0xffffffffu, first, ol);
+  }
+  if (lane == 0) {
+    dphy_placement o;
+    o.min_muts = -1; o.num_best = 0; o.branch = -1; o.mut_idx = -1;
+    if (first >= 0) {
+      const dphy_candidate_region fr = place_region_record(P, first);
+      o.min_muts = B + best; o.num_best = count; o.branch = fr.branch; o.mut_idx = fr.mut_idx;
+    }
+    P.out[k] = o;
+  }
+  if (P.max_best <= 0) return;
+
+  // (5) the first max_best regions attaining the minimum, in emission order: the pieces whose minimum hits it, leaf by leaf
+  dphy_candidate_region* bo = P.best + (size_t)k * P.max_best;
+  int emitted = 0;
+  carry = 0;
+  for (int b0 = -1; first >= 0 && b0 < n && emitted < P.max_best; b0 += 32) {
+    const int j = b0 + lane;
+    const int c = (j >= 0 && j < n) ? (int)vs[j] : 0;
+    const int corr = warp_scan_incl(c, lane) + carry;
+    carry = __shfl_sync(0xffffffffu, corr, 31);
+    int l = 0, r = 0, hit = 0, m = 0;
+    if (j < n) {
+      l = j < 0 ? start0 : max((int)ks[j], start0); r = j + 1 < n ? (int)ks[j + 1] : P.R;
+      if (l < r) { const int2 q = seg_query(P.seg, P.P2, l, r); m = q.x; hit = q.x + corr == best ? q.y : 0; }
+    }
+    const int incl = warp_scan_incl(hit, lane);
+    const int off = emitted + incl - hit;
+    const int take = off < P.max_best ? min(hit, P.max_best - off) : 0;
+    for (int t = 0; t < take; ++t) {
+      const int p = seg_find_first(P.seg, P.P2, l, m);
+      dphy_candidate_region rr = place_region_record(P, p);
+      rr.min_muts = B + best;
+      bo[off + t] = rr;
+      l = p + 1;
+    }
+    emitted = min(P.max_best, emitted + __shfl_sync(0xffffffffu, incl, 31));
+  }
+  for (int t = emitted + lane; t < P.max_best; t += 32) {
+    dphy_candidate_region u;
+    u.branch = -1; u.mut_idx = 0; u.t_min = 0.0; u.t_max = 0.0; u.min_muts = 0; u.pad_ = 0; u.log_W_over_Wmax = 0.0; u.W_over_Wmax = 0.0;
+    bo[t] = u;
+  }
+}
+
+namespace {
+size_t al(size_t x) { return (x + 255) / 256 * 256; }
+int bits_for(int64_t max_value) { int b = 1; while (b < 31 && ((int64_t)1 << b) <= max_value) ++b; return b; }
+
+// the per-tree index: built by the first placement on the tree, freed with the forest (dphy_forest_apply_rows swaps in a fresh forest,
+// so a rebuilt tree gets a fresh index; dphy_forest_set_node_times changes no entry, the times are read when the records are made)
+int ensure_place_index(dphy_ctx* ctx, dphy_forest* fo, int tree) {
+  if (fo->place.size() != fo->trees.size()) fo->place.assign(fo->trees.size(), PlaceIndex{});
+  PlaceIndex& X = fo->place[tree];
+  if (X.seg) return DPHY_OK;
+  const TreeDev& T = fo->trees[tree];
+  const dphy_sites* si = fo->sites[T.sites_id];
+  const int nb = T.node_base, N = T.num_nodes, L = si->L;
+  int32_t h_mo[3];
+  DPHY_CUDA(ctx, cudaMemcpyAsync(h_mo, fo->h.mut_off + nb, sizeof(int32_t) * 2, cudaMemcpyDeviceToHost, ctx->stream));
+  DPHY_CUDA(ctx, cudaMemcpyAsync(h_mo + 2, fo->h.mut_off + nb + N, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  DPHY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  const int64_t M = (int64_t)h_mo[2] - h_mo[0];
+  const int64_t R = (int64_t)N + M - (h_mo[1] - h_mo[0]);
+  if (R + 2 >= (int64_t)1 << 30) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: tree too large");
+  int64_t P2 = 1;
+  while (P2 < R) P2 <<= 1;
+  // resident: site_off [L+1], rec [M], seg [2 P2]; temporaries (freed once built): fill [L], diff [R+2], scan tiles
+  const size_t b_so = 0, b_rec = al(sizeof(int32_t) * (L + 1)), b_seg = b_rec + al(sizeof(int4) * std::max<int64_t>(M, 1));
+  const size_t total = b_seg + al(sizeof(int2) * 2 * P2);
+  const size_t b_fill = 0, b_diff = al(sizeof(int32_t) * L), b_tt = b_diff + al(sizeof(int32_t) * (R + 2));
+  const size_t tmp_bytes = b_tt + al(sizeof(int32_t) * ((std::max<int64_t>(L, R + 1) + 1) / 8192 + 2));
+  char* d = nullptr;
+  char* tmp = nullptr;
+  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index)");
+  if (cudaMallocAsync((void**)&tmp, tmp_bytes, ctx->stream) != cudaSuccess) {
+    cudaFreeAsync(d, ctx->stream);
+    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index scratch)");
+  }
+  int32_t* so = (int32_t*)(d + b_so); int4* rec = (int4*)(d + b_rec); int2* seg = (int2*)(d + b_seg);
+  int32_t* fill = (int32_t*)(tmp + b_fill); int32_t* diff = (int32_t*)(tmp + b_diff); int32_t* tt = (int32_t*)(tmp + b_tt);
+  int st = check_cuda(ctx, cudaMemsetAsync(d, 0, b_rec, ctx->stream), "place index memset");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaMemsetAsync(tmp, 0, b_tt, ctx->stream), "place index memset");
+  if (st == DPHY_OK) {
+    const int m0 = h_mo[0], Mi = (int)M;
+    if (Mi > 0) place_site_hist_kernel<<<(Mi + 255) / 256, 256, 0, ctx->stream>>>(fo->h, m0, Mi, so);
+    st = launch_scan_i32(ctx, so, L + 1, tt);
+    if (st == DPHY_OK && Mi > 0)
+      place_site_scatter_kernel<<<(Mi + 255) / 256, 256, 0, ctx->stream>>>(fo->h, nb, N, (int)R, m0, Mi, si->d_ref, so, fill, rec, diff);
+    if (st == DPHY_OK) st = launch_scan_i32(ctx, diff, (int)R + 2, tt);
+    if (st == DPHY_OK) {
+      place_seg_leaves_kernel<<<(unsigned)((P2 + 255) / 256), 256, 0, ctx->stream>>>(diff, (int)R, (int)P2, seg);
+      ctx->launches += 3;
+      for (int64_t lo = P2 / 2; lo >= 1; lo /= 2) { place_seg_level_kernel<<<(unsigned)((lo + 255) / 256), 256, 0, ctx->stream>>>(seg, (int)lo); ++ctx->launches; }
+      st = check_cuda(ctx, cudaGetLastError(), "place index kernels");
+    }
+  }
+  std::vector<int32_t> h_so(L + 1);
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaMemcpyAsync(h_so.data(), so, sizeof(int32_t) * (L + 1), cudaMemcpyDeviceToHost, ctx->stream), "D2H");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "place index build");
+  cudaFreeAsync(tmp, ctx->stream);
+  if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return st; }
+  fo->allocs.push_back(d);
+  fo->bytes += total;
+  X.R = (int32_t)R; X.P2 = (int32_t)P2; X.L = L;
+  X.site_off = so; X.rec = rec; X.seg = seg; X.bytes = total;
+  X.h_site_off = std::move(h_so);
+  return DPHY_OK;
+}
+}  // namespace
+
+}  // namespace dphy
+
+using namespace dphy;
+
+extern "C" {
+
+int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sample_set* set, int32_t can_change_root,
+                              int32_t max_best, dphy_placement* out, dphy_candidate_region* best) {
+  if (!ctx || !fo || !set || max_best < 0 || set->num_samples < 0) return DPHY_ERR_INVALID_ARGUMENT;
+  if (tree < 0 || tree >= fo->h.num_trees) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "place: tree index out of range");
+  const int S = set->num_samples;
+  if (S == 0) return DPHY_OK;
+  if (!out || (max_best > 0 && !best)) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: output buffers missing");
+  if (!set->delta_off || !set->miss_off) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: offset arrays missing");
+  // ---- validation (the rules of a DPHY_SPR_X_REL_REF request), before anything is written ----
+  const int32_t* dof = set->delta_off; const int32_t* mof = set->miss_off;
+  if (dof[0] < 0 || mof[0] < 0) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: negative offsets");
+  for (int k = 0; k < S; ++k)
+    if (dof[k + 1] < dof[k] || mof[k + 1] < mof[k]) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: offsets not monotone");
+  const int64_t D = (int64_t)dof[S] - dof[0], I = (int64_t)mof[S] - mof[0];
+  if ((D > 0 && (!set->delta_site || !set->delta_to)) || (I > 0 && (!set->miss_start || !set->miss_end)))
+    return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: sample arrays missing");
+  const TreeDev& T = fo->trees[tree];
+  const int L = fo->sites[T.sites_id]->L;
+  for (int64_t i = dof[0]; i < dof[S]; ++i)
+    if (set->delta_site[i] < 0 || set->delta_site[i] >= L || set->delta_to[i] > 3) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "place: delta out of range");
+  for (int64_t i = mof[0]; i < mof[S]; ++i)
+    if (set->miss_start[i] < 0 || set->miss_end[i] > L || set->miss_start[i] >= set->miss_end[i])
+      return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "place: missing interval out of range");
+  cudaSetDevice(ctx->device);
+  int st = ensure_place_index(ctx, fo, tree);
+  if (st != DPHY_OK) return st;
+  const PlaceIndex& X = fo->place[tree];
+  // ---- scratch per sample: endpoint pairs (2 per mutation of A, bounded by the site table's runs), delta and interval pairs; each
+  // ping-ponged by the radix sort: 4 words per pair ----
+  const int32_t* so = X.h_site_off.data();
+  std::vector<int64_t> scr(S + 1, 0);
+  for (int k = 0; k < S; ++k) {
+    int64_t a = 0;
+    for (int i = dof[k]; i < dof[k + 1]; ++i) a += so[set->delta_site[i] + 1] - so[set->delta_site[i]];
+    for (int i = mof[k]; i < mof[k + 1]; ++i) a += so[set->miss_end[i]] - so[set->miss_start[i]];
+    if (2 * a > INT_MAX) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: sample too large");
+    scr[k + 1] = scr[k] + 4 * (2 * a + (dof[k + 1] - dof[k]) + (mof[k + 1] - mof[k]));
+  }
+  // samples go in batches of at most kBudget scratch words (at least one sample per batch)
+  constexpr int64_t kBudget = (int64_t)64 << 20;
+  std::vector<int> cuts{0};
+  int64_t max_words = 1;
+  for (int k = 0; k < S; ++k) {
+    if (k > cuts.back() && scr[k + 1] - scr[cuts.back()] > kBudget) cuts.push_back(k);
+    max_words = std::max(max_words, scr[k + 1] - scr[cuts.back()]);
+  }
+  cuts.push_back(S);
+  // ---- inputs through the pinned slab; outputs back through it ----
+  const size_t b_doff = 0, b_moff = al(4 * (size_t)(S + 1)), b_ds = b_moff + al(4 * (size_t)(S + 1)), b_dt = b_ds + al(4 * (size_t)D);
+  const size_t b_ms = b_dt + al((size_t)D), b_me = b_ms + al(4 * (size_t)I), b_scr = b_me + al(4 * (size_t)I);
+  const size_t in_bytes = b_scr + al(8 * (size_t)(S + 1));
+  const size_t b_out = in_bytes, b_best = b_out + al(sizeof(dphy_placement) * (size_t)S);
+  const size_t io_bytes = b_best + al(sizeof(dphy_candidate_region) * (size_t)S * max_best);
+  const size_t b_scratch = io_bytes, total = b_scratch + al(4 * (size_t)max_words);
+  char* d = nullptr;
+  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place)");
+  void* hv = nullptr;
+  st = acquire_pinned(ctx, io_bytes, &hv);
+  if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return st; }
+  char* h = (char*)hv;
+  int32_t* h_doff = (int32_t*)(h + b_doff); int32_t* h_moff = (int32_t*)(h + b_moff);
+  for (int k = 0; k <= S; ++k) { h_doff[k] = dof[k] - dof[0]; h_moff[k] = mof[k] - mof[0]; }
+  if (D) { std::memcpy(h + b_ds, set->delta_site + dof[0], 4 * D); std::memcpy(h + b_dt, set->delta_to + dof[0], D); }
+  if (I) { std::memcpy(h + b_ms, set->miss_start + mof[0], 4 * I); std::memcpy(h + b_me, set->miss_end + mof[0], 4 * I); }
+  std::memcpy(h + b_scr, scr.data(), 8 * (size_t)(S + 1));
+  cudaError_t ce = cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
+  PlaceParams P;
+  std::memset(&P, 0, sizeof(P));
+  P.f = fo->h; P.nb = T.node_base; P.N = T.num_nodes; P.R = X.R; P.P2 = X.P2; P.L = L;
+  P.site_bits = bits_for(L); P.pos_bits = bits_for(X.R); P.can_change_root = can_change_root != 0; P.max_best = max_best;
+  P.site_off = X.site_off; P.rec = X.rec; P.seg = X.seg; P.ref = fo->sites[T.sites_id]->d_ref;
+  P.delta_off = (const int32_t*)(d + b_doff); P.delta_site = (const int32_t*)(d + b_ds); P.delta_to = (const uint8_t*)(d + b_dt);
+  P.miss_off = (const int32_t*)(d + b_moff); P.miss_start = (const int32_t*)(d + b_ms); P.miss_end = (const int32_t*)(d + b_me);
+  P.scr_off = (const int64_t*)(d + b_scr); P.scratch = (uint32_t*)(d + b_scratch);
+  P.out = (dphy_placement*)(d + b_out); P.best = (dphy_candidate_region*)(d + b_best);
+  for (size_t c = 0; c + 1 < cuts.size() && ce == cudaSuccess; ++c) {
+    P.s0 = cuts[c]; P.s1 = cuts[c + 1];
+    place_samples_kernel<<<(P.s1 - P.s0 + kPlaceWarps - 1) / kPlaceWarps, kPlaceWarps * 32, 0, ctx->stream>>>(P);
+    ++ctx->launches;
+    ce = cudaGetLastError();
+  }
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(h + b_out, d + b_out, io_bytes - b_out, cudaMemcpyDeviceToHost, ctx->stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
+  cudaFreeAsync(d, ctx->stream);
+  if (ce != cudaSuccess) { release_pinned_async(ctx); return check_cuda(ctx, ce, "place samples"); }
+  std::memcpy(out, h + b_out, sizeof(dphy_placement) * (size_t)S);
+  if (max_best > 0) std::memcpy(best, h + b_best, sizeof(dphy_candidate_region) * (size_t)S * max_best);
+  release_pinned_async(ctx);
+  return DPHY_OK;
+}
+
+}  // extern "C"

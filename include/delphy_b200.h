@@ -399,6 +399,45 @@ int  dphy_spr_batch_log_alpha_in_region(dphy_ctx* ctx, dphy_spr_batch* batch, in
 int  dphy_gamma_q(dphy_ctx* ctx, int32_t n, const double* a, const double* x, double* out);
 int  dphy_gamma_q_inv(dphy_ctx* ctx, int32_t n, const double* a, const double* q, double* out);
 
+/* ---- placement of new samples (maximum parsimony) ---------------------------------------------------------------------------------
+ * Where on tree `tree` does each new sequence go, at how many mutations, and how many equally good places are there -- the per-tip step
+ * of build_usher_like_tree (core/phylo_tree.cpp:918-932), UShER-style placement of fresh samples onto an existing or posterior tree.
+ * For sample k, take the regions dphy_spr_study_batch enumerates for the request
+ *   {tree, X = -1, x_state_mode = DPHY_SPR_X_REL_REF, start = (root, #root mutations), max_muts_from_start = INT32_MAX,
+ *    t_X = DBL_MAX, lambda_X = 0, can_change_root, x deltas / missing intervals = sample k's}
+ * (the region list of the reference's unbounded study from the root; core/spr_study.cpp:9-209).  Then out[k] holds
+ *   min_muts = the least min_muts over those regions,  num_best = how many regions attain it,
+ *   (branch, mut_idx) = the FIRST region attaining it in the study's emission order;
+ * and, with max_best > 0, best[k * max_best + i] the first max_best such regions in emission order as full records (branch, mut_idx,
+ * t_min, t_max, min_muts; weights 0); unused slots are zero with branch = -1.  A tree without regions (a lone root and
+ * can_change_root == 0) gives min_muts = -1, num_best = 0, branch = mut_idx = -1.  Everything equals what the study gives, bit for bit.
+ * Samples are those of a DPHY_SPR_X_REL_REF request: x = the reference overlaid with the deltas in array order (a later delta of
+ * the same site wins); a site inside any interval is missing (intervals may overlap and come in any order).  Sample k's deltas are
+ * [delta_off[k], delta_off[k+1]) and its intervals [miss_off[k], miss_off[k+1]) -- the arrays dphy_maple_view gives.
+ * Validation as for a request, before anything is written: DPHY_ERR_OUT_OF_RANGE for a tree index, a site outside [0, L), a state
+ * above 3 or an interval outside 0 <= start < end <= L; DPHY_ERR_INVALID_ARGUMENT for decreasing offsets or missing arrays.
+ * Precondition (as for the study's own delta arithmetic): every mutation's `from` is the state of the sequence above it.
+ * Cost: a per-tree index (mutations by site with the block of regions below each, and a min / count segment tree over the regions'
+ * reference Hamming potential; 16 B per mutation + 8 B per segment-tree entry, 2 x the power of two >= R entries) is built by the first call on the tree and kept with the
+ * forest (dphy_forest_apply_rows drops it, dphy_forest_set_node_times needs no rebuild: times are read when the records are made);
+ * per sample the work is O(|A| log R), A = the tree's mutations at the sample's delta and missing sites, R = the number of regions.
+ * Synchronous: host arrays in, host results out.
+ * Out of scope: date-constrained placement (dropping the regions with t_min >= t_X, remove_regions_in_Xs_future): with a per-sample
+ * t_X the kept regions differ per sample; use dphy_spr_study_batch for it. */
+typedef struct dphy_sample_set {
+  int32_t num_samples;
+  int32_t reserved;
+  const int32_t* delta_off;           /* [num_samples + 1] */
+  const int32_t* delta_site; const uint8_t* delta_to;
+  const int32_t* miss_off;            /* [num_samples + 1] */
+  const int32_t* miss_start; const int32_t* miss_end;
+} dphy_sample_set;
+typedef struct dphy_placement {
+  int32_t min_muts, num_best, branch, mut_idx;   /* branch: host node index */
+} dphy_placement;
+int  dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* forest, int32_t tree, const dphy_sample_set* samples, int32_t can_change_root,
+                               int32_t max_best, dphy_placement* out, dphy_candidate_region* best /* [num_samples * max_best] or NULL */);
+
 /* ---- tree partitioning (one or more parts per GPU) ------------------------------------------------------------- */
 /* generate_random_partition_stencil (core/tree_partitioning.h:139-194): up to num_parts-1 cut points.  The coin flips are the
  * reference's: std::bernoulli_distribution{0.5} drawn from std::mt19937{(uint32_t)seed} through absl::BitGenRef, interleaved with
