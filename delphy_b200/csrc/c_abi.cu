@@ -677,7 +677,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   const int b_ioff = slab.reserve(sizeof(int32_t) * (N + 1)), b_is = slab.reserve(sizeof(int2) * I + 64);
   const int b_foff = slab.reserve(sizeof(int32_t) * (N + 1)), b_fsite = slab.reserve(sizeof(int32_t) * F + 64), b_ffrom = slab.reserve(F + 64);
   const int b_fsw = slab.reserve(sizeof(int16_t) * (size_t)fsw_stride * N + 64);
-  const int b_bw = slab.reserve(sizeof(int32_t) * (size_t)fsw_stride * N + 64);
+  const int b_cnt = slab.reserve(sizeof(int32_t) * (size_t)fsw_stride * N + 64);
   // outputs + workspaces
   const int b_lambda = slab.reserve(sizeof(double) * N), b_nsmn = slab.reserve(sizeof(int32_t) * N);
   const int b_fastl = slab.reserve(sizeof(int32_t) * ctiles), b_slowl = slab.reserve(sizeof(int32_t) * ctiles);
@@ -716,9 +716,12 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   // the raw (host-order) arrays stay resident next to the flattened forest: dphy_forest_apply_rows patches them on the device and
   // re-flattens from there, so an edited tree never crosses PCIe again.  The flatten workspaces live in their own block, freed below.
   Slab work;
-  const int w_arcs0 = work.reserve(sizeof(int4) * 2 * N), w_arcs1 = work.reserve(sizeof(int4) * 2 * N);
+  // the Euler-tour arcs (two ping-pong buffers of 2N int4) are dead once the node records are scattered: the count scan's
+  // post-order prefix (N rows of fsw_stride int32) reuses their block
+  const int w_arcs = work.reserve(std::max(sizeof(int4) * 4 * N, sizeof(int32_t) * (size_t)fsw_stride * N));
   const int64_t scan_tiles = (N + 1023) / 1024;
   const int w_scan = work.reserve(sizeof(int32_t) * 3 * scan_tiles);
+  const int w_cnttot = work.reserve(sizeof(uint4) * 2 * (fsw_stride / 4) * scan_tiles);
   const int w_status = work.reserve(sizeof(uint32_t) * 4 + sizeof(int32_t) * num_trees);
   const int w_jobs = work.reserve(sizeof(DeviceCopyJob) * ((size_t)num_trees * 15 + 1));     // device-resident sources only (see below)
 
@@ -851,7 +854,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   h.miss_off = slab.at<int32_t>(dbase, b_ioff); h.miss_se = slab.at<int2>(dbase, b_is);
   h.fs_off = slab.at<int32_t>(dbase, b_foff); h.fs_site = slab.at<int32_t>(dbase, b_fsite); h.fs_code = slab.at<uint8_t>(dbase, b_ffrom);
   h.fsw = slab.at<int16_t>(dbase, b_fsw); h.fsw_stride = fsw_stride; h.pad1 = 0;
-  h.bw = slab.at<int32_t>(dbase, b_bw);
+  h.C = slab.at<int32_t>(dbase, b_cnt);
   fo->d_lambda = slab.at<double>(dbase, b_lambda); fo->d_nsmn = slab.at<int32_t>(dbase, b_nsmn);
   fo->d_tree_out = slab.at<double>(dbase, b_tout); fo->d_tree_iout = slab.at<int32_t>(dbase, b_tiout);
   fo->d_tile_agg = slab.at<double>(dbase, b_tagg); fo->d_tile_iagg = slab.at<int32_t>(dbase, b_tiagg);
@@ -864,7 +867,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   // ---- device side: Euler tour + list ranking -> DFS order; CSR offsets; lists ------------------------------------------
   FlattenParams P{};
   P.trees = h.trees; P.sites = h.sites; P.tile_tree = h.tile_tree; P.raw = tmp.at<RawTreeDev>(tbase, r_raw);
-  P.arcs[0] = work.at<int4>(wbase, w_arcs0); P.arcs[1] = work.at<int4>(wbase, w_arcs1);
+  P.arcs[0] = work.at<int4>(wbase, w_arcs); P.arcs[1] = P.arcs[0] + 2 * N;
   P.scan_tiles = work.at<int32_t>(wbase, w_scan);
   P.status = work.at<uint32_t>(wbase, w_status); P.max_depth = reinterpret_cast<int32_t*>(P.status + 4);
   P.strad_list = fo->d_strad_list;
@@ -880,7 +883,8 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   P.miss_off = const_cast<int32_t*>(h.miss_off); P.miss_se = const_cast<int2*>(h.miss_se);
   P.fs_off = const_cast<int32_t*>(h.fs_off); P.fs_site = const_cast<int32_t*>(h.fs_site); P.fs_code = const_cast<uint8_t*>(h.fs_code);
   P.fsw = const_cast<int16_t*>(h.fsw); P.fsw_stride = fsw_stride;
-  P.bw = const_cast<int32_t*>(h.bw);
+  P.C = const_cast<int32_t*>(h.C);
+  P.cnt_y = work.at<int32_t>(wbase, w_arcs); P.cnt_tot = work.at<uint4>(wbase, w_cnttot);
   if (order_from) {
     P.old_pos_of_node = order_from->h.pos_of_node; P.old_depth = order_from->h.depth; P.old_subtree_size = order_from->h.subtree_size;
     P.old_parent_pos = order_from->h.parent_pos;
@@ -909,7 +913,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
     }
     if (st != DPHY_OK) { sync_copy_streams(ctx); return fail(st); }
     release_pinned_async(ctx);
-    st = launch_flatten_ctiles(ctx, P);
+    st = launch_flatten_finish(ctx, P);
   } else {
     st = launch_flatten(ctx, P, (int)tiles, max_tree_nodes);
   }

@@ -122,12 +122,15 @@ struct ForestDev {
   // - #(overrides whose from-state is a).  With uniform site rates the branch's delta-lambda term is a 4-term dot product.
   const int16_t* fsw;
   int32_t fsw_stride, pad1;
-  // every per-branch list folded into one weight vector (structure only, built at upload by fold_branch_weights_kernel):
-  //   bw[p * fsw_stride + part*4 + a] = #(mutations to a) - #(mutations from a) - #(sites going missing whose reference state is a)
-  //                                     + #(overrides whose reference state is a) - #(overrides whose from-state is a)
-  // With uniform site rates the branch's delta-lambda (core/phylo_tree_calc.h:121-155) is  sum_k mu nu q_a(a) bw[k];
-  // for the root, ref_freq + bw is the state count vector of calc_log_root_prior (core/phylo_tree_calc.cpp:467-504).
-  const int32_t* bw;
+  // per-node state counts (structure only, built at upload by fold_branch_weights_kernel + the count scan of kernels_flatten.cu).
+  // Every per-branch list is folded into one weight vector
+  //   bw[p][part*4 + a] = #(mutations to a) - #(mutations from a) - #(sites going missing whose reference state is a)
+  //                       + #(overrides whose reference state is a) - #(overrides whose from-state is a),
+  // and C is its root -> q prefix:  C[q * fsw_stride + k] = sum of bw[a][k] over the nodes a on the path from the root to q, both
+  // included.  ref_freq + C[q] is the state count vector of the sequence at q, so with uniform site rates
+  // lambda_i(q) = lambda_ref + sum_k mu nu q_a(a) C[q][k] (core/phylo_tree_calc.h:121-155 summed down the path), and for the root
+  // ref_freq + C is the state count vector of calc_log_root_prior (core/phylo_tree_calc.cpp:467-504).
+  const int32_t* C;
   // host-order lookup: device position of (tree, host node id) = pos_of_node[tree.node_base + id]
   const int32_t* pos_of_node;
 };
@@ -170,7 +173,9 @@ struct FlattenParams {
   int32_t* miss_off; int2* miss_se;
   int32_t* fs_off; int32_t* fs_site; uint8_t* fs_code;
   int16_t* fsw; int32_t fsw_stride;
-  int32_t* bw;
+  int32_t* C;
+  int32_t* cnt_y;              // [num_nodes][fsw_stride] workspace of the count scan: prefix of bw over the post-order lists
+  uint4* cnt_tot;              // [ceil(num_nodes / 1024)][fsw_stride / 4][2] its per-tile totals
   // re-flatten of trees whose links did not change (dphy_forest_apply_rows): the DFS order of the forest being replaced is reused
   // and the Euler-tour ranking skipped (null: rank from scratch)
   const int32_t* old_pos_of_node = nullptr; const int32_t* old_depth = nullptr; const int32_t* old_subtree_size = nullptr;
@@ -320,9 +325,11 @@ int refresh_sites(dphy_ctx* ctx, dphy_forest* f);   // c_abi.cu
 // stage 0: Euler-tour ranking (needs parent / child0 / child1 only); stage 1: node records + CSR offset scans (needs t and the
 // three offset arrays); stage 2: list gathers, weight fold, tile descriptors (needs the lists); -1: all
 int launch_flatten(dphy_ctx* ctx, const FlattenParams& P, int num_tiles, int max_tree_nodes, int stage = -1);
-// stage 2 split per tree (direct uploads: each tree's lists are gathered as soon as its own arrays have landed)
+// stage 2 split per tree (direct uploads: each tree's lists are gathered as soon as its own arrays have landed) ...
 int launch_flatten_lists(dphy_ctx* ctx, FlattenParams P, int first_tile, int num_tiles);
-int launch_flatten_ctiles(dphy_ctx* ctx, const FlattenParams& P);
+// ... then, once every tree's lists are folded: per-node state counts (ForestDev::C), log-G tile descriptors.  launch_flatten
+// calls it itself.
+int launch_flatten_finish(dphy_ctx* ctx, const FlattenParams& P);
 // exclusive scan of n int32 in place (api_tree.cu); tile_tot holds (n + 8191) / 8192 ints
 int launch_scan_i32(dphy_ctx* ctx, int32_t* v, int n, int32_t* tile_tot);
 // many device-to-device array copies in one launch (16-byte aligned sources and destinations)

@@ -301,8 +301,122 @@ __global__ void __launch_bounds__(kTile) fold_branch_weights_kernel(FlattenParam
       const int fk = k < K ? s_f[tid * kBwRow + k] : 0;
       if (fk > 32767 || fk < -32768) flag_error(P, kFlattenErrFswRange);
       P.fsw[(size_t)p * stride + k] = (int16_t)fk;
-      P.bw[(size_t)p * stride + k] = (k < K ? s_w[tid * kBwRow + k] : 0) + fk;
+      P.C[(size_t)p * stride + k] = (k < K ? s_w[tid * kBwRow + k] : 0) + fk;   // bw; turned into C by the count scan below
     }
+  }
+}
+
+// ---- (3e) per-node state counts: C[q] = sum of bw over the root -> q path (see ForestDev::C) ---------------------------------------------
+// With X the inclusive prefix of bw over the forest in device order and Y the exclusive prefix of bw over the post-order lists
+// (tree after tree), C[q] = X[q] - Y[q - depth[q]]: the nodes opened up to q minus the q - depth[q] nodes of q's tree closed before
+// q.  Every tree's post-order list holds exactly that tree's nodes, so the earlier trees' totals cancel.  X and Y may wrap; they
+// are summed as uint32, and the difference, a bounded state count, comes out exact.  Each int4 column group of the rows is
+// scanned on its own (blockIdx.y); bw lies in P.C, and the last kernel replaces it in place.
+__device__ __forceinline__ uint4 u4_add(uint4 a, uint4 b) { return make_uint4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+__device__ __forceinline__ uint4 u4_sub(uint4 a, uint4 b) { return make_uint4(a.x - b.x, a.y - b.y, a.z - b.z, a.w - b.w); }
+__device__ __forceinline__ uint4 u4_shfl_up(uint4 v, int o) {
+  return make_uint4(__shfl_up_sync(0xffffffffu, v.x, o), __shfl_up_sync(0xffffffffu, v.y, o), __shfl_up_sync(0xffffffffu, v.z, o),
+                    __shfl_up_sync(0xffffffffu, v.w, o));
+}
+// inclusive block scan of one uint4 per thread (blockDim.x == kTile); *total = the block total
+__device__ __forceinline__ uint4 block_scan_incl_u4(uint4 v, uint4* ws, uint4* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint4 u = u4_shfl_up(v, o);
+    if (lane >= o) v = u4_add(v, u);
+  }
+  if (lane == 31) ws[warp] = v;
+  __syncthreads();
+  uint4 base = make_uint4(0, 0, 0, 0), tot = make_uint4(0, 0, 0, 0);
+#pragma unroll
+  for (int w = 0; w < kTile / 32; ++w) { if (w < warp) base = u4_add(base, ws[w]); tot = u4_add(tot, ws[w]); }
+  __syncthreads();                         // ws may be rewritten by the next scan
+  *total = tot;
+  return u4_add(base, v);
+}
+
+// per scan tile of kScanTile rows: totals of X's and Y's terms -> cnt_tot[(tile * G + g) * 2 + {0, 1}]
+__global__ void __launch_bounds__(kTile) counts_scan_reduce_kernel(FlattenParams P) {
+  __shared__ uint4 s_ws[kTile / 32];
+  const int G = P.fsw_stride / 4, g = blockIdx.y;
+  const uint4* __restrict__ bw4 = reinterpret_cast<const uint4*>(P.C);
+  const int base = blockIdx.x * kScanTile + threadIdx.x * kScanItems;
+  uint4 a = make_uint4(0, 0, 0, 0), b = make_uint4(0, 0, 0, 0);
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    const int i = base + k;
+    if (i < P.num_nodes) {
+      a = u4_add(a, bw4[(size_t)i * G + g]);
+      b = u4_add(b, bw4[(size_t)P.post_node[i] * G + g]);
+    }
+  }
+  uint4 ta, tb;
+  block_scan_incl_u4(a, s_ws, &ta);
+  block_scan_incl_u4(b, s_ws, &tb);
+  if (threadIdx.x == 0) {
+    P.cnt_tot[((size_t)blockIdx.x * G + g) * 2 + 0] = ta;
+    P.cnt_tot[((size_t)blockIdx.x * G + g) * 2 + 1] = tb;
+  }
+}
+
+// exclusive prefix of the tile totals, in place: one CTA per (column group, X | Y)
+__global__ void __launch_bounds__(kTile) counts_scan_spine_kernel(FlattenParams P, int num_scan_tiles) {
+  __shared__ uint4 s_ws[kTile / 32];
+  const int G = P.fsw_stride / 4, col = blockIdx.x;            // col = g * 2 + (0: X, 1: Y)
+  uint4 carry = make_uint4(0, 0, 0, 0);
+  for (int j0 = 0; j0 < num_scan_tiles; j0 += kTile) {
+    const int j = j0 + threadIdx.x;
+    uint4* slot = P.cnt_tot + ((size_t)j * G) * 2 + col;
+    const uint4 v = j < num_scan_tiles ? *slot : make_uint4(0, 0, 0, 0);
+    uint4 tot;
+    const uint4 incl = block_scan_incl_u4(v, s_ws, &tot);
+    if (j < num_scan_tiles) *slot = u4_add(carry, u4_sub(incl, v));
+    carry = u4_add(carry, tot);
+  }
+}
+
+// Y: exclusive prefix of bw over the post-order lists -> cnt_y
+__global__ void __launch_bounds__(kTile) counts_scan_post_kernel(FlattenParams P) {
+  __shared__ uint4 s_ws[kTile / 32];
+  const int G = P.fsw_stride / 4, g = blockIdx.y;
+  const uint4* __restrict__ bw4 = reinterpret_cast<const uint4*>(P.C);
+  uint4* __restrict__ y4 = reinterpret_cast<uint4*>(P.cnt_y);
+  const int base = blockIdx.x * kScanTile + threadIdx.x * kScanItems;
+  uint4 v[kScanItems], run = make_uint4(0, 0, 0, 0);
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    v[k] = base + k < P.num_nodes ? bw4[(size_t)P.post_node[base + k] * G + g] : make_uint4(0, 0, 0, 0);
+    run = u4_add(run, v[k]);
+  }
+  uint4 tot;
+  uint4 ex = u4_sub(block_scan_incl_u4(run, s_ws, &tot), run);
+  ex = u4_add(ex, P.cnt_tot[((size_t)blockIdx.x * G + g) * 2 + 1]);
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) { if (base + k < P.num_nodes) y4[(size_t)(base + k) * G + g] = ex; ex = u4_add(ex, v[k]); }
+}
+
+// C[q] = X[q] - Y[q - depth[q]], X formed here (inclusive prefix of bw in device order), written over bw in place
+__global__ void __launch_bounds__(kTile) counts_scan_apply_kernel(FlattenParams P) {
+  __shared__ uint4 s_ws[kTile / 32];
+  const int G = P.fsw_stride / 4, g = blockIdx.y;
+  uint4* __restrict__ c4 = reinterpret_cast<uint4*>(P.C);
+  const uint4* __restrict__ y4 = reinterpret_cast<const uint4*>(P.cnt_y);
+  const int base = blockIdx.x * kScanTile + threadIdx.x * kScanItems;
+  uint4 v[kScanItems], run = make_uint4(0, 0, 0, 0);
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    v[k] = base + k < P.num_nodes ? c4[(size_t)(base + k) * G + g] : make_uint4(0, 0, 0, 0);
+    run = u4_add(run, v[k]);
+  }
+  uint4 tot;
+  uint4 x = u4_sub(block_scan_incl_u4(run, s_ws, &tot), run);
+  x = u4_add(x, P.cnt_tot[((size_t)blockIdx.x * G + g) * 2 + 0]);
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    const int q = base + k;
+    x = u4_add(x, v[k]);
+    if (q < P.num_nodes) c4[(size_t)q * G + g] = u4_sub(x, y4[(size_t)(q - P.depth[q]) * G + g]);
   }
 }
 
@@ -426,9 +540,9 @@ int launch_flatten(dphy_ctx* ctx, const FlattenParams& P, int num_tiles, int max
   }
   flatten_events_kernel<<<num_tiles, kTile, 0, ctx->stream>>>(P);
   fold_branch_weights_kernel<<<num_tiles, kTile, 0, ctx->stream>>>(P);
-  flatten_ctiles_kernel<<<(P.num_ctiles + 255) / 256, 256, 0, ctx->stream>>>(P);
-  ctx->launches += 3;
-  return check_cuda(ctx, cudaGetLastError(), "flatten kernels launch");
+  ctx->launches += 2;
+  const int st = check_cuda(ctx, cudaGetLastError(), "flatten kernels launch");
+  return st != DPHY_OK ? st : launch_flatten_finish(ctx, P);
 }
 
 // grid = (slices, jobs): job blockIdx.y copied by its slices in 16-byte pieces (+ a byte tail)
@@ -458,10 +572,16 @@ int launch_flatten_lists(dphy_ctx* ctx, FlattenParams P, int first_tile, int num
   return check_cuda(ctx, cudaGetLastError(), "flatten kernels launch (lists)");
 }
 
-int launch_flatten_ctiles(dphy_ctx* ctx, const FlattenParams& P) {
+int launch_flatten_finish(dphy_ctx* ctx, const FlattenParams& P) {
+  if (P.num_nodes == 0) return DPHY_OK;
+  const int nst = (P.num_nodes + kScanTile - 1) / kScanTile, G = P.fsw_stride / 4;
+  counts_scan_reduce_kernel<<<dim3(nst, G), kTile, 0, ctx->stream>>>(P);
+  counts_scan_spine_kernel<<<2 * G, kTile, 0, ctx->stream>>>(P, nst);
+  counts_scan_post_kernel<<<dim3(nst, G), kTile, 0, ctx->stream>>>(P);
+  counts_scan_apply_kernel<<<dim3(nst, G), kTile, 0, ctx->stream>>>(P);
   flatten_ctiles_kernel<<<(P.num_ctiles + 255) / 256, 256, 0, ctx->stream>>>(P);
-  ctx->launches += 1;
-  return check_cuda(ctx, cudaGetLastError(), "flatten kernels launch (tile descriptors)");
+  ctx->launches += 5;
+  return check_cuda(ctx, cudaGetLastError(), "flatten kernels launch (state counts, tile descriptors)");
 }
 
 }  // namespace dphy

@@ -445,209 +445,86 @@ __global__ void __launch_bounds__(kTreeThreads) emat_log_G_tree_kernel(const Log
 }
 
 // ---- folded fast path (uniform site rates) ------------------------------------------------------------------------------------------------
-// With no site-rate heterogeneity every term of a branch's delta-lambda is  mu nu q_a(a)  times an integer that depends only
-// on the tree (ForestDev::bw, built once at upload): the kernel never touches the missation / from-state lists, and the
-// delta of a straddling closer is a 4P-term dot product gathered in place (no pre-pass).  The mutation lists are still
-// walked, in list order, for the  sum_m [ d_m (t_m - t_P) + log(mu nu q_from,to) ]  part of calc_branch_log_G
-// (core/phylo_tree_calc.h:185-206).  nsmn and the num_muts tallies do not depend on the evo model nor on times: they come
-// from the general pass that runs once at upload.  One CTA per tile of kLgTile positions, ~40 registers, 8.4 KB of shared
-// memory => 6-8 CTAs per SM keep enough independent loads in flight to cover HBM latency without any staging.
-struct FoldSmem {
-  double dl[kLgTile];
-  double clx[kLgTile + 2];
-  double wsd[kNW * 2];
-  double muq[kMaxPartitions * 4];
-};
-
-__device__ __forceinline__ double block_scan_excl1(double& a, double* wsd) {   // returns the block total; a <- exclusive prefix
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  double ia = a;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const double ua = __shfl_up_sync(0xffffffffu, ia, o);
-    if (lane >= o) ia += ua;
-  }
-  if (lane == 31) wsd[warp] = ia;
-  __syncthreads();
-  double pa = 0.0, ta = 0.0;
-#pragma unroll
-  for (int w = 0; w < kNW; ++w) {          // fixed order: deterministic
-    const double wa = wsd[w];
-    if (w < warp) pa += wa;
-    ta += wa;
-  }
-  a = pa + ia - a;
-  __syncthreads();                         // wsd may be rewritten by the next scan
-  return ta;
-}
-
-// delta-lambda of branch p from its folded weights; the same expression serves the tile's own nodes and the straddlers,
-// so what a closer subtracts is bit-identical to what its opening added
-__device__ __forceinline__ double folded_delta(const int32_t* __restrict__ bw, int stride, const double* muq, int p) {
-  const int4* w4 = reinterpret_cast<const int4*>(bw + (size_t)p * stride);
-  double d = 0.0;
-  for (int k = 0; k < stride; k += 4) {
-    const int4 w = __ldg(w4 + (k >> 2));
-    d += muq[k] * (double)w.x + muq[k + 1] * (double)w.y + muq[k + 2] * (double)w.z + muq[k + 3] * (double)w.w;
-  }
-  return d;
-}
-
-template <int kMinBlocks>
-__global__ void __launch_bounds__(kLgThreads, kMinBlocks) emat_log_G_folded_kernel(const __grid_constant__ LogGParams P) {
-  __shared__ FoldSmem sm;
+// With no site-rate heterogeneity every term of a branch's delta-lambda is  mu nu q_a(a)  times an integer that depends only on
+// the tree, and so is their sum down the path from the root: ForestDev::C, the per-node state counts built at upload.  lambda_i
+// of every node is then one 4P-term dot product, lambda_ref + sum_k mu nu q_a(a) C[q][k], with no dependence between nodes: the
+// tile kernel is a streaming pass with no scan and no closer list.  The mutation lists are still walked, in list order, for the
+// sum_m [ d_m (t_m - t_P) + log(mu nu q_from,to) ]  part of calc_branch_log_G (core/phylo_tree_calc.h:185-206).  nsmn and the
+// num_muts tallies do not depend on the evo model nor on times: they come from the general pass that runs once at upload.
+// One CTA per tile of kLgTile positions (the ctile grid of the general schedule), thread tid owning positions tid and
+// tid + kLgThreads; the per-tile partials are summed per tree in a fixed order, so log G is bit-reproducible.
+// 6 resident CTAs per SM (40 registers, no spills): measured fastest against 4 (64 registers) and 8 (32 registers, with spills)
+__global__ void __launch_bounds__(kLgThreads, 6) emat_log_G_folded_kernel(const __grid_constant__ LogGParams P) {
+  __shared__ double s_muq[kMaxPartitions * 4];
+  __shared__ double s_w[kNW * 2];
   const ForestDev& f = P.f;
   const int tid = threadIdx.x;
   const int tile = blockIdx.x;
   const int4 ct = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile));
-  const int4 cl = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile) + 2);
-  const int tile_start = ct.x, n_act = ct.y, node_base = ct.z;
+  const int tile_start = ct.x, n_act = ct.y;
   const SitesDev& S = f.sites[ct.w];
-  const int stride = f.fsw_stride;
-  if (tid < kMaxPartitions * 4) sm.muq[tid] = S.tab_muq[tid];
-  // the first chunk of the tile's closer slice does not depend on anything else: get it in flight together with the node records
-  const int32_t* __restrict__ post = f.post_node + node_base;
-  int pre_post[2] = {-1, -1};
-#pragma unroll
-  for (int u = 0; u < 2; ++u) { const int j = cl.z + 2 * tid + u; if (j < cl.w) pre_post[u] = __ldg(post + j); }
-  __syncthreads();
-
-  // ---- node records: 2 consecutive positions per thread ------------------------------------------------------------------------------
-  // (a packed 48-byte per-node record -- parent, depth, list range, t, the parent's t and the weights in three 16-byte loads, no
-  // dependent gather -- was built and measured: 95-99 vs 92 us in stream; the scalar SoA loads below are not the limiter)
-  const int q0 = 2 * tid, p0 = tile_start + q0;
-  const bool act0 = q0 < n_act, act1 = q0 + 1 < n_act;
-  int dep[2] = {0, 0};
-  bool nonroot[2] = {false, false};
-  double len[2] = {0.0, 0.0}, d[2] = {0.0, 0.0}, g[2] = {0.0, 0.0};
-  int par[2] = {-1, -1}, moff[2] = {0, 0}, mcnt[2] = {0, 0};
-  double tN[2] = {0.0, 0.0}, tP[2] = {0.0, 0.0};
-  if (act0) {
-    par[0] = __ldg(f.parent_pos + p0); dep[0] = __ldg(f.depth + p0); tN[0] = f.t[p0];
-    moff[0] = __ldg(f.mut_off + p0); mcnt[0] = __ldg(f.mut_off + p0 + 1) - moff[0];
-    d[0] = folded_delta(f.bw, stride, sm.muq, p0);
-  }
-  if (act1) {
-    par[1] = __ldg(f.parent_pos + p0 + 1); dep[1] = __ldg(f.depth + p0 + 1); tN[1] = f.t[p0 + 1];
-    moff[1] = moff[0] + mcnt[0]; mcnt[1] = __ldg(f.mut_off + p0 + 2) - moff[1];
-    d[1] = folded_delta(f.bw, stride, sm.muq, p0 + 1);
-  }
-#pragma unroll
-  for (int k = 0; k < 2; ++k) if (par[k] >= 0) tP[k] = f.t[par[k]];
-  // ---- mutations (list order): g_node = sum_m [d_m t_m + log(mu nu q_from,to)] - t_P sum_m d_m ---------------------------------------
-#pragma unroll
-  for (int k = 0; k < 2; ++k) {
-    if (par[k] >= 0) {       // the root's list ("mutations" above the root) is not part of log G
-      double es = 0.0, ds = 0.0;
-      for (int i = moff[k]; i < moff[k] + mcnt[k]; ++i) {
-        const int code = __ldg(f.mut_code + i) & 63;
-        const double dd = __ldg(S.tab_md + code);
-        es += dd * f.mut_t[i] + __ldg(S.tab_lq + code);
-        ds += dd;
-      }
-      g[k] = es - tP[k] * ds;
-      len[k] = tN[k] - tP[k];
-      nonroot[k] = true;
-    }
-  }
-
-  // ---- D = inclusive prefix of the deltas over the tile's positions ----------------------------------------------------------------------
-  sm.dl[q0] = d[0]; sm.dl[q0 + 1] = d[1];
-  double D0, D1;
-  {
-    double a = d[0] + d[1];
-    block_scan_excl1(a, sm.wsd);            // its barriers also publish dl to the whole CTA
-    D0 = a + d[0]; D1 = D0 + d[1];
-  }
-
-  // ---- closers: prefix over the tile's slice of the post-order list, gathered at c(q) = q - depth[q] ----------------------------------
-  double CL0 = 0.0, CL1 = 0.0;
-  {
-    const int cl0 = cl.z, cl1 = cl.w;
-    const int q_first = tile_start - node_base;
-    const int myc0 = act0 ? (q_first + q0) - dep[0] : cl0, myc1 = act1 ? (q_first + q0 + 1) - dep[1] : cl0;
-    double carry = 0.0;
-    for (int c0 = cl0; c0 < cl1; c0 += kLgTile) {
-      double a[2] = {0.0, 0.0};
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        const int j = c0 + 2 * tid + u;
-        if (j < cl1) {
-          const int p = c0 == cl0 ? pre_post[u] : __ldg(post + j);
-          const int qa = p - tile_start;
-          a[u] = qa >= 0 ? sm.dl[qa] : folded_delta(f.bw, stride, sm.muq, p);   // straddler: opened in an earlier tile
-        }
-      }
-      double sa = a[0] + a[1];
-      const double ta = block_scan_excl1(sa, sm.wsd);
-      sm.clx[2 * tid] = carry + sa; sm.clx[2 * tid + 1] = carry + sa + a[0];
-      carry += ta;
-      if (tid == 0) sm.clx[kLgTile] = carry;
-      __syncthreads();
-      if (myc0 > c0 && myc0 <= c0 + kLgTile) CL0 = sm.clx[myc0 - c0];
-      if (myc1 > c0 && myc1 <= c0 + kLgTile) CL1 = sm.clx[myc1 - c0];
-      __syncthreads();
-    }
-  }
-
-  // ---- tile-local lambda_i (device order); per-tile partial sums ---------------------------------------------------------------------------
+  const int G = f.fsw_stride / 4;
+  if (tid < kMaxPartitions * 4) s_muq[tid] = S.tab_muq[tid];
   const double lambda_ref = __ldg(S.cumQ + S.L);
+  __syncthreads();
   double contrib = 0.0, tcontrib = 0.0;
-  if (act0) {
-    const double loc = D0 - CL0, lam = lambda_ref + loc;       // + the tile's prefix (tile_agg after pass 2)
-    P.lambda_out[p0] = lam;
-    if (q0 == n_act - 1) P.tile_agg[tile] = loc;
-    if (nonroot[0]) { contrib += -lam * len[0] + g[0]; tcontrib += len[0]; }
-  }
-  if (act1) {
-    const double loc = D1 - CL1, lam = lambda_ref + loc;
-    P.lambda_out[p0 + 1] = lam;
-    if (q0 + 1 == n_act - 1) P.tile_agg[tile] = loc;
-    if (nonroot[1]) { contrib += -lam * len[1] + g[1]; tcontrib += len[1]; }
-  }
-  {
-    const int lane = tid & 31, warp = tid >> 5;
-    contrib = warp_sum(contrib); tcontrib = warp_sum(tcontrib);
-    if (lane == 0) { sm.wsd[warp * 2 + 0] = contrib; sm.wsd[warp * 2 + 1] = tcontrib; }
-    __syncthreads();
-    if (warp == 0) {
-      double a = lane < kNW ? sm.wsd[lane * 2 + 0] : 0.0;
-      double b = lane < kNW ? sm.wsd[lane * 2 + 1] : 0.0;
-      a = warp_sum(a); b = warp_sum(b);
-      if (lane == 0) { P.tile_part[tile * 2 + 0] = a; P.tile_part[tile * 2 + 1] = b; }
+#pragma unroll
+  for (int u = 0; u < kLgNPT; ++u) {
+    const int q = u * kLgThreads + tid, p = tile_start + q;
+    if (q < n_act) {
+      const int par = __ldg(f.parent_pos + p);
+      const double tN = __ldg(f.t + p);
+      const int m0 = __ldg(f.mut_off + p), m1 = __ldg(f.mut_off + p + 1);
+      const uint4* c4 = reinterpret_cast<const uint4*>(f.C) + (size_t)p * G;
+      double dot = 0.0;
+      for (int k = 0; k < G; ++k) {
+        const int4 w = __ldg(reinterpret_cast<const int4*>(c4 + k));
+        dot += s_muq[4 * k] * (double)w.x + s_muq[4 * k + 1] * (double)w.y + s_muq[4 * k + 2] * (double)w.z + s_muq[4 * k + 3] * (double)w.w;
+      }
+      const double lam = lambda_ref + dot;
+      P.lambda_out[p] = lam;
+      if (par >= 0) {        // the root's list ("mutations" above the root) is not part of log G
+        const double tP = __ldg(f.t + par);
+        double es = 0.0, ds = 0.0;
+        for (int i = m0; i < m1; ++i) {
+          const int code = __ldg(f.mut_code + i) & 63;
+          const double dd = __ldg(S.tab_md + code);
+          es += dd * __ldg(f.mut_t + i) + __ldg(S.tab_lq + code);
+          ds += dd;
+        }
+        const double len = tN - tP;
+        contrib += -lam * len + (es - tP * ds);
+        tcontrib += len;
+      }
     }
+  }
+  const int lane = tid & 31, warp = tid >> 5;
+  contrib = warp_sum(contrib); tcontrib = warp_sum(tcontrib);
+  if (lane == 0) { s_w[warp * 2 + 0] = contrib; s_w[warp * 2 + 1] = tcontrib; }
+  __syncthreads();
+  if (warp == 0) {
+    double a = lane < kNW ? s_w[lane * 2 + 0] : 0.0;
+    double b = lane < kNW ? s_w[lane * 2 + 1] : 0.0;
+    a = warp_sum(a); b = warp_sum(b);
+    if (lane == 0) { P.tile_part[tile * 2 + 0] = a; P.tile_part[tile * 2 + 1] = b; }
   }
 }
 
-// pass 2 of the folded path: one CTA per tree -- exclusive scan of the tile aggregates, log G fold, root prior from the root's
-// folded weights (ref_freq + bw[root] is exactly the state count vector of core/phylo_tree_calc.cpp:467-504).
+// pass 2 of the folded path: one CTA per tree -- the tile partials summed in a fixed order, the tile prefixes of lambda_i set to 0
+// (the tile kernel wrote final values; the getter adds the prefix the general schedule leaves there), and the root prior from the
+// root's state counts (ref_freq + C[root] is exactly the state count vector of core/phylo_tree_calc.cpp:467-504).
 __global__ void __launch_bounds__(kTreeThreads) emat_log_G_folded_tree_kernel(const LogGParams P) {
   __shared__ double s_wsd[kTreeThreads / 32];
-  __shared__ double s_carry;
   const ForestDev& f = P.f;
   const int tid = threadIdx.x;
   const int tree = blockIdx.x;
   const TreeDev T = f.trees[tree];
   const SitesDev& S = f.sites[T.sites_id];
-  if (tid == 0) s_carry = 0.0;
-  __syncthreads();
   double a1 = 0.0, a2 = 0.0;
-  for (int j0 = 0; j0 < T.num_ctiles; j0 += kTreeThreads) {
-    const int j = T.first_ctile + j0 + tid;
-    const bool ok = j0 + tid < T.num_ctiles;
-    const double v = ok ? P.tile_agg[j] : 0.0;
-    double tot;
-    const double incl = block_scan_incl<double, kTreeThreads>(v, s_wsd, &tot);
-    if (ok) {
-      const double pre = s_carry + (incl - v);          // exclusive prefix of this tile
-      P.tile_agg[j] = pre;
-      const double A1 = P.tile_part[j * 2 + 0], A2 = P.tile_part[j * 2 + 1];
-      a1 += A1 - pre * A2;                              // sum over the tile of -(lambda_local + pre) len + g
-      a2 += A2;
-    }
-    __syncthreads();
-    if (tid == 0) s_carry += tot;
-    __syncthreads();
+  for (int j = T.first_ctile + tid; j < T.first_ctile + T.num_ctiles; j += kTreeThreads) {
+    a1 += P.tile_part[j * 2 + 0];
+    a2 += P.tile_part[j * 2 + 1];
+    P.tile_agg[j] = 0.0;
   }
   a1 = block_sum<double, kTreeThreads>(a1, s_wsd);
   a2 = block_sum<double, kTreeThreads>(a2, s_wsd);
@@ -655,13 +532,13 @@ __global__ void __launch_bounds__(kTreeThreads) emat_log_G_folded_tree_kernel(co
     P.tree_out[tree * 4 + 1] = a1;
     P.tree_out[tree * 4 + 2] = a2;
     P.tree_out[tree * 4 + 3] = S.cumQ[S.L] + 0.0;
-    const int32_t* wr = f.bw + (size_t)T.node_base * f.fsw_stride;   // the root is the first position of its tree
+    const int32_t* cr = f.C + (size_t)T.node_base * f.fsw_stride;   // the root is the first position of its tree
     double lp = 0.0;
     bool impossible = false;
     for (int b = 0; b < S.P; ++b) {
       for (int a = 0; a < 4; ++a) {
         const double pi = S.pi[b * 4 + a];
-        const int c = S.ref_freq[b * 4 + a] + wr[b * 4 + a];
+        const int c = S.ref_freq[b * 4 + a] + cr[b * 4 + a];
         if (pi != 0.0) lp += c * log(pi);
         else if (c != 0) impossible = true;
       }
@@ -751,20 +628,11 @@ static int launch_log_G_folded(dphy_ctx* ctx, dphy_forest* fo) {
   P.tile_agg = fo->d_tile_agg;
   P.tile_part = fo->d_tile_part;
   P.tree_out = fo->d_tree_out;
-  // resident CTAs per SM: 6 (40 registers) by default -- measured fastest (the kernel is latency-bound); DPHY_FOLDED_OCC = 4 / 5
-  // selects the 64- / 48-register builds (tuning knob)
-  static const int occ = [] { const char* e = getenv("DPHY_FOLDED_OCC"); return e ? atoi(e) : 6; }();
-  // (a variant that gave each CTA two tiles -- 4 positions per thread, in-CTA closers across the pair -- was measured slower,
-  // 110 vs 92 us: its 64 registers halve the resident warps, and the kernel lives on warps in flight, not on bytes per CTA)
   const int grid = fo->h.num_ctiles;
   // profiling only: DPHY_FOLDED_REPEAT=n launches the tile kernel n times per evaluation (idempotent), to separate its in-stream
-  // duration (84 us) from launch gaps and the per-tree kernel (8 us); ncu's isolated, cache-flushed replay reports 59 us
+  // duration from launch gaps and the per-tree kernel
   static const int repeat = [] { const char* e = getenv("DPHY_FOLDED_REPEAT"); return e ? std::max(1, atoi(e)) : 1; }();
-  for (int rep = 0; rep < repeat; ++rep) {
-    if (occ == 4) emat_log_G_folded_kernel<4><<<grid, kLgThreads, 0, ctx->stream>>>(P);
-    else if (occ == 5) emat_log_G_folded_kernel<5><<<grid, kLgThreads, 0, ctx->stream>>>(P);
-    else emat_log_G_folded_kernel<6><<<grid, kLgThreads, 0, ctx->stream>>>(P);
-  }
+  for (int rep = 0; rep < repeat; ++rep) emat_log_G_folded_kernel<<<grid, kLgThreads, 0, ctx->stream>>>(P);
   // one CTA per tree folds the tile partials (fusing this into the tile kernel with a last-CTA ticket was measured slower:
   // every CTA then waits a device-wide atomic round trip before it can retire -- 102 vs 96 us per evaluation)
   emat_log_G_folded_tree_kernel<<<fo->h.num_trees, kTreeThreads, 0, ctx->stream>>>(P);

@@ -1,4 +1,4 @@
-"""Folded log-G timing (back-to-back evaluations between two events).  usage: DPHY_FOLDED_OCC=4|5|6 python tools/logg_occ.py [chains] [cfg]"""
+"""Folded log-G timing (back-to-back evaluations between two events).  usage: python tools/logg_occ.py [chains] [cfg]"""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -20,4 +20,4 @@ for path in ("auto", "general"):
     a.record(st); t0 = time.perf_counter()
     for _ in range(200): fo.eval_log_G()
     t1 = time.perf_counter(); b.record(st); ctx.synchronize()
-    print(f"occ={os.environ.get('DPHY_FOLDED_OCC','5')} path={path} eval={a.elapsed_time(b)/200*1e3:8.1f} us  host_enqueue={(t1-t0)/200*1e6:6.1f} us  logG0={fo.log_G()[2][0]:.9f}")
+    print(f"path={path} eval={a.elapsed_time(b)/200*1e3:8.1f} us  host_enqueue={(t1-t0)/200*1e6:6.1f} us  logG0={fo.log_G()[2][0]:.9f}")
