@@ -296,6 +296,7 @@ def lib() -> C.CDLL:
     L.dphy_forest_get_lambda_i.argtypes = [vp, vp, C.c_int32, f64p]
     L.dphy_forest_get_num_sites_missing.argtypes = [vp, vp, C.c_int32, i32p]
     L.dphy_log_G_host.argtypes = [vp, C.POINTER(EmatHost), C.POINTER(SitesHost), f64p, f64p, f64p]
+    L.dphy_forest_log_coalescent_prior.argtypes = [vp, vp, C.c_double, C.c_double, C.c_double, f64p]
     L.dphy_forest_calc_tallies.argtypes = [vp, vp, C.POINTER(Tallies)]
     L.dphy_forest_calc_num_muts_beta_ab.argtypes = [vp, vp, C.c_int32, i32p]
     L.dphy_forest_calc_num_muts_l.argtypes = [vp, vp, C.c_int32, i32p, i32p]
@@ -793,6 +794,18 @@ class Forest:
         arr = (NodeRow * max(n, 1))(*rows)
         nr = None if new_roots is None else np.ascontiguousarray(new_roots, np.int32)
         self.ctx.check(lib().dphy_forest_apply_rows(self.ctx._h, self._h, n, arr, _p(nr, i32p) if nr is not None else None))
+
+    def log_coalescent_prior(self, n0, g, t0=0.0):
+        """dphy_forest_log_coalescent_prior: float64 array [num_trees], the log-density of each tree's node times under the
+        exponential-growth coalescent N(t) = n0 * exp(g * (t - t0)).  Times grow toward the present (a parent is never later than
+        its children), so g > 0 means growth toward the present; n0 is in the unit of the node times, g in its inverse.  Tips add a
+        lineage going back in time, inner nodes (coalescences) remove one; with k lineages on the interval (a, b) between two
+        consecutive events,
+            log P = sum_c -log N(t_c) - sum_(a,b) C(k, 2) * exp(-g (a - t0)) / n0 * (1 - exp(-g (b - a))) / g,
+        the last factor being b - a at g = 0 (evaluated as -expm1(-g (b - a)) / g: no cancellation for tiny |g|)."""
+        out = np.zeros(max(self.num_trees, 1), np.float64)
+        self.ctx.check(lib().dphy_forest_log_coalescent_prior(self.ctx._h, self._h, float(n0), float(g), float(t0), _p(out, f64p)))
+        return out[:self.num_trees]
 
     def tallies(self):
         out = (Tallies * self.num_trees)()

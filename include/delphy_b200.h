@@ -335,6 +335,18 @@ int  dphy_forest_get_num_sites_missing(dphy_ctx* ctx, dphy_forest* forest, int32
 int  dphy_log_G_host(dphy_ctx* ctx, const dphy_emat_host* tree, const dphy_sites_host* sites,
                      double* log_root_prior, double* log_G_below_root, double* lambda_i);
 
+/* ---- coalescent prior ---------------------------------------------------------------------------------------------------------------
+ * Log-density of the node times of EVERY tree of the forest under the coalescent with exponential growth, N(t) = n0 exp(g (t - t0)),
+ * in the time convention of the tree: t grows toward the present (a node is never earlier than its parent), so g > 0 is a population
+ * growing toward the present.  n0 is in the unit of t, g in its inverse.  Tips are sampling events and add a lineage going back in
+ * time; inner nodes are coalescences and remove one.  With k lineages on an interval (a, b) between consecutive events,
+ *   out[k] = sum over inner nodes c of -log N(t_c)  -  sum over intervals of C(k, 2) * exp(-g (a - t0)) / n0 * (1 - exp(-g (b - a))) / g
+ * (the last factor is b - a at g = 0; the device evaluates it as -expm1(-g (b - a)) / g, so tiny |g| loses nothing to cancellation).
+ * Tied times give the same value in any order.  out[num_trees]; DPHY_ERR_INVALID_ARGUMENT unless n0 > 0 and n0, g, t0 are finite.
+ * Synchronous: the node times as they are on the device (after dphy_forest_set_node_times / dphy_forest_apply_rows), one double per
+ * tree back to the host.  Each tree is taken as a whole tree: for the parts of a partitioned tree the value is not that tree's prior. */
+int  dphy_forest_log_coalescent_prior(dphy_ctx* ctx, dphy_forest* forest, double n0, double g, double t0, double* out);
+
 /* ---- tallies ------------------------------------------------------------------------------------------ */
 /* calc_num_muts / _ab / calc_T + the log-G pieces for every tree; out[num_trees]. */
 int  dphy_forest_calc_tallies(dphy_ctx* ctx, dphy_forest* forest, dphy_tallies* out);
