@@ -327,6 +327,8 @@ def lib() -> C.CDLL:
     L.dphy_forest_download_tree.argtypes = [vp, vp, C.c_int32, C.POINTER(EmatHost)]
     L.dphy_forest_place_samples.argtypes = [vp, vp, C.c_int32, C.POINTER(SampleSet), C.c_int32, C.c_int32, C.POINTER(Placement),
                                             C.POINTER(CandidateRegion)]
+    L.dphy_forest_place_dated_samples.argtypes = [vp, vp, C.c_int32, C.POINTER(SampleSet), f64p, C.c_int32, C.c_int32,
+                                                  C.POINTER(Placement), C.POINTER(CandidateRegion)]
     L.dphy_maple_parse.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(vp)]
     L.dphy_maple_get.argtypes = [vp, C.POINTER(MapleView)]
     L.dphy_maple_free.argtypes = [vp]; L.dphy_maple_free.restype = None
@@ -855,11 +857,16 @@ class Forest:
         return tw, nm
 
     # -- placement of new samples
-    def place_samples(self, samples, tree=0, can_change_root=True, max_best=0):
+    def place_samples(self, samples, tree=0, can_change_root=True, max_best=0, t_X=None):
         """dphy_forest_place_samples: maximum-parsimony placement of new sequences on tree `tree`.  `samples` is the dict maple_parse
         returns, or any dict with its six arrays (delta_off / delta_site / delta_to, miss_off / miss_start / miss_end).  Returns a dict of
         numpy arrays: min_muts, num_best, branch, mut_idx (one entry per sample) and best, a [S, max_best] REGION_DTYPE array of the
-        first max_best best regions in the study's emission order (unused slots: branch == -1)."""
+        first max_best best regions in the study's emission order (unused slots: branch == -1).
+
+        t_X: None places without a date limit.  Otherwise one float64 per sample, its date limit, in the tree's time unit
+        (dphy_forest_place_dated_samples): only regions starting before t_X count, and t_max is clipped to t_X.  For a sample known
+        by a date range, pass the end you want to hold it to -- usually maple_parse(...)["t_max"], the latest time it could have
+        been taken; the library does not choose."""
         a = dict(delta_off=np.ascontiguousarray(samples["delta_off"], np.int32), delta_site=np.ascontiguousarray(samples["delta_site"], np.int32),
                  delta_to=np.ascontiguousarray(samples["delta_to"], np.uint8), miss_off=np.ascontiguousarray(samples["miss_off"], np.int32),
                  miss_start=np.ascontiguousarray(samples["miss_start"], np.int32), miss_end=np.ascontiguousarray(samples["miss_end"], np.int32))
@@ -870,8 +877,16 @@ class Forest:
                        _p(a["miss_start"], i32p), _p(a["miss_end"], i32p))
         out = np.zeros(max(S, 1), PLACEMENT_DTYPE)
         best = np.zeros((max(S, 1), max_best), REGION_DTYPE)
-        self.ctx.check(lib().dphy_forest_place_samples(self.ctx._h, self._h, tree, C.byref(ss), int(bool(can_change_root)), max_best,
-                                                       _p(out, C.POINTER(Placement)), _p(best, C.POINTER(CandidateRegion)) if max_best > 0 else None))
+        outs = (_p(out, C.POINTER(Placement)), _p(best, C.POINTER(CandidateRegion)) if max_best > 0 else None)
+        if t_X is None:
+            self.ctx.check(lib().dphy_forest_place_samples(self.ctx._h, self._h, tree, C.byref(ss), int(bool(can_change_root)), max_best,
+                                                           *outs))
+        else:
+            tx = np.ascontiguousarray(t_X, np.float64)
+            if tx.shape != (S,):
+                raise ValueError("place_samples: t_X must hold one value per sample")
+            self.ctx.check(lib().dphy_forest_place_dated_samples(self.ctx._h, self._h, tree, C.byref(ss), _p(tx, f64p),
+                                                                 int(bool(can_change_root)), max_best, *outs))
         return dict(min_muts=out["min_muts"][:S].copy(), num_best=out["num_best"][:S].copy(), branch=out["branch"][:S].copy(),
                     mut_idx=out["mut_idx"][:S].copy(), best=best[:S])
 

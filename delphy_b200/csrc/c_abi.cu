@@ -1010,6 +1010,9 @@ int dphy_forest_set_node_times(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, int
   if (ctx) dphy_ctx_join_side_streams(ctx);        // the tail of an SPR batch may still be reading the node times
   if (!ctx || !fo || tree < 0 || tree >= fo->h.num_trees || count < 0 || (count > 0 && (!nodes || !t))) return DPHY_ERR_INVALID_ARGUMENT;
   if (count == 0) return DPHY_OK;
+  // the tree's dated placement index is stale from here on, also when the checks below fail after some times were written
+  if (fo->times_version.size() != fo->trees.size()) fo->times_version.assign(fo->trees.size(), 0);
+  ++fo->times_version[tree];
   cudaSetDevice(ctx->device);
   const size_t mark = ctx->arena.mark();
   int32_t* d_nodes = (int32_t*)ctx->arena.alloc(sizeof(int32_t) * count);

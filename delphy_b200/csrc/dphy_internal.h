@@ -190,6 +190,18 @@ struct PlaceIndex {
   int2* seg = nullptr;                     // [2 P2] (min, count) segment tree over Hr, leaves at P2 + region
   size_t bytes = 0;                        // resident bytes
   std::vector<int32_t> h_site_off;         // host copy of site_off (scratch bounds per sample)
+  // dated part (dphy_forest_place_dated_samples): a merge-sort tree over region index, keyed by the regions' t_min.  Built by the
+  // first dated call that drops a region; it depends on the node and mutation times, so it is rebuilt (in the same block) once
+  // dphy_forest_set_node_times has bumped the tree's times version.
+  int32_t lg = 0;                          // log2 P2: levels s = 1..lg of the merge-sort tree (level 0 is the segment tree's leaves)
+  double* tkey = nullptr;                  // [R] the regions' t_min, ascending (stable: ties by region index); null until first built
+  int32_t* lc = nullptr;                   // [lg][P2] level s, entry i of node [a, a + 2^s): how many of its first i - a + 1 entries
+                                           // (in t_min order) come from its left child
+  int2* pre = nullptr;                     // [lg][P2] level s, entry i: (min Hr, count) over the node's first i - a + 1 entries
+  size_t dated_bytes = 0;                  // resident bytes of the dated part
+  uint64_t dated_at = ~0ull;               // times version the dated part was built at (~0: not valid)
+  uint64_t max_at = ~0ull;                 // times version max_key was computed at (~0: not known)
+  double max_key = 0.0;                    // the largest t_min: a t_X above it drops no region
 };
 
 }  // namespace dphy
@@ -288,6 +300,10 @@ struct dphy_forest {
   // study-independent tables of the event-scan SPR path (kernels_spr_group2.cuh), built by the first grouped batch on this forest
   int32_t* d_spr_eopen = nullptr; int32_t* d_spr_tnode = nullptr; int32_t* d_spr_ev = nullptr;
   std::vector<dphy::PlaceIndex> place;   // per tree: the placement index (kernels_place.cu), empty until the first placement
+  // per tree: bumped by every dphy_forest_set_node_times that gets past argument checks (empty: all 0); the dated placement index
+  // compares it with the version it was built at
+  std::vector<uint64_t> times_version;
+  uint64_t tree_times_version(int tree) const { return (size_t)tree < times_version.size() ? times_version[tree] : 0; }
   bool evaluated = false;
   bool struct_valid = false;    // nsmn / num_muts tallies (structure-only outputs of the general log-G pass) are current
   uint32_t epoch = 0;           // look-back flag value of the current launch (flag == epoch means "published")

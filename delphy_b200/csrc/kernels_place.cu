@@ -17,12 +17,23 @@
 // Hr is study-independent: it lives in a min / count segment tree next to a site-sorted table of the mutations' region ranges (the
 // per-tree index, built once per forest).  A sample's correction is piecewise constant between the 2|A| range endpoints: sort them,
 // sweep, and ask the segment tree for (min, count) per piece -- O(|A| log R) per sample instead of O(R + L).
+//
+// Dated placement (remove_regions_in_Xs_future with a per-sample t_X, core/spr_study.cpp:211-224) keeps the regions with
+// t_min < t_X: the first K = #{t_min < t_X} regions in (t_min, region) order.  A sample with K == R runs the path above unchanged;
+// one with K < R asks the same per-piece questions restricted to the kept regions, of the dated part of the index: a merge-sort tree
+// over region index whose nodes list their regions in t_min order, with prefix (min, count) of Hr and fractional-cascading left
+// counts, so that a range query or a restricted find-first is still O(log R).
 #include "dphy_internal.h"
 #include "device_utils.cuh"
+
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 #include <algorithm>
 #include <cfloat>
 #include <climits>
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -93,6 +104,142 @@ __device__ __forceinline__ int seg_find_first(const int2* __restrict__ seg, int 
   return v - P2;
 }
 
+// ---- dated part: merge-sort tree over region index, entries of every node in t_min order -----------------------------------------------
+// The node of level s at [a, a + 2^s) keeps its entries at [a, a + 2^s) of the level's tables.  With K = #{regions: t_min < t_X} the
+// kept regions are the first K in t_min order, so the kept entries of every node are a prefix of its list; its length k is carried
+// from the root (k = K) to the children through lc in O(1) per level.
+struct DatedView { const int2* seg; const int32_t* lc; const int2* pre; int32_t P2; };
+
+// (min Hr, count) over the first k entries of node (s, a)
+__device__ __forceinline__ int2 dated_node(const DatedView& D, int s, int a, int k) {
+  if (k <= 0) return make_int2(INT_MAX, 0);
+  if (s == 0) return __ldg(D.seg + D.P2 + a);
+  return __ldg(D.pre + (size_t)(s - 1) * D.P2 + a + k - 1);
+}
+// how many of the first k entries of node (s >= 1, a) come from its left child
+__device__ __forceinline__ int dated_left(const DatedView& D, int s, int a, int k) {
+  return k > 0 ? __ldg(D.lc + (size_t)(s - 1) * D.P2 + a + k - 1) : 0;
+}
+
+// (min, count) of Hr over the kept regions of [l, r), l < r: descend to the node where [l, r) splits, then walk its two boundary paths
+__device__ int2 dated_query(const DatedView& D, int lg, int K, int l, int r) {
+  int s = lg, a = 0, k = K;
+  for (;;) {
+    if (k == 0) return make_int2(INT_MAX, 0);
+    if (l == a && r == a + (1 << s)) return dated_node(D, s, a, k);
+    const int h = 1 << (s - 1), kl = dated_left(D, s, a, k);
+    if (r <= a + h) { --s; k = kl; }
+    else if (l >= a + h) { --s; a += h; k -= kl; }
+    else break;
+  }
+  const int h = 1 << (s - 1), kl = dated_left(D, s, a, k);
+  int2 acc = make_int2(INT_MAX, 0);
+  for (int ss = s - 1, aa = a, kk = kl; kk > 0;) {              // [l, aa + 2^ss) in node (ss, aa)
+    if (l == aa) { acc = seg_comb(acc, dated_node(D, ss, aa, kk)); break; }
+    const int hh = 1 << (ss - 1), kkl = dated_left(D, ss, aa, kk);
+    if (l < aa + hh) { acc = seg_comb(acc, dated_node(D, ss - 1, aa + hh, kk - kkl)); kk = kkl; }
+    else { aa += hh; kk -= kkl; }
+    --ss;
+  }
+  for (int ss = s - 1, aa = a + h, kk = k - kl; kk > 0;) {      // [aa, r) in node (ss, aa)
+    if (r == aa + (1 << ss)) { acc = seg_comb(acc, dated_node(D, ss, aa, kk)); break; }
+    const int hh = 1 << (ss - 1), kkl = dated_left(D, ss, aa, kk);
+    if (r > aa + hh) { acc = seg_comb(acc, dated_node(D, ss - 1, aa, kkl)); aa += hh; kk -= kkl; }
+    else kk = kkl;
+    --ss;
+  }
+  return acc;
+}
+
+// first kept region at or after l whose Hr is <= target (seg_find_first restricted to the kept regions): on the path from the root
+// to leaf l, the deepest right sibling holding such a region is the nearest; descend from it to its leftmost one
+__device__ int dated_find_first(const DatedView& D, int lg, int K, int l, int target) {
+  int s = lg, a = 0, k = K, cs = -1, ca = 0, ck = 0;
+  while (s > 0 && k > 0) {
+    const int h = 1 << (s - 1), kl = dated_left(D, s, a, k);
+    if (l < a + h) {
+      if (k > kl && dated_node(D, s - 1, a + h, k - kl).x <= target) { cs = s - 1; ca = a + h; ck = k - kl; }
+      k = kl;
+    } else { a += h; k -= kl; }
+    --s;
+  }
+  if (s == 0 && k > 0 && __ldg(D.seg + D.P2 + a).x <= target) return a;
+  if (cs < 0) return -1;
+  for (s = cs, a = ca, k = ck; s > 0; --s) {
+    const int kl = dated_left(D, s, a, k);
+    if (dated_node(D, s - 1, a, kl).x <= target) k = kl;
+    else { a += 1 << (s - 1); k -= kl; }
+  }
+  return a;
+}
+
+// ---- dated part: build ------------------------------------------------------------------------------------------------------------------
+// the key of every region (remove_regions_in_Xs_future compares it with t_X): -DBL_MAX for the root region, t[parent] for (v, 0),
+// mut_t[j - 1] for (v, j); one thread per node
+__global__ void place_tkey_kernel(ForestDev f, int nb, int N, double* __restrict__ key, int32_t* __restrict__ idx) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  if (i == 0) { key[0] = -DBL_MAX; idx[0] = 0; return; }
+  const int p = nb + i, b = region_base(f, nb, p), m0 = f.mut_off[p], n = f.mut_off[p + 1] - m0;
+  key[b] = f.t[f.parent_pos[p]]; idx[b] = b;
+  for (int j = 1; j <= n; ++j) { key[b + j] = f.mut_t[m0 + j - 1]; idx[b + j] = b + j; }
+}
+
+// doubles as monotone unsigned integers (atomicMax of the largest key)
+__device__ __forceinline__ unsigned long long ordered_bits(double x) {
+  const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+  return (u >> 63) ? ~u : u | (1ull << 63);
+}
+__global__ void place_tkey_max_kernel(ForestDev f, int nb, int N, unsigned long long* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  unsigned long long m = ordered_bits(-DBL_MAX);
+  if (i > 0 && i < N) {
+    const int p = nb + i;
+    m = max(m, ordered_bits(f.t[f.parent_pos[p]]));
+    for (int j = f.mut_off[p]; j < f.mut_off[p + 1]; ++j) m = max(m, ordered_bits(f.mut_t[j]));
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(out, m);
+}
+
+__global__ void place_pad_list_kernel(int32_t* __restrict__ list, int R, int P2) {
+  const int i = R + blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < P2) list[i] = i;                 // padding regions rank after every region and are never kept
+}
+
+struct DatedAcc { int lc, m, c; };
+struct DatedComb {
+  __device__ __forceinline__ DatedAcc operator()(const DatedAcc& a, const DatedAcc& b) const {
+    const int m = min(a.m, b.m);
+    return DatedAcc{a.lc + b.lc, m, (a.m == m ? a.c : 0) + (b.m == m ? b.c : 0)};
+  }
+};
+struct SameNode {                          // scan keys are list positions; a node of level s is an aligned run of 2^s of them
+  int s;
+  __device__ __forceinline__ bool operator()(int a, int b) const { return (a >> s) == (b >> s); }
+};
+// level s: entry i of the level's list -> (comes from the left child, Hr, 1); padding leaves are (INT_MAX, 0) and never win
+__global__ void place_dated_vals_kernel(const int32_t* __restrict__ list, const int2* __restrict__ seg, int P2, int s,
+                                        DatedAcc* __restrict__ vals) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P2) return;
+  const int r = list[i];
+  const int2 q = seg[P2 + r];
+  vals[i] = DatedAcc{((r >> (s - 1)) & 1) ^ 1, q.x, q.y};
+}
+// the scanned level: its two tables, and its list stably partitioned into the lists of its children (the next level's list)
+__global__ void place_dated_level_kernel(const int32_t* __restrict__ list, const DatedAcc* __restrict__ acc, int P2, int s,
+                                         int32_t* __restrict__ lc, int2* __restrict__ pre, int32_t* __restrict__ next) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P2) return;
+  const DatedAcc v = acc[i];
+  lc[i] = v.lc;
+  pre[i] = make_int2(v.m, v.c);
+  const int r = list[i], a = i & ~((1 << s) - 1), h = 1 << (s - 1);
+  next[((r >> (s - 1)) & 1) ? a + h + (i - a) - v.lc : a + v.lc - 1] = r;
+}
+
 // ---- stable warp-level LSD radix sort of (key, value) pairs in global scratch -----------------------------------------------------------
 // Sorts n pairs by key bits [0, bits), ping-ponging between (k0, v0) and (k1, v1); returns true if the result is in (k1, v1).  Equal
 // keys keep their order (a chunk of 32 is scattered in lane order: rank among the lanes of the same digit).
@@ -140,8 +287,11 @@ __device__ __forceinline__ int warp_min(int v) {
 
 struct PlaceParams {
   ForestDev f;
-  int32_t nb, N, R, P2, L, site_bits, pos_bits, can_change_root, max_best, s0, s1, pad;
+  int32_t nb, N, R, P2, L, site_bits, pos_bits, can_change_root, max_best, s0, s1, lg;
   const int32_t* site_off; const int4* rec; const int2* seg; const uint8_t* ref;
+  const double* t_X;             // [S] date limits (null: undated call)
+  const double* tkey;            // the dated part (null: not needed by this call, every K == R) ...
+  const int32_t* lc; const int2* pre;
   const int32_t* delta_off; const int32_t* delta_site; const uint8_t* delta_to;
   const int32_t* miss_off; const int32_t* miss_start; const int32_t* miss_end;
   const int64_t* scr_off;        // [S + 1] words of scratch per sample (prefix); a batch uses scratch + scr_off[k] - scr_off[s0]
@@ -151,7 +301,7 @@ struct PlaceParams {
 };
 
 // region index -> (device position, mut_idx) and the record the study would emit for it
-__device__ __forceinline__ dphy_candidate_region place_region_record(const PlaceParams& P, int r) {
+__device__ __forceinline__ dphy_candidate_region place_region_record(const PlaceParams& P, int r, double tX) {
   const ForestDev& f = P.f;
   dphy_candidate_region c;
   if (r == 0) {
@@ -164,8 +314,17 @@ __device__ __forceinline__ dphy_candidate_region place_region_record(const Place
     c.t_min = j == 0 ? f.t[f.parent_pos[lo]] : f.mut_t[m0 + j - 1];
     c.t_max = j == n ? f.t[lo] : f.mut_t[m0 + j];
   }
+  if (P.t_X && c.t_max > tX) c.t_max = tX;
   c.min_muts = 0; c.pad_ = 0; c.log_W_over_Wmax = 0.0; c.W_over_Wmax = 0.0;
   return c;
+}
+
+// K == R (nothing dropped): the undated segment tree
+__device__ __forceinline__ int2 place_query(const PlaceParams& P, int K, int l, int r) {
+  return K == P.R ? seg_query(P.seg, P.P2, l, r) : dated_query(DatedView{P.seg, P.lc, P.pre, P.P2}, P.lg, K, l, r);
+}
+__device__ __forceinline__ int place_find_first(const PlaceParams& P, int K, int l, int target) {
+  return K == P.R ? seg_find_first(P.seg, P.P2, l, target) : dated_find_first(DatedView{P.seg, P.lc, P.pre, P.P2}, P.lg, K, l, target);
 }
 
 constexpr int kPlaceWarps = 8;
@@ -258,7 +417,15 @@ __global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(Plac
   const uint32_t* ks = ealt ? ek1 : ek0;
   const uint32_t* vs = ealt ? ev1 : ev0;
 
-  // (4) sweep: piece j in [-1, n) is [pos_j, pos_{j+1}) (pos_{-1} = first region, pos_n = R) with correction = prefix of c up to j
+  // (4) sweep: piece j in [-1, n) is [pos_j, pos_{j+1}) (pos_{-1} = first region, pos_n = R) with correction = prefix of c up to j;
+  // with a date limit only the regions with t_min < t_X count: the first K in t_min order
+  const double tX = P.t_X ? P.t_X[k] : DBL_MAX;
+  int K = P.R;
+  if (P.tkey) {
+    int lo = 0, hi = P.R;
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (__ldg(P.tkey + mid) < tX) lo = mid + 1; else hi = mid; }
+    K = lo;
+  }
   const int start0 = P.can_change_root ? 0 : 1;
   int bv = INT_MAX, bc = 0, bl = 0, bm = 0;
   carry = 0;
@@ -269,8 +436,8 @@ __global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(Plac
     carry = __shfl_sync(0xffffffffu, corr, 31);
     if (j < n) {
       const int l = j < 0 ? start0 : max((int)ks[j], start0), r = j + 1 < n ? (int)ks[j + 1] : P.R;
-      if (l < r) {
-        const int2 q = seg_query(P.seg, P.P2, l, r);
+      const int2 q = l < r ? place_query(P, K, l, r) : make_int2(INT_MAX, 0);
+      if (q.y > 0) {                    // a piece without kept regions (only under a date limit) offers nothing
         const int v = q.x + corr;
         if (v < bv) { bv = v; bc = q.y; bl = l; bm = q.x; }
         else if (v == bv) bc += q.y;
@@ -284,14 +451,14 @@ __global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(Plac
   const unsigned owner = __ballot_sync(0xffffffffu, bv == best && bl == first_l && best != INT_MAX);
   if (owner) {
     const int ol = __ffs(owner) - 1;
-    if (lane == ol) first = seg_find_first(P.seg, P.P2, bl, bm);
+    if (lane == ol) first = place_find_first(P, K, bl, bm);
     first = __shfl_sync(0xffffffffu, first, ol);
   }
   if (lane == 0) {
     dphy_placement o;
     o.min_muts = -1; o.num_best = 0; o.branch = -1; o.mut_idx = -1;
     if (first >= 0) {
-      const dphy_candidate_region fr = place_region_record(P, first);
+      const dphy_candidate_region fr = place_region_record(P, first, tX);
       o.min_muts = B + best; o.num_best = count; o.branch = fr.branch; o.mut_idx = fr.mut_idx;
     }
     P.out[k] = o;
@@ -310,14 +477,14 @@ __global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(Plac
     int l = 0, r = 0, hit = 0, m = 0;
     if (j < n) {
       l = j < 0 ? start0 : max((int)ks[j], start0); r = j + 1 < n ? (int)ks[j + 1] : P.R;
-      if (l < r) { const int2 q = seg_query(P.seg, P.P2, l, r); m = q.x; hit = q.x + corr == best ? q.y : 0; }
+      if (l < r) { const int2 q = place_query(P, K, l, r); m = q.x; hit = q.y > 0 && q.x + corr == best ? q.y : 0; }
     }
     const int incl = warp_scan_incl(hit, lane);
     const int off = emitted + incl - hit;
     const int take = off < P.max_best ? min(hit, P.max_best - off) : 0;
     for (int t = 0; t < take; ++t) {
-      const int p = seg_find_first(P.seg, P.P2, l, m);
-      dphy_candidate_region rr = place_region_record(P, p);
+      const int p = place_find_first(P, K, l, m);
+      dphy_candidate_region rr = place_region_record(P, p, tX);
       rr.min_muts = B + best;
       bo[off + t] = rr;
       l = p + 1;
@@ -395,16 +562,103 @@ int ensure_place_index(dphy_ctx* ctx, dphy_forest* fo, int tree) {
   X.h_site_off = std::move(h_so);
   return DPHY_OK;
 }
-}  // namespace
 
-}  // namespace dphy
+// the largest t_min of the tree (a date limit above it drops no region), cached per times version
+int place_max_key(dphy_ctx* ctx, dphy_forest* fo, int tree, uint64_t ver) {
+  PlaceIndex& X = fo->place[tree];
+  if (X.max_at == ver) return DPHY_OK;
+  const TreeDev& T = fo->trees[tree];
+  const size_t mark = ctx->arena.mark();
+  unsigned long long* d_max = (unsigned long long*)ctx->arena.alloc(sizeof(unsigned long long));
+  if (!d_max) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "arena exhausted (place)");
+  unsigned long long h_max = 0;
+  int st = check_cuda(ctx, cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), ctx->stream), "place memset");
+  if (st == DPHY_OK) {
+    place_tkey_max_kernel<<<(T.num_nodes + 255) / 256, 256, 0, ctx->stream>>>(fo->h, T.node_base, T.num_nodes, d_max);
+    ++ctx->launches;
+    st = check_cuda(ctx, cudaGetLastError(), "place_tkey_max_kernel");
+  }
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaMemcpyAsync(&h_max, d_max, sizeof(h_max), cudaMemcpyDeviceToHost, ctx->stream), "D2H");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "place max key");
+  ctx->arena.release(mark);
+  if (st != DPHY_OK) return st;
+  const unsigned long long u = (h_max >> 63) ? h_max & ~(1ull << 63) : ~h_max;
+  std::memcpy(&X.max_key, &u, sizeof(u));
+  X.max_at = ver;
+  return DPHY_OK;
+}
 
-using namespace dphy;
+// The dated part of the index (lc / pre: lg levels x P2 entries, 12 B each; tkey: 8 B per region).  Its block is allocated by the
+// first build and reused by every rebuild (R and P2 do not depend on times).  Level by level from the root: the level's list (the
+// regions of each node in t_min order; the root's is the sorted order itself) is scanned per node for (left-child count, min Hr,
+// count), which gives the level's tables and, by a stable partition on the next bit of the region index, the next level's list.
+int ensure_dated_index(dphy_ctx* ctx, dphy_forest* fo, int tree, uint64_t ver) {
+  PlaceIndex& X = fo->place[tree];
+  if (X.tkey && X.dated_at == ver) return DPHY_OK;
+  const TreeDev& T = fo->trees[tree];
+  const int R = X.R, P2 = X.P2;
+  int lg = 0;
+  while ((1 << lg) < P2) ++lg;
+  size_t sort_bytes = 0, scan_bytes = 0;
+  DPHY_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const double*)nullptr, (double*)nullptr, (const int32_t*)nullptr,
+                                                 (int32_t*)nullptr, R, 0, 64, ctx->stream));
+  DPHY_CUDA(ctx, cub::DeviceScan::InclusiveScanByKey(nullptr, scan_bytes, thrust::counting_iterator<int>(0), (const DatedAcc*)nullptr,
+                                                     (DatedAcc*)nullptr, DatedComb{}, P2, SameNode{1}, ctx->stream));
+  const size_t b_lc = al(sizeof(double) * R), b_pre = b_lc + al(sizeof(int32_t) * (size_t)lg * P2);
+  const size_t total = b_pre + al(sizeof(int2) * (size_t)lg * P2);
+  // temporaries: unsorted keys, region indices, two level lists, scan input and output, CUB's storage
+  const size_t b_idx = al(sizeof(double) * R), b_l0 = b_idx + al(sizeof(int32_t) * R), b_l1 = b_l0 + al(sizeof(int32_t) * P2);
+  const size_t b_vin = b_l1 + al(sizeof(int32_t) * P2), b_vout = b_vin + al(sizeof(DatedAcc) * P2), b_cub = b_vout + al(sizeof(DatedAcc) * P2);
+  const size_t tmp_bytes = b_cub + al(std::max(sort_bytes, scan_bytes));
+  char* d = (char*)X.tkey;
+  const bool fresh = d == nullptr;
+  if (fresh && cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) {
+    cudaGetLastError();
+    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index)");
+  }
+  char* tmp = nullptr;
+  if (cudaMallocAsync((void**)&tmp, tmp_bytes, ctx->stream) != cudaSuccess) {
+    cudaGetLastError();
+    if (fresh) cudaFreeAsync(d, ctx->stream);
+    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index scratch)");
+  }
+  if (fresh) {
+    fo->allocs.push_back(d);
+    fo->bytes += total;
+    X.tkey = (double*)d; X.lc = (int32_t*)(d + b_lc); X.pre = (int2*)(d + b_pre); X.dated_bytes = total; X.lg = lg;
+  }
+  X.dated_at = ~0ull;                       // not valid until the build below has finished
+  double* key = (double*)tmp; int32_t* idx = (int32_t*)(tmp + b_idx);
+  int32_t* list = (int32_t*)(tmp + b_l0); int32_t* next = (int32_t*)(tmp + b_l1);
+  DatedAcc* vin = (DatedAcc*)(tmp + b_vin); DatedAcc* vout = (DatedAcc*)(tmp + b_vout); void* cub_tmp = tmp + b_cub;
+  place_tkey_kernel<<<(T.num_nodes + 255) / 256, 256, 0, ctx->stream>>>(fo->h, T.node_base, T.num_nodes, key, idx);
+  if (P2 > R) place_pad_list_kernel<<<(P2 - R + 255) / 256, 256, 0, ctx->stream>>>(list, R, P2);
+  // every CUB call below is counted as one launch
+  cudaError_t ce = cub::DeviceRadixSort::SortPairs(cub_tmp, sort_bytes, (const double*)key, X.tkey, (const int32_t*)idx, list, R, 0, 64,
+                                                   ctx->stream);
+  ctx->launches += 3;
+  const unsigned blocks = (unsigned)((P2 + 255) / 256);
+  for (int lv = lg; lv >= 1 && ce == cudaSuccess; --lv) {
+    place_dated_vals_kernel<<<blocks, 256, 0, ctx->stream>>>(list, X.seg, P2, lv, vin);
+    ce = cub::DeviceScan::InclusiveScanByKey(cub_tmp, scan_bytes, thrust::counting_iterator<int>(0), (const DatedAcc*)vin, vout,
+                                             DatedComb{}, P2, SameNode{lv}, ctx->stream);
+    if (ce == cudaSuccess)
+      place_dated_level_kernel<<<blocks, 256, 0, ctx->stream>>>(list, vout, P2, lv, X.lc + (size_t)(lv - 1) * P2,
+                                                                 X.pre + (size_t)(lv - 1) * P2, next);
+    std::swap(list, next);
+    ctx->launches += 3;
+  }
+  int st = check_cuda(ctx, ce, "dated place index");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaGetLastError(), "dated place index kernels");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "dated place index build");
+  cudaFreeAsync(tmp, ctx->stream);
+  if (st == DPHY_OK) X.dated_at = ver;
+  return st;
+}
 
-extern "C" {
-
-int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sample_set* set, int32_t can_change_root,
-                              int32_t max_best, dphy_placement* out, dphy_candidate_region* best) {
+// dphy_forest_place_samples (t_X == nullptr, dated == false) and dphy_forest_place_dated_samples
+int place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sample_set* set, const double* t_X, bool dated,
+                  int32_t can_change_root, int32_t max_best, dphy_placement* out, dphy_candidate_region* best) {
   if (!ctx || !fo || !set || max_best < 0 || set->num_samples < 0) return DPHY_ERR_INVALID_ARGUMENT;
   if (tree < 0 || tree >= fo->h.num_trees) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "place: tree index out of range");
   const int S = set->num_samples;
@@ -426,10 +680,27 @@ int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, cons
   for (int64_t i = mof[0]; i < mof[S]; ++i)
     if (set->miss_start[i] < 0 || set->miss_end[i] > L || set->miss_start[i] >= set->miss_end[i])
       return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "place: missing interval out of range");
+  if (dated && !t_X) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: t_X missing");
+  if (dated)
+    for (int k = 0; k < S; ++k)
+      if (std::isnan(t_X[k])) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "place: t_X is NaN");
   cudaSetDevice(ctx->device);
   int st = ensure_place_index(ctx, fo, tree);
   if (st != DPHY_OK) return st;
   const PlaceIndex& X = fo->place[tree];
+  // the dated part is needed once some sample drops a region (t_X <= the largest t_min); a current one is used as it is
+  bool use_dated = false;
+  if (dated) {
+    const uint64_t ver = fo->tree_times_version(tree);
+    use_dated = X.tkey && X.dated_at == ver;
+    if (!use_dated) {
+      st = place_max_key(ctx, fo, tree, ver);
+      if (st != DPHY_OK) return st;
+      for (int k = 0; k < S && !use_dated; ++k) use_dated = t_X[k] <= X.max_key;
+      if (use_dated) st = ensure_dated_index(ctx, fo, tree, ver);
+      if (st != DPHY_OK) return st;
+    }
+  }
   // ---- scratch per sample: endpoint pairs (2 per mutation of A, bounded by the site table's runs), delta and interval pairs; each
   // ping-ponged by the radix sort: 4 words per pair ----
   const int32_t* so = X.h_site_off.data();
@@ -453,7 +724,7 @@ int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, cons
   // ---- inputs through the pinned slab; outputs back through it ----
   const size_t b_doff = 0, b_moff = al(4 * (size_t)(S + 1)), b_ds = b_moff + al(4 * (size_t)(S + 1)), b_dt = b_ds + al(4 * (size_t)D);
   const size_t b_ms = b_dt + al((size_t)D), b_me = b_ms + al(4 * (size_t)I), b_scr = b_me + al(4 * (size_t)I);
-  const size_t in_bytes = b_scr + al(8 * (size_t)(S + 1));
+  const size_t b_tx = b_scr + al(8 * (size_t)(S + 1)), in_bytes = b_tx + (dated ? al(8 * (size_t)S) : 0);
   const size_t b_out = in_bytes, b_best = b_out + al(sizeof(dphy_placement) * (size_t)S);
   const size_t io_bytes = b_best + al(sizeof(dphy_candidate_region) * (size_t)S * max_best);
   const size_t b_scratch = io_bytes, total = b_scratch + al(4 * (size_t)max_words);
@@ -468,12 +739,15 @@ int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, cons
   if (D) { std::memcpy(h + b_ds, set->delta_site + dof[0], 4 * D); std::memcpy(h + b_dt, set->delta_to + dof[0], D); }
   if (I) { std::memcpy(h + b_ms, set->miss_start + mof[0], 4 * I); std::memcpy(h + b_me, set->miss_end + mof[0], 4 * I); }
   std::memcpy(h + b_scr, scr.data(), 8 * (size_t)(S + 1));
+  if (dated) std::memcpy(h + b_tx, t_X, 8 * (size_t)S);
   cudaError_t ce = cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
   PlaceParams P;
   std::memset(&P, 0, sizeof(P));
   P.f = fo->h; P.nb = T.node_base; P.N = T.num_nodes; P.R = X.R; P.P2 = X.P2; P.L = L;
   P.site_bits = bits_for(L); P.pos_bits = bits_for(X.R); P.can_change_root = can_change_root != 0; P.max_best = max_best;
   P.site_off = X.site_off; P.rec = X.rec; P.seg = X.seg; P.ref = fo->sites[T.sites_id]->d_ref;
+  if (dated) P.t_X = (const double*)(d + b_tx);
+  if (use_dated) { P.tkey = X.tkey; P.lc = X.lc; P.pre = X.pre; P.lg = X.lg; }
   P.delta_off = (const int32_t*)(d + b_doff); P.delta_site = (const int32_t*)(d + b_ds); P.delta_to = (const uint8_t*)(d + b_dt);
   P.miss_off = (const int32_t*)(d + b_moff); P.miss_start = (const int32_t*)(d + b_ms); P.miss_end = (const int32_t*)(d + b_me);
   P.scr_off = (const int64_t*)(d + b_scr); P.scratch = (uint32_t*)(d + b_scratch);
@@ -492,6 +766,23 @@ int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, cons
   if (max_best > 0) std::memcpy(best, h + b_best, sizeof(dphy_candidate_region) * (size_t)S * max_best);
   release_pinned_async(ctx);
   return DPHY_OK;
+}
+}  // namespace
+
+}  // namespace dphy
+
+using namespace dphy;
+
+extern "C" {
+
+int dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sample_set* set, int32_t can_change_root,
+                              int32_t max_best, dphy_placement* out, dphy_candidate_region* best) {
+  return place_samples(ctx, fo, tree, set, nullptr, false, can_change_root, max_best, out, best);
+}
+
+int dphy_forest_place_dated_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sample_set* set, const double* t_X,
+                                    int32_t can_change_root, int32_t max_best, dphy_placement* out, dphy_candidate_region* best) {
+  return place_samples(ctx, fo, tree, set, t_X, true, can_change_root, max_best, out, best);
 }
 
 }  // extern "C"

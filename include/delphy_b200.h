@@ -434,8 +434,18 @@ int  dphy_gamma_q_inv(dphy_ctx* ctx, int32_t n, const double* a, const double* q
  * forest (dphy_forest_apply_rows drops it, dphy_forest_set_node_times needs no rebuild: times are read when the records are made);
  * per sample the work is O(|A| log R), A = the tree's mutations at the sample's delta and missing sites, R = the number of regions.
  * Synchronous: host arrays in, host results out.
- * Out of scope: date-constrained placement (dropping the regions with t_min >= t_X, remove_regions_in_Xs_future): with a per-sample
- * t_X the kept regions differ per sample; use dphy_spr_study_batch for it. */
+ * Dated placement, dphy_forest_place_dated_samples: sample k may only go where the tree is earlier than its date limit t_X[k].  Its
+ * regions are those above after remove_regions_in_Xs_future (core/spr_study.cpp:211-224) with t_X = t_X[k]: a region with
+ * t_min >= t_X[k] is dropped (a tie too), and t_max is clipped to t_X[k] where it is larger; the outputs are then as above over the
+ * regions left, bit for bit, best records carrying the clipped t_max.  t_X[k] = +inf or DBL_MAX keeps every region (the undated
+ * result); t_X[k] <= -DBL_MAX keeps none, not even the root region (t_min = -DBL_MAX), and gives min_muts = -1, num_best = 0,
+ * branch = mut_idx = -1.  A sample with a date range passes the end it stands for (usually t_max of dphy_maple_view, the latest
+ * time it could have been taken).  Validation, outputs and precondition as for dphy_forest_place_samples, and before anything is
+ * written: DPHY_ERR_INVALID_ARGUMENT for t_X == NULL with num_samples > 0 or a NaN in it.  Node and mutation times are compared as
+ * numbers (none may be NaN).  Cost: a dated part of the per-tree index, a merge-sort tree over the regions keyed by t_min (12 B per
+ * entry, lg2(P2) levels of P2 entries, P2 = the power of two >= R, plus 8 B per region), is built by the first dated call that
+ * drops a region of the tree and kept with the forest (dphy_forest_device_bytes includes it; dphy_forest_set_node_times marks it
+ * stale and the next such call rebuilds it in the same memory); a sample that drops a region costs O(|A| log R) as well. */
 typedef struct dphy_sample_set {
   int32_t num_samples;
   int32_t reserved;
@@ -449,6 +459,9 @@ typedef struct dphy_placement {
 } dphy_placement;
 int  dphy_forest_place_samples(dphy_ctx* ctx, dphy_forest* forest, int32_t tree, const dphy_sample_set* samples, int32_t can_change_root,
                                int32_t max_best, dphy_placement* out, dphy_candidate_region* best /* [num_samples * max_best] or NULL */);
+int  dphy_forest_place_dated_samples(dphy_ctx* ctx, dphy_forest* forest, int32_t tree, const dphy_sample_set* samples,
+                                     const double* t_X /* [num_samples] */, int32_t can_change_root, int32_t max_best,
+                                     dphy_placement* out, dphy_candidate_region* best /* [num_samples * max_best] or NULL */);
 
 /* ---- tree partitioning (one or more parts per GPU) ------------------------------------------------------------- */
 /* generate_random_partition_stencil (core/tree_partitioning.h:139-194): up to num_parts-1 cut points.  The coin flips are the
