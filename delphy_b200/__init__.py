@@ -329,6 +329,12 @@ def lib() -> C.CDLL:
                                             C.POINTER(CandidateRegion)]
     L.dphy_forest_place_dated_samples.argtypes = [vp, vp, C.c_int32, C.POINTER(SampleSet), f64p, C.c_int32, C.c_int32,
                                                   C.POINTER(Placement), C.POINTER(CandidateRegion)]
+    L.dphy_clade_table_create.argtypes = [vp, C.POINTER(vp)]
+    L.dphy_clade_table_destroy.argtypes = [vp, vp]; L.dphy_clade_table_destroy.restype = None
+    L.dphy_clade_table_add.argtypes = [vp, vp, vp]
+    L.dphy_clade_table_info.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    L.dphy_clade_table_score.argtypes = [vp, vp, vp, f64p]
+    L.dphy_clade_table_node_support.argtypes = [vp, vp, vp, C.c_int32, C.POINTER(C.c_int64), f64p]
     L.dphy_maple_parse.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(vp)]
     L.dphy_maple_get.argtypes = [vp, C.POINTER(MapleView)]
     L.dphy_maple_free.argtypes = [vp]; L.dphy_maple_free.restype = None
@@ -897,6 +903,59 @@ class Forest:
     def close(self):
         if self._h:
             lib().dphy_forest_destroy(self.ctx._h, self._h)
+            self._h = C.c_void_p()
+
+
+class CladeTable:
+    """dphy_clade_table: clade counts and summed clade times over every tree added, for clade support and the maximum clade
+    credibility (MCC) tree.  A clade is the set of tips (nodes with child0 == -1, identified by host node index) below a node; the
+    first add fixes the tip set, and every tree added or scored later must have the same number of nodes and the same tip indices.
+    score(forest)[k] = sum over the nodes v of tree k of log(count(v) / num_trees): the MCC tree is the argmax over the added trees."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        self._h = C.c_void_p()
+        ctx.check(lib().dphy_clade_table_create(ctx._h, C.byref(self._h)))
+
+    def add(self, forest: Forest):
+        """Count every tree of `forest` as it is resident now."""
+        self.ctx.check(lib().dphy_clade_table_add(self.ctx._h, self._h, forest._h))
+
+    def _info(self):
+        v = [C.c_int64() for _ in range(3)]
+        self.ctx.check(lib().dphy_clade_table_info(self._h, *[C.byref(x) for x in v]))
+        return [x.value for x in v]
+
+    @property
+    def num_trees(self):
+        return self._info()[0]
+
+    @property
+    def num_clades(self):
+        return self._info()[1]
+
+    @property
+    def device_bytes(self):
+        return self._info()[2]
+
+    def score(self, forest: Forest):
+        """float64 [num_trees]: sum of log(count / num_trees) over each tree's nodes (-inf where a clade was never added)."""
+        out = np.zeros(max(forest.num_trees, 1), np.float64)
+        self.ctx.check(lib().dphy_clade_table_score(self.ctx._h, self._h, forest._h, _p(out, f64p)))
+        return out[:forest.num_trees]
+
+    def node_support(self, forest: Forest, tree=0):
+        """(count int64 [num_nodes], mean_t float64 [num_nodes]) of tree `tree`, host node order: how many added trees contain each
+        node's clade, and its mean node time over them (0 and NaN for a clade never added)."""
+        n = forest.emats[tree].num_nodes if 0 <= tree < forest.num_trees else 1
+        count, mean_t = np.zeros(max(n, 1), np.int64), np.zeros(max(n, 1), np.float64)
+        self.ctx.check(lib().dphy_clade_table_node_support(self.ctx._h, self._h, forest._h, tree, _p(count, C.POINTER(C.c_int64)),
+                                                           _p(mean_t, f64p)))
+        return count[:n], mean_t[:n]
+
+    def close(self):
+        if self._h:
+            lib().dphy_clade_table_destroy(self.ctx._h, self._h)
             self._h = C.c_void_p()
 
 

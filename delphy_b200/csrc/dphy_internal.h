@@ -204,6 +204,11 @@ struct PlaceIndex {
   double max_key = 0.0;                    // the largest t_min: a t_X above it drops no region
 };
 
+// One distinct clade of a dphy_clade_table (kernels_clade.cu): its 128-bit key (two wrapping u64 sums of per-tip keys, lanes j = 0
+// and 1) and what the trees added so far say about it.  Tables keep keys and values in two arrays sorted by (k0, k1), 32 B a clade.
+struct alignas(16) CladeKey { uint64_t k0, k1; };
+struct alignas(16) CladeVal { int64_t count; double t_sum; };
+
 }  // namespace dphy
 
 struct dphy_ctx {
@@ -314,6 +319,19 @@ struct dphy_forest {
     for (size_t i = 0; i < sites.size(); ++i) if (eval_version[i] != sites[i]->version) return false;
     return true;
   }
+};
+
+// Clade counts over every tree added so far (kernels_clade.cu).  No pointer to a forest is kept: forests may change or go after an add.
+struct dphy_clade_table {
+  dphy_ctx* ctx = nullptr;          // the ctx that made the table (its stream orders every use)
+  int32_t num_nodes = -1;           // N of every tree, fixed by the first add (-1: nothing added yet)
+  int32_t num_tips = 0;             // (N + 1) / 2 for binary trees
+  int64_t num_trees = 0;
+  int64_t num_clades = 0;
+  uint32_t* d_tips = nullptr;       // [(N + 31) / 32] bitmap of the tips' host node indices
+  dphy::CladeKey* d_keys = nullptr; // [num_clades] ascending by (k0, k1), unique
+  dphy::CladeVal* d_vals = nullptr; // [num_clades] (count, sum of the clade's node time), in d_keys's block
+  size_t bytes = 0;                 // resident bytes (bitmap + keys + values)
 };
 
 namespace dphy {

@@ -347,6 +347,40 @@ int  dphy_log_G_host(dphy_ctx* ctx, const dphy_emat_host* tree, const dphy_sites
  * tree back to the host.  Each tree is taken as a whole tree: for the parts of a partitioned tree the value is not that tree's prior. */
 int  dphy_forest_log_coalescent_prior(dphy_ctx* ctx, dphy_forest* forest, double n0, double g, double t0, double* out);
 
+/* ---- clade support and the maximum clade credibility (MCC) tree ----------------------------------------------------------------------
+ * A clade table counts, over every tree added to it, how many trees contain each clade, and sums the clade's node time over them.
+ *   Tips: a tip is a node with child0 == -1, identified by its HOST node index.  The first add fixes the table's tip set: N nodes per
+ *     tree and which indices are tips.  Every tree later added or scored must have the same N and exactly the same tip indices;
+ *     otherwise the call returns DPHY_ERR_INVALID_ARGUMENT before anything is changed.  Tips are not matched by name: renumber first.
+ *   Clades: the clade of node v is the set of tips below it, v included -- tips, inner nodes and the root all have one.  Trees are
+ *     rooted, so a binary tree contains each clade at most once.
+ *   Key: a clade is keyed by 128 bits, two independent wrapping uint64 sums over its tips i of k_j(i) = splitmix64((uint64)i << 1 | j),
+ *     j = 0 and 1, where splitmix64(x): z = x + 0x9e3779b97f4a7c15; z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9;
+ *     z = (z ^ (z >> 27)) * 0x94d049bb133111eb; return z ^ (z >> 31)  (one step of SplitMix64 from state x).  Two different tip sets
+ *     share a key with probability about 2^-128 per pair; such a collision is NOT detected (the two clades would count as one).
+ *   Table: per distinct clade, count = how many of the trees added so far contain it, and the sum of its node time over them.
+ *     T = the number of trees added.  Memory: 32 B per distinct clade plus a bitmap of N bits (dphy_clade_table_info's device_bytes);
+ *     an add also takes stream-ordered scratch of about 90 B per node of the forest plus 64 B per clade of the merged table.
+ *   Score: score(tree) = sum over every node v of log(count(v) / T), the log of the product of clade frequencies TreeAnnotator
+ *     maximises for its MCC tree.  Tips and the root add exactly 0; a tree with a clade the table has never seen scores -inf.
+ *   Node support (one tree, host node order): count(v) (0 for an unseen clade) and mean_t(v) = sum of t / count (NaN if count == 0).
+ *   The MCC tree is the argmax of the scores over the added trees; its node support annotates it (frequency count / T, mean clade time).
+ * Every call is synchronous with host results, and a table is used with the ctx that made it.  dphy_clade_table_add takes every tree of
+ * the forest as it is resident now (after dphy_forest_set_node_times / dphy_forest_apply_rows); the table keeps no pointer to the forest,
+ * so the forest may be edited or destroyed afterwards.  Adding forests one after another gives the counts of one forest holding all
+ * their trees, which is how a posterior larger than HBM is summarised: add every batch, then score every batch.  The same sequence of
+ * adds gives bit-identical mean_t and scores: time sums run in tree order within a batch, the table's sum before the batch's.
+ * DPHY_ERR_OUT_OF_MEMORY for a failed allocation, the table then unchanged.  Scoring or node support before any add is
+ * DPHY_ERR_INVALID_ARGUMENT. */
+typedef struct dphy_clade_table dphy_clade_table;
+int  dphy_clade_table_create(dphy_ctx* ctx, dphy_clade_table** out);
+void dphy_clade_table_destroy(dphy_ctx* ctx, dphy_clade_table* table);
+int  dphy_clade_table_add(dphy_ctx* ctx, dphy_clade_table* table, dphy_forest* forest);
+int  dphy_clade_table_info(const dphy_clade_table* table, int64_t* num_trees, int64_t* num_clades, int64_t* device_bytes);
+int  dphy_clade_table_score(dphy_ctx* ctx, dphy_clade_table* table, dphy_forest* forest, double* out /* [num_trees] */);
+int  dphy_clade_table_node_support(dphy_ctx* ctx, dphy_clade_table* table, dphy_forest* forest, int32_t tree,
+                                   int64_t* count /* [num_nodes] */, double* mean_t /* [num_nodes] */);
+
 /* ---- tallies ------------------------------------------------------------------------------------------ */
 /* calc_num_muts / _ab / calc_T + the log-G pieces for every tree; out[num_trees]. */
 int  dphy_forest_calc_tallies(dphy_ctx* ctx, dphy_forest* forest, dphy_tallies* out);
