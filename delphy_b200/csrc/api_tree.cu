@@ -31,6 +31,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <optional>
 #include <vector>
 
 namespace dphy {
@@ -316,8 +317,6 @@ __global__ void apitree_pack_kernel(RawTreeDev R, ApiNode* __restrict__ nodes, A
   for (int k = R.miss_off[x]; k < R.miss_off[x + 1]; ++k) { ApiInterval v; v.branch = x; v.start = R.miss_start[k]; v.end = R.miss_end[k]; ivls[k] = v; }
 }
 
-size_t al256(size_t x) { return (x + 255) / 256 * 256; }
-
 bool pinned_host(const void* p) {
   cudaPointerAttributes a{};
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -416,26 +415,25 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
     const int si = sites_index ? sites_index[k] : 0;
     if (si < 0 || si >= num_sites_tables || !sites[si]) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "sites_index out of range");
     if (v.num_sites != sites[si]->L) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "api tree: ref_seq differs from the sites table's reference sequence");
-    stage += al256(16 * (size_t)v.num_nodes) + al256(16 * (size_t)v.num_mutations) + al256(12 * (size_t)v.num_missation_intervals) + al256((size_t)v.num_sites);
+    stage += align_up(16 * (size_t)v.num_nodes) + align_up(16 * (size_t)v.num_mutations) + align_up(12 * (size_t)v.num_missation_intervals) + align_up((size_t)v.num_sites);
   }
   // ---- the struct vectors cross PCIe as they lie (one pinned staging pass; nothing is converted on the host) ------------------------------------
   bool staged_any = false;
   for (int k = 0; k < num_trees; ++k) staged_any = staged_any || !pinned_host(bufs[k]);
-  void* hbv = nullptr;
-  int st = staged_any ? acquire_pinned(ctx, stage, &hbv) : DPHY_OK;
-  if (st != DPHY_OK) return st;
-  char* hb = static_cast<char*>(hbv);
-  std::vector<void*> scratch;
-  auto free_scratch = [&]() { for (void* p : scratch) cudaFreeAsync(p, ctx->stream); };
+  std::optional<PinnedStage> pin;
+  if (staged_any) {
+    pin.emplace(ctx, stage);
+    if (pin->status != DPHY_OK) return pin->status;
+  }
+  char* hb = pin ? pin->p : nullptr;
+  std::vector<DevBlock> scratch;    // freed stream-ordered once the forest is built
   auto dalloc = [&](size_t bytes) -> char* {
-    char* p = nullptr;
-    if (cudaMallocAsync((void**)&p, std::max<size_t>(bytes, 256), ctx->stream) != cudaSuccess) return nullptr;
-    scratch.push_back(p);
-    return p;
+    scratch.emplace_back(ctx->stream);
+    return scratch.back().alloc(std::max<size_t>(bytes, 256)) ? scratch.back().p : nullptr;
   };
   char* d_in = dalloc(stage);
   uint32_t* d_status = reinterpret_cast<uint32_t*>(dalloc(256));
-  if (!d_in || !d_status) { free_scratch(); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree)"); }
+  if (!d_in || !d_status) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree)");
   std::vector<ApiTreeDev> dev(num_trees);
   struct DirectCopy { size_t at; const void* src; size_t bytes; };
   std::vector<DirectCopy> direct_copies;
@@ -454,7 +452,7 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
           if (direct) direct_copies.push_back({at, src, bytes});
           else std::memcpy(hb + o, src, bytes);
         }
-        o += al256(bytes);
+        o += align_up(bytes);
         return at;
       };
       A.nodes = reinterpret_cast<const ApiNode*>(d_in + put(v.nodes, 16 * (size_t)A.n));
@@ -465,11 +463,11 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
   }
   cudaError_t ce = cudaSuccess;
   if (stage && staged_any) ce = cudaMemcpyAsync(d_in, hb, stage, cudaMemcpyHostToDevice, ctx->stream);   // (gaps left by direct buffers: garbage, overwritten next)
-  if (staged_any) release_pinned_async(ctx);
+  pin.reset();
   for (size_t i = 0; i < direct_copies.size() && ce == cudaSuccess; ++i)
     ce = cudaMemcpyAsync(d_in + direct_copies[i].at, direct_copies[i].src, direct_copies[i].bytes, cudaMemcpyHostToDevice, ctx->stream);
   if (ce == cudaSuccess) ce = cudaMemsetAsync(d_status, 0, 256, ctx->stream);
-  if (ce != cudaSuccess) { free_scratch(); return check_cuda(ctx, ce, "H2D api tree"); }
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "H2D api tree");
 
   // ---- per tree: struct-of-arrays split, CSR offsets, the local checks ------------------------------------------------------------------------
   std::vector<RawOut> outs(num_trees);
@@ -478,14 +476,14 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
     const ApiTreeDev& A = dev[k];
     const size_t n = A.n, M = A.M, I = A.I, L = A.L;
     size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t at = o; o = al256(o + std::max<size_t>(bytes, 1)); return at; };
+    auto take = [&](size_t bytes) { const size_t at = o; o = align_up(o + std::max<size_t>(bytes, 1)); return at; };
     const size_t a_par = take(4 * n), a_c0 = take(4 * n), a_c1 = take(4 * n), a_t = take(8 * n);
     const size_t a_moff = take(4 * (n + 1)), a_msite = take(4 * M), a_mfrom = take(M), a_mto = take(M), a_mt = take(8 * M);
     const size_t a_ioff = take(4 * (n + 1)), a_is = take(4 * I), a_ie = take(4 * I), a_foff = take(4 * (n + 1));
     const size_t a_soff = take(4 * (L + 1)), a_sfill = take(4 * L), a_rec = take(16 * M), a_ivo = take(4 * (I + 1));
     const size_t zero_from = a_foff, zero_to = a_rec;          // fs_off (an empty list per node for the first flatten), site counters
     char* nb = dalloc(o);
-    if (!nb) { free_scratch(); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree arrays)"); }
+    if (!nb) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree arrays)");
     cudaMemsetAsync(nb + zero_from, 0, zero_to - zero_from, ctx->stream);
     cudaMemsetAsync(nb + a_ivo, 0, 4 * (I + 1), ctx->stream);        // a tree without missations: F is read from ivl_off[0]
     RawOut& O = outs[k];
@@ -503,7 +501,7 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
     apitree_local_form_kernel<<<(A.n + 127) / 128, 128, 0, ctx->stream>>>(A, O, d_status);
     ctx->launches += 3;
   }
-  st = check_cuda(ctx, cudaGetLastError(), "api tree kernels");
+  int st = check_cuda(ctx, cudaGetLastError(), "api tree kernels");
   uint32_t h_status = 0;
   auto read_status = [&]() {
     int s2 = check_cuda(ctx, cudaMemcpyAsync(&h_status, d_status, 4, cudaMemcpyDeviceToHost, ctx->stream), "D2H");
@@ -515,7 +513,7 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
   for (int k = 0; k < num_trees && st == DPHY_OK; ++k)
     st = check_cuda(ctx, cudaMemcpyAsync(&h_root[2 * k], outs[k].mut_off + dev[k].root, 8, cudaMemcpyDeviceToHost, ctx->stream), "D2H");
   if (st == DPHY_OK) st = read_status();
-  if (st != DPHY_OK) { free_scratch(); return st; }
+  if (st != DPHY_OK) return st;
 
   // ---- first flatten, without from_states: topology / range validation of an upload, DFS positions and subtree sizes -------------------------------
   std::vector<dphy_emat_host> ev(num_trees);
@@ -534,7 +532,7 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
   }
   dphy_forest* fo = nullptr;
   st = forest_from_device_arrays(ctx, num_trees, ev.data(), totals.data(), sites_index, num_sites_tables, sites, &fo);
-  if (st != DPHY_OK) { free_scratch(); return st; }
+  if (st != DPHY_OK) return st;
 
   // ---- from_states (and the `from` CHECK) off the site-sorted mutation table ---------------------------------------------------------------------
   bool any_fs = false;
@@ -576,9 +574,9 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
     const size_t F = (size_t)h_F[k];
     if (F == 0) continue;
     any_fs = true;
-    char* fb = dalloc(al256(4 * F) + al256(F));
+    char* fb = dalloc(align_up(4 * F) + align_up(F));
     if (!fb) { st = set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree from_states)"); break; }
-    O.fs_site = (int32_t*)fb; O.fs_from = (uint8_t*)(fb + al256(4 * F));
+    O.fs_site = (int32_t*)fb; O.fs_from = (uint8_t*)(fb + align_up(4 * F));
     apitree_from_states_kernel<true><<<(int)(((int64_t)A.I * 32 + 255) / 256), 256, 0, ctx->stream>>>(A, O, ords[k]);
     apitree_fs_off_kernel<<<(A.n + 1 + 255) / 256, 256, 0, ctx->stream>>>(A, O, ords[k]);
     ctx->launches += 2;
@@ -588,7 +586,7 @@ extern "C" int dphy_forest_upload_api_trees(dphy_ctx* ctx, int32_t num_trees, co
   if (st == DPHY_OK) st = check_cuda(ctx, cudaGetLastError(), "api tree from_states (fill)");
   // ---- second flatten with the from_states in place; the links did not change, so the DFS order is reused (no Euler-tour ranking) ----------------
   if (st == DPHY_OK && any_fs) st = rebuild_forest_from_device(ctx, fo, ev.data(), totals.data(), true);
-  free_scratch();
+  scratch.clear();
   if (st != DPHY_OK) { dphy_forest_destroy(ctx, fo); return st; }
   *out = fo;
   return DPHY_OK;
@@ -636,22 +634,24 @@ extern "C" int64_t dphy_forest_write_api_tree(dphy_ctx* ctx, dphy_forest* fo, in
                 total = (v_ref + 4 + L + 3) / 4 * 4;
   if (!outv) return total;                                // size query
   if ((int64_t)cap < total) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "write_api_tree: buffer too small");
-  char* d = nullptr;
-  if (cudaMallocAsync((void**)&d, (size_t)total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree out)");
+  DevBlock blk(ctx->stream);
+  if (!blk.alloc((size_t)total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(api tree out)");
+  char* d = blk.p;
   cudaMemsetAsync(d, 0, (size_t)total, ctx->stream);
   apitree_pack_kernel<<<(int)((n + 127) / 128), 128, 0, ctx->stream>>>(R, reinterpret_cast<ApiNode*>(d + v_nodes + 4), reinterpret_cast<ApiMutation*>(d + v_muts + 4),
                                                                     reinterpret_cast<ApiInterval*>(d + v_ivls + 4));
   ++ctx->launches;
   cudaError_t ce = cudaGetLastError();
   if (ce == cudaSuccess && L > 0) ce = cudaMemcpyAsync(d + v_ref + 4, s->d_ref, (size_t)L, cudaMemcpyDeviceToDevice, ctx->stream);
-  // through the context's pinned slab: a device-to-pageable copy is staged by the driver in small pieces (measured 4x slower)
-  void* hbv = nullptr;
-  if (ce == cudaSuccess && acquire_pinned(ctx, (size_t)total, &hbv) != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return DPHY_ERR_OUT_OF_MEMORY; }
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(hbv, d, (size_t)total, cudaMemcpyDeviceToHost, ctx->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-  cudaFreeAsync(d, ctx->stream);
   if (ce != cudaSuccess) return check_cuda(ctx, ce, "write_api_tree");
-  std::memcpy(outv, hbv, (size_t)total);
+  // through the context's pinned slab: a device-to-pageable copy is staged by the driver in small pieces (measured 4x slower)
+  PinnedStage pin(ctx, (size_t)total);
+  if (pin.status != DPHY_OK) return DPHY_ERR_OUT_OF_MEMORY;
+  ce = cudaMemcpyAsync(pin.p, d, (size_t)total, cudaMemcpyDeviceToHost, ctx->stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
+  blk.reset();
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "write_api_tree");
+  std::memcpy(outv, pin.p, (size_t)total);
   uint8_t* o = static_cast<uint8_t*>(outv);
   auto w32 = [&](int64_t at, uint32_t v) { std::memcpy(o + at, &v, 4); };
   auto w16 = [&](int64_t at, uint16_t v) { std::memcpy(o + at, &v, 2); };

@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <new>
 
 namespace dphy {
@@ -25,26 +26,6 @@ int check_cuda(dphy_ctx* ctx, cudaError_t e, const char* what) {
   if (e == cudaSuccess) return DPHY_OK;
   return set_error(ctx, DPHY_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
-
-namespace {
-
-constexpr size_t kAlign = 256;
-size_t align_up(size_t x) { return (x + kAlign - 1) / kAlign * kAlign; }
-
-// A layout planner: reserve() all blocks, then carve them out of one host staging slab and one device slab.
-struct Slab {
-  struct Block { size_t off, bytes; };
-  std::vector<Block> blocks;
-  size_t total = 0;
-  int reserve(size_t bytes) {
-    blocks.push_back({total, bytes});
-    total = align_up(total + std::max<size_t>(bytes, 1));
-    return (int)blocks.size() - 1;
-  }
-  template <typename T> T* at(void* base, int id) const { return reinterpret_cast<T*>(static_cast<char*>(base) + blocks[id].off); }
-};
-
-}  // namespace
 
 // Pinned staging buffer owned by the ctx, grown geometrically.  Copies out of it are asynchronous: the next user waits
 // on the event recorded by release_pinned_async() instead of synchronizing the whole stream.
@@ -271,11 +252,10 @@ static int validate_sequence(dphy_ctx* ctx, const dphy_sites_host* host) {
 // stage ref / partition / nu through the pinned slab and re-derive every table (stream-ordered)
 static int upload_sequence_and_derive(dphy_ctx* ctx, dphy_sites* s, const dphy_sites_host* host) {
   const int L = s->L;
-  const size_t off_part = (L + 255) / 256 * 256, off_nu = 2 * off_part, total = off_nu + sizeof(double) * (size_t)L;
-  void* hbv = nullptr;
-  int st = acquire_pinned(ctx, total, &hbv);
-  if (st != DPHY_OK) return st;
-  char* hb = static_cast<char*>(hbv);
+  const size_t off_part = align_up(L), off_nu = 2 * off_part, total = off_nu + sizeof(double) * (size_t)L;
+  PinnedStage pin(ctx, total);
+  if (pin.status != DPHY_OK) return pin.status;
+  char* hb = pin.p;
   std::memcpy(hb, host->ref, L);
   uint8_t* hp = reinterpret_cast<uint8_t*>(hb + off_part);
   for (int l = 0; l < L; ++l) hp[l] = (uint8_t)host->partition_for_site[l];
@@ -285,9 +265,9 @@ static int upload_sequence_and_derive(dphy_ctx* ctx, dphy_sites* s, const dphy_s
   cudaError_t e = cudaMemcpyAsync(s->d_ref, hb, L, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess) e = cudaMemcpyAsync(s->d_part, hb + off_part, L, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess) e = cudaMemcpyAsync(s->d_nu, hb + off_nu, sizeof(double) * L, cudaMemcpyHostToDevice, ctx->stream);
-  release_pinned_async(ctx);
+  pin.reset();
   if (e != cudaSuccess) return check_cuda(ctx, e, "H2D sites");
-  st = launch_sites_derive(ctx, s);
+  int st = launch_sites_derive(ctx, s);
   if (st == DPHY_OK) st = launch_sites_ref_counts(ctx, s);
   return st;
 }
@@ -301,10 +281,10 @@ int dphy_sites_upload(dphy_ctx* ctx, const dphy_sites_host* host, dphy_sites** o
   int st = validate_sequence(ctx, host);
   if (st == DPHY_OK) st = validate_evo(ctx, P, L, host->nu_l, host->mu, host->pi_a, host->q_ab);
   if (st != DPHY_OK) return st;
-  auto* s = new (std::nothrow) dphy_sites();
+  std::unique_ptr<dphy_sites> s(new (std::nothrow) dphy_sites());
   if (!s) return DPHY_ERR_OUT_OF_MEMORY;
   s->L = L; s->P = P;
-  fill_evo(s, host->mu, host->pi_a, host->q_ab);
+  fill_evo(s.get(), host->mu, host->pi_a, host->q_ab);
   cudaSetDevice(ctx->device);
   Slab slab;
   const int b_ref = slab.reserve(L), b_part = slab.reserve(L), b_nu = slab.reserve(sizeof(double) * L);
@@ -313,9 +293,10 @@ int dphy_sites_upload(dphy_ctx* ctx, const dphy_sites_host* host, dphy_sites** o
   const int b_freq = slab.reserve(sizeof(int32_t) * kMaxPartitions * 4);
   const int b_cnu = slab.reserve(sizeof(double) * (size_t)P * 4 * (L + 1));
   const int b_cref = slab.reserve(sizeof(int32_t) * (size_t)P * 4 * (L + 1));
-  char* dbase = nullptr;
   // stream-ordered pool allocation: no device-wide synchronization, and a freed table's block is reused by the next one
-  if (cudaMallocAsync((void**)&dbase, slab.total, ctx->stream) != cudaSuccess) { delete s; return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(sites)"); }
+  DevBlock blk(ctx->stream);
+  if (!blk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(sites)");
+  char* dbase = blk.p;
   s->bytes = slab.total;
   s->d_ref = slab.at<uint8_t>(dbase, b_ref); s->d_part = slab.at<uint8_t>(dbase, b_part); s->d_nu = slab.at<double>(dbase, b_nu);
   s->d_munu = slab.at<double>(dbase, b_munu); s->d_cumQ = slab.at<double>(dbase, b_cumQ);
@@ -324,9 +305,10 @@ int dphy_sites_upload(dphy_ctx* ctx, const dphy_sites_host* host, dphy_sites** o
   s->d_cref = slab.at<int32_t>(dbase, b_cref);
   s->h.L = L; s->h.P = P; s->h.ref = s->d_ref; s->h.part = s->d_part; s->h.nu = s->d_nu; s->h.munu = s->d_munu;
   s->h.cumQ = s->d_cumQ; s->h.ref_freq = s->d_ref_freq; s->h.cref = s->d_cref;
-  st = upload_sequence_and_derive(ctx, s, host);
-  if (st != DPHY_OK) { cudaFreeAsync(dbase, ctx->stream); delete s; return st; }
-  *out = s;
+  st = upload_sequence_and_derive(ctx, s.get(), host);
+  if (st != DPHY_OK) return st;
+  blk.release();                // s->d_ref is the block's base
+  *out = s.release();
   return DPHY_OK;
 }
 
@@ -359,13 +341,11 @@ int dphy_sites_set_evo(dphy_ctx* ctx, dphy_sites* s, const double* nu_l, const d
   if (st != DPHY_OK) return st;
   fill_evo(s, mu, pi_a, q_ab);
   if (nu_l) {
-    void* hbv = nullptr;
-    st = acquire_pinned(ctx, sizeof(double) * s->L, &hbv);
-    if (st != DPHY_OK) return st;
-    std::memcpy(hbv, nu_l, sizeof(double) * s->L);
+    PinnedStage pin(ctx, sizeof(double) * s->L);
+    if (pin.status != DPHY_OK) return pin.status;
+    std::memcpy(pin.p, nu_l, sizeof(double) * s->L);
     set_nu_uniform(s, nu_l);
-    DPHY_CUDA(ctx, cudaMemcpyAsync(s->d_nu, hbv, sizeof(double) * s->L, cudaMemcpyHostToDevice, ctx->stream));
-    release_pinned_async(ctx);
+    DPHY_CUDA(ctx, cudaMemcpyAsync(s->d_nu, pin.p, sizeof(double) * s->L, cudaMemcpyHostToDevice, ctx->stream));
   }
   fill_tables(s);
   s->version += 1;
@@ -651,7 +631,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   }
   const int fsw_stride = 4 * maxP;
 
-  auto* fo = new (std::nothrow) dphy_forest();
+  std::unique_ptr<dphy_forest> fo(new (std::nothrow) dphy_forest());
   if (!fo) return DPHY_ERR_OUT_OF_MEMORY;
   fo->total_muts = M; fo->total_ivls = I; fo->total_fs = F; fo->total_nonroot_muts = Mnr;
   fo->sites.assign(sites, sites + num_sites_tables);
@@ -725,26 +705,19 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   const int w_status = work.reserve(sizeof(uint32_t) * 4 + sizeof(int32_t) * num_trees);
   const int w_jobs = work.reserve(sizeof(DeviceCopyJob) * ((size_t)num_trees * 15 + 1));     // device-resident sources only (see below)
 
-  char* dbase = nullptr; char* tbase = nullptr; char* wbase = nullptr;
-  if (cudaMallocAsync((void**)&dbase, slab.total, ctx->stream) != cudaSuccess) { delete fo; return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest)"); }
-  if (cudaMallocAsync((void**)&tbase, tmp.total, ctx->stream) != cudaSuccess) {
-    cudaFreeAsync(dbase, ctx->stream); delete fo; return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest raw arrays)");
-  }
-  if (cudaMallocAsync((void**)&wbase, work.total, ctx->stream) != cudaSuccess) {
-    cudaFreeAsync(tbase, ctx->stream); cudaFreeAsync(dbase, ctx->stream); delete fo; return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest workspace)");
-  }
-  fo->allocs.push_back(dbase);
+  DevBlock dblk(ctx->stream), tblk(ctx->stream), wblk(ctx->stream);
+  if (!dblk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest)");
+  if (!tblk.alloc(tmp.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest raw arrays)");
+  if (!wblk.alloc(work.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(forest workspace)");
+  char* dbase = dblk.p; char* tbase = tblk.p; char* wbase = wblk.p;
   fo->bytes = slab.total;
-  if (ensure_copy_stream(ctx) != DPHY_OK || cudaEventRecord(ctx->ev_main, ctx->stream) != cudaSuccess) {
-    cudaFreeAsync(wbase, ctx->stream); cudaFreeAsync(tbase, ctx->stream); cudaFreeAsync(dbase, ctx->stream); delete fo;
+  if (ensure_copy_stream(ctx) != DPHY_OK || cudaEventRecord(ctx->ev_main, ctx->stream) != cudaSuccess)
     return set_error(ctx, DPHY_ERR_CUDA, "upload: copy stream / event");
-  }
-  auto fail = [&](int st) { cudaFreeAsync(wbase, ctx->stream); cudaFreeAsync(tbase, ctx->stream); cudaFreeAsync(dbase, ctx->stream); delete fo; return st; };
 
-  void* hbv = nullptr;
-  int st = acquire_pinned(ctx, header_bytes + raw_upload_bytes, &hbv);
-  if (st != DPHY_OK) return fail(st);
-  char* hb = static_cast<char*>(hbv);          // [header | raw]
+  PinnedStage pin(ctx, header_bytes + raw_upload_bytes);
+  if (pin.status != DPHY_OK) return pin.status;
+  int st = DPHY_OK;
+  char* hb = pin.p;                            // [header | raw]
   char* hraw = hb + header_bytes;
 
   // ---- host side: only the per-tree / per-tile descriptors; the arrays are streamed verbatim ---------------------------
@@ -806,12 +779,12 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   cudaError_t ce = cudaMemcpyAsync(dbase, hb, header_bytes, cudaMemcpyHostToDevice, ctx->stream);
   if (ce == cudaSuccess) ce = cudaMemsetAsync(dbase + header_bytes, 0, slab.total - header_bytes, ctx->stream);
   if (ce == cudaSuccess) ce = cudaMemsetAsync(wbase + work.blocks[w_status].off, 0, work.blocks[w_status].bytes, ctx->stream);
-  if (ce != cudaSuccess) return fail(check_cuda(ctx, ce, "H2D forest header"));
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "H2D forest header");
   // the RawTreeDev records were written straight into the pinned slab above; everything in [0, raw_upload_bytes) not
   // covered by a job (those records, alignment gaps) is copied as it lies
   while ((int)ctx->ev_tree.size() < num_trees) {
     cudaEvent_t e = nullptr;
-    if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return fail(set_error(ctx, DPHY_ERR_CUDA, "cudaEventCreate"));
+    if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return set_error(ctx, DPHY_ERR_CUDA, "cudaEventCreate");
     ctx->ev_tree.push_back(e);
   }
   std::vector<char> tree_has_lists(num_trees, 0);
@@ -836,8 +809,8 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   } else {
     st = staged_upload(ctx, hraw, jobs, tbase, raw_upload_bytes, &two_phase);
   }
-  if (!two_phase) release_pinned_async(ctx);
-  if (st != DPHY_OK) return fail(st);
+  if (!two_phase) pin.reset();           // (two-phase: once the copy streams are joined below)
+  if (st != DPHY_OK) return st;
 
   ForestDev& h = fo->h;
   h.num_trees = num_trees; h.num_nodes = (int32_t)N; h.num_tiles = (int32_t)tiles; h.num_sites_tables = num_sites_tables;
@@ -892,13 +865,13 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   if (two_phase) {
     // Euler-tour ranking as soon as the topology arrays have landed; the rest once the lists have
     ce = cudaStreamWaitEvent(ctx->stream, ctx->ev_topo, 0);
-    if (ce != cudaSuccess) return fail(check_cuda(ctx, ce, "wait topology upload"));
+    if (ce != cudaSuccess) return check_cuda(ctx, ce, "wait topology upload");
     st = launch_flatten(ctx, P, (int)tiles, max_tree_nodes, 0);
-    if (st != DPHY_OK) { sync_copy_streams(ctx); return fail(st); }
+    if (st != DPHY_OK) { sync_copy_streams(ctx); return st; }
     ce = cudaStreamWaitEvent(ctx->stream, ctx->ev_nodes, 0);
-    if (ce != cudaSuccess) { sync_copy_streams(ctx); return fail(check_cuda(ctx, ce, "wait node upload")); }
+    if (ce != cudaSuccess) { sync_copy_streams(ctx); return check_cuda(ctx, ce, "wait node upload"); }
     st = launch_flatten(ctx, P, (int)tiles, max_tree_nodes, 1);
-    if (st != DPHY_OK) { sync_copy_streams(ctx); return fail(st); }
+    if (st != DPHY_OK) { sync_copy_streams(ctx); return st; }
     // lists: each tree is gathered and folded as soon as its own arrays have landed, while the next trees' are still in flight
     for (int k = 0; k < num_trees && st == DPHY_OK; ++k) {
       if (tree_has_lists[k]) {
@@ -911,35 +884,36 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
       ce = cudaStreamWaitEvent(ctx->stream, ctx->ev_lists, 0);
       if (ce != cudaSuccess) st = check_cuda(ctx, ce, "wait list upload");
     }
-    if (st != DPHY_OK) { sync_copy_streams(ctx); return fail(st); }
-    release_pinned_async(ctx);
+    if (st != DPHY_OK) { sync_copy_streams(ctx); return st; }
+    pin.reset();
     st = launch_flatten_finish(ctx, P);
   } else {
     st = launch_flatten(ctx, P, (int)tiles, max_tree_nodes);
   }
-  if (st != DPHY_OK) return fail(st);
+  if (st != DPHY_OK) return st;
   std::vector<int32_t> status(4 + num_trees, 0);
   ce = cudaMemcpyAsync(status.data(), P.status, sizeof(int32_t) * status.size(), cudaMemcpyDeviceToHost, ctx->stream);
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-  if (ce != cudaSuccess) return fail(check_cuda(ctx, ce, "forest flatten"));
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "forest flatten");
   st = flatten_status_to_error(ctx, (uint32_t)status[0]);
-  if (st != DPHY_OK) return fail(st);
+  if (st != DPHY_OK) return st;
   for (int k = 0; k < num_trees; ++k) fo->tree_max_depth[k] = status[4 + k];
   fo->num_strad = status[1]; fo->num_fast_ctiles = status[2]; fo->num_slow_ctiles = status[3];
-  cudaFreeAsync(wbase, ctx->stream);
-  fo->allocs.push_back(tbase);                       // the raw arrays stay (freed with the forest)
+  wblk.reset();
   fo->bytes += tmp.total;
   fo->raw.assign(h_raw, h_raw + num_trees);          // device pointers of every tree's host-order arrays
   fo->sites_index.resize(num_trees);
   for (int k = 0; k < num_trees; ++k) fo->sites_index[k] = sites_index ? sites_index[k] : 0;
   // first evaluation.  Forests whose site rates are uniform take the folded schedule; the structure-only outputs (nsmn, the
   // num_muts tallies) then come from a general pass the first time a getter asks for them (ensure_struct_outputs)
-  st = launch_log_G(ctx, fo);
-  if (st != DPHY_OK) { cudaStreamSynchronize(ctx->stream); cudaFreeAsync(tbase, ctx->stream); cudaFreeAsync(dbase, ctx->stream); delete fo; return st; }
+  st = launch_log_G(ctx, fo.get());
+  if (st != DPHY_OK) { cudaStreamSynchronize(ctx->stream); return st; }
+  fo->allocs.push_back(dblk.release());
+  fo->allocs.push_back(tblk.release());              // the raw arrays stay (freed with the forest)
   fo->evaluated = true;         // that pass is a complete evaluation under the current evo model
   fo->eval_version.resize(fo->sites.size());
   for (size_t i = 0; i < fo->sites.size(); ++i) fo->eval_version[i] = fo->sites[i]->version;
-  *out = fo;
+  *out = fo.release();
   return DPHY_OK;
 }
 

@@ -4,6 +4,7 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -373,6 +374,62 @@ int launch_set_node_times(dphy_ctx* ctx, dphy_forest* fo, int tree, const int32_
 // Pinned staging buffer of the ctx: acquire waits for the previous async copy out of it; release records an event.
 int acquire_pinned(dphy_ctx* ctx, size_t bytes, void** out);
 void release_pinned_async(dphy_ctx* ctx);
+
+// ---- host-side helpers of the entry points ------------------------------------------------------------------------------
+constexpr size_t kAlign = 256;
+inline size_t align_up(size_t x) { return (x + kAlign - 1) / kAlign * kAlign; }
+
+// A layout planner: reserve() all blocks, then carve them out of one host staging slab and one device slab.
+struct Slab {
+  struct Block { size_t off, bytes; };
+  std::vector<Block> blocks;
+  size_t total = 0;
+  int reserve(size_t bytes) {
+    blocks.push_back({total, bytes});
+    total = align_up(total + std::max<size_t>(bytes, 1));
+    return (int)blocks.size() - 1;
+  }
+  template <typename T> T* at(void* base, int id) const { return reinterpret_cast<T*>(static_cast<char*>(base) + blocks[id].off); }
+};
+
+// A stream-ordered device allocation, freed when it goes out of scope unless released.
+struct DevBlock {
+  cudaStream_t s;
+  char* p = nullptr;
+  explicit DevBlock(cudaStream_t st) : s(st) {}
+  DevBlock(DevBlock&& o) noexcept : s(o.s), p(o.release()) {}     // move-only (so that it can live in a std::vector)
+  ~DevBlock() { reset(); }
+  bool alloc(size_t bytes, cudaError_t* why = nullptr) {
+    const cudaError_t e = cudaMallocAsync((void**)&p, std::max<size_t>(bytes, 1), s);
+    if (why) *why = e;
+    if (e == cudaSuccess) return true;
+    p = nullptr;
+    cudaGetLastError();
+    return false;
+  }
+  void reset() { if (p) cudaFreeAsync(p, s); p = nullptr; }
+  char* release() { char* q = p; p = nullptr; return q; }
+};
+
+// The ctx's pinned staging buffer for one call: acquired on construction (check `status`), released once -- by reset() or on
+// scope exit -- after the copies out of it have been enqueued.
+struct PinnedStage {
+  dphy_ctx* ctx;
+  char* p = nullptr;
+  int status; bool held;
+  PinnedStage(dphy_ctx* c, size_t bytes) : ctx(c) {
+    void* v = nullptr;
+    status = acquire_pinned(c, bytes, &v);
+    held = status == DPHY_OK;
+    p = static_cast<char*>(v);
+  }
+  PinnedStage(PinnedStage&&) = delete;
+  ~PinnedStage() { reset(); }
+  void reset() { if (held) release_pinned_async(ctx); held = false; }
+};
+
+// bits of a radix-sort key that holds 0 .. max_value (at least 1, at most 31)
+inline int bits_for(int64_t max_value) { int b = 1; while (b < 31 && ((int64_t)1 << b) <= max_value) ++b; return b; }
 }  // namespace dphy
 
 #endif  // DPHY_INTERNAL_H_

@@ -176,23 +176,7 @@ __global__ void clade_node_support_kernel(ForestDev f, int tree, const CladeKey*
   }
 }
 
-size_t al(size_t x) { return (x + 255) / 256 * 256; }
 unsigned blocks(int64_t n) { return (unsigned)((n + 255) / 256); }
-
-// A stream-ordered device allocation, freed when it goes out of scope unless released.
-struct DevBlock {
-  cudaStream_t s;
-  char* p = nullptr;
-  explicit DevBlock(cudaStream_t st) : s(st) {}
-  ~DevBlock() { if (p) cudaFreeAsync(p, s); }
-  bool alloc(size_t bytes) {
-    if (cudaMallocAsync((void**)&p, std::max<size_t>(bytes, 1), s) == cudaSuccess) return true;
-    p = nullptr;
-    cudaGetLastError();
-    return false;
-  }
-  char* release() { char* q = p; p = nullptr; return q; }
-};
 
 // Every tree of `fo` must have N nodes (N = the table's, or tree 0's for a table that is still empty).
 int check_sizes(dphy_ctx* ctx, const dphy_clade_table* tab, const dphy_forest* fo, int* N) {
@@ -223,14 +207,15 @@ int clade_keys(dphy_ctx* ctx, dphy_forest* fo, const uint32_t* tips, int bitmap_
   const int N = fo->h.num_nodes;
   size_t scan_bytes = 0;
   DPHY_CUDA(ctx, cub::DeviceScan::InclusiveScan(nullptr, scan_bytes, (const CladeKey*)nullptr, (CladeKey*)nullptr, CladeKeyAdd{}, N, ctx->stream));
-  const size_t b_S = al(sizeof(unsigned long long) * kStLen), b_h = b_S + al(sizeof(CladeKey) * ((size_t)N + 1));
-  const size_t b_cub = b_h + al(sizeof(CladeKey) * (size_t)N), b_extra = b_cub + al(scan_bytes);
-  if (!ks.blk.alloc(b_extra + extra)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table scratch)");
+  Slab slab;
+  const int b_st = slab.reserve(sizeof(unsigned long long) * kStLen), b_S = slab.reserve(sizeof(CladeKey) * ((size_t)N + 1));
+  const int b_h = slab.reserve(sizeof(CladeKey) * (size_t)N), b_cub = slab.reserve(scan_bytes), b_extra = slab.reserve(extra);
+  if (!ks.blk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table scratch)");
   char* d = ks.blk.p;
-  ks.status = (unsigned long long*)d;
-  ks.S = (CladeKey*)(d + b_S);
-  ks.h = (CladeKey*)(d + b_h);
-  ks.extra = d + b_extra;
+  ks.status = slab.at<unsigned long long>(d, b_st);
+  ks.S = slab.at<CladeKey>(d, b_S);
+  ks.h = slab.at<CladeKey>(d, b_h);
+  ks.extra = slab.at<char>(d, b_extra);
   DPHY_CUDA(ctx, cudaMemsetAsync(ks.status, 0, sizeof(unsigned long long) * kStLen, ctx->stream));
   DPHY_CUDA(ctx, cudaMemsetAsync(ks.S, 0, sizeof(CladeKey), ctx->stream));
   if (!tips) {
@@ -242,7 +227,7 @@ int clade_keys(dphy_ctx* ctx, dphy_forest* fo, const uint32_t* tips, int bitmap_
     tips = bm;
   }
   clade_tip_keys_kernel<<<blocks(N), 256, 0, ctx->stream>>>(fo->h, tips, ks.h, ks.status);
-  DPHY_CUDA(ctx, cub::DeviceScan::InclusiveScan(d + b_cub, scan_bytes, (const CladeKey*)ks.h, ks.S + 1, CladeKeyAdd{}, N, ctx->stream));
+  DPHY_CUDA(ctx, cub::DeviceScan::InclusiveScan(slab.at<char>(d, b_cub), scan_bytes, (const CladeKey*)ks.h, ks.S + 1, CladeKeyAdd{}, N, ctx->stream));
   clade_keys_kernel<<<blocks(N), 256, 0, ctx->stream>>>(fo->h, ks.S, ks.h);
   ctx->launches += 3;
   return check_cuda(ctx, cudaGetLastError(), "clade keys");
@@ -308,18 +293,19 @@ int dphy_clade_table_add(dphy_ctx* ctx, dphy_clade_table* tab, dphy_forest* fo) 
   DPHY_CUDA(ctx, cub::DeviceRunLengthEncode::Encode(nullptr, rle_bytes, (const CladeKey*)nullptr, (CladeKey*)nullptr, (int32_t*)nullptr,
                                                     (int32_t*)nullptr, N, s));
   DPHY_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, off_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, N, s));
-  const size_t b_hs = first ? al(sizeof(uint32_t) * words) : 0, b_ts = b_hs + al(sizeof(CladeKey) * (size_t)N);
-  const size_t b_len = b_ts + al(sizeof(double) * (size_t)N), b_off = b_len + al(sizeof(int32_t) * (size_t)N);
-  const size_t b_nr = b_off + al(sizeof(int32_t) * (size_t)N), b_cub = b_nr + 256;
-  const size_t cub_bytes = std::max(sort_bytes, std::max(rle_bytes, off_bytes));
+  Slab ex;
+  if (first) ex.reserve(sizeof(uint32_t) * words);    // the tip bitmap, at the block's start (clade_keys)
+  const int b_hs = ex.reserve(sizeof(CladeKey) * (size_t)N), b_ts = ex.reserve(sizeof(double) * (size_t)N);
+  const int b_len = ex.reserve(sizeof(int32_t) * (size_t)N), b_off = ex.reserve(sizeof(int32_t) * (size_t)N);
+  const int b_nr = ex.reserve(sizeof(int32_t)), b_cub = ex.reserve(std::max(sort_bytes, std::max(rle_bytes, off_bytes)));
   KeyScratch ks(s);
-  if ((st = clade_keys(ctx, fo, first ? nullptr : tab->d_tips, words, b_cub + al(cub_bytes), ks)) != DPHY_OK) return st;
-  CladeKey* hs = (CladeKey*)(ks.extra + b_hs);
-  double* ts = (double*)(ks.extra + b_ts);
-  int32_t* run_len = (int32_t*)(ks.extra + b_len);
-  int32_t* run_off = (int32_t*)(ks.extra + b_off);
-  int32_t* d_nruns = (int32_t*)(ks.extra + b_nr);
-  void* cub_tmp = ks.extra + b_cub;
+  if ((st = clade_keys(ctx, fo, first ? nullptr : tab->d_tips, words, ex.total, ks)) != DPHY_OK) return st;
+  CladeKey* hs = ex.at<CladeKey>(ks.extra, b_hs);
+  double* ts = ex.at<double>(ks.extra, b_ts);
+  int32_t* run_len = ex.at<int32_t>(ks.extra, b_len);
+  int32_t* run_off = ex.at<int32_t>(ks.extra, b_off);
+  int32_t* d_nruns = ex.at<int32_t>(ks.extra, b_nr);
+  void* cub_tmp = ex.at<char>(ks.extra, b_cub);
   CladeKey* bkey = ks.S;
   CladeVal* bval = (CladeVal*)ks.h;
   DPHY_CUDA(ctx, cub::DeviceRadixSort::SortPairs(cub_tmp, sort_bytes, (const CladeKey*)ks.h, hs, (const double*)fo->h.t, ts, N,
@@ -352,11 +338,12 @@ int dphy_clade_table_add(dphy_ctx* ctx, dphy_clade_table* tab, dphy_forest* fo) 
     return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "clade table: more than 2^31 - 1 clades");
 
   // ---- step 3: the new table at its exact size
+  Slab tbl;
+  const int t_keys = tbl.reserve(sizeof(CladeKey) * (size_t)n_new), t_vals = tbl.reserve(sizeof(CladeVal) * (size_t)n_new);
   DevBlock table_blk(s);
-  if (!table_blk.alloc(al(sizeof(CladeKey) * (size_t)n_new) + sizeof(CladeVal) * (size_t)n_new))
-    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table)");
-  CladeKey* new_keys = (CladeKey*)table_blk.p;
-  CladeVal* new_vals = (CladeVal*)(table_blk.p + al(sizeof(CladeKey) * (size_t)n_new));
+  if (!table_blk.alloc(tbl.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table)");
+  CladeKey* new_keys = tbl.at<CladeKey>(table_blk.p, t_keys);
+  CladeVal* new_vals = tbl.at<CladeVal>(table_blk.p, t_vals);
   DevBlock tips_blk(s);
   if (first) {
     if (!tips_blk.alloc(sizeof(uint32_t) * words)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table tips)");
@@ -374,13 +361,14 @@ int dphy_clade_table_add(dphy_ctx* ctx, dphy_clade_table* tab, dphy_forest* fo) 
                                                 CladeKeyLess{}, s));
     DPHY_CUDA(ctx, cub::DeviceReduce::ReduceByKey(nullptr, rbk_bytes, (const CladeKey*)nullptr, (CladeKey*)nullptr, (const CladeVal*)nullptr,
                                                   (CladeVal*)nullptr, (int32_t*)nullptr, CladeValAdd{}, m, s));
+    Slab mg;
+    const int b_mkey = mg.reserve(sizeof(CladeKey) * (size_t)m), b_mval = mg.reserve(sizeof(CladeVal) * (size_t)m);
+    const int b_mcub = mg.reserve(std::max(merge_bytes, rbk_bytes));
     DevBlock mblk(s);
-    const size_t b_mval = al(sizeof(CladeKey) * (size_t)m), b_mcub = b_mval + al(sizeof(CladeVal) * (size_t)m);
-    if (!mblk.alloc(b_mcub + al(std::max(merge_bytes, rbk_bytes))))
-      return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table merge)");
-    CladeKey* mkey = (CladeKey*)mblk.p;
-    CladeVal* mval = (CladeVal*)(mblk.p + b_mval);
-    void* mcub = mblk.p + b_mcub;
+    if (!mblk.alloc(mg.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(clade table merge)");
+    CladeKey* mkey = mg.at<CladeKey>(mblk.p, b_mkey);
+    CladeVal* mval = mg.at<CladeVal>(mblk.p, b_mval);
+    void* mcub = mg.at<char>(mblk.p, b_mcub);
     DPHY_CUDA(ctx, cub::DeviceMerge::MergePairs(mcub, merge_bytes, (const CladeKey*)tab->d_keys, (const CladeVal*)tab->d_vals, (int)nt,
                                                 (const CladeKey*)bkey, (const CladeVal*)bval, nb, mkey, mval, CladeKeyLess{}, s));
     DPHY_CUDA(ctx, cub::DeviceReduce::ReduceByKey(mcub, rbk_bytes, (const CladeKey*)mkey, new_keys, (const CladeVal*)mval, new_vals, d_nruns,
@@ -418,10 +406,11 @@ int dphy_clade_table_score(dphy_ctx* ctx, dphy_clade_table* tab, dphy_forest* fo
   if ((st = check_sizes(ctx, tab, fo, &Nt)) != DPHY_OK) return st;
   cudaSetDevice(ctx->device);
   KeyScratch ks(ctx->stream);
-  const size_t b_out = al(sizeof(double) * tiles);
-  if ((st = clade_keys(ctx, fo, tab->d_tips, 0, b_out + sizeof(double) * T, ks)) != DPHY_OK) return st;
-  double* tile_part = (double*)ks.extra;
-  double* d_out = (double*)(ks.extra + b_out);
+  Slab ex;
+  const int b_part = ex.reserve(sizeof(double) * tiles), b_out = ex.reserve(sizeof(double) * T);
+  if ((st = clade_keys(ctx, fo, tab->d_tips, 0, ex.total, ks)) != DPHY_OK) return st;
+  double* tile_part = ex.at<double>(ks.extra, b_part);
+  double* d_out = ex.at<double>(ks.extra, b_out);
   clade_score_tile_kernel<<<tiles, kTile, 0, ctx->stream>>>(fo->h, ks.h, view_of(tab), tile_part);
   clade_tree_sum_kernel<<<T, kTile, 0, ctx->stream>>>(fo->h, tile_part, d_out);
   ctx->launches += 2;
@@ -447,10 +436,11 @@ int dphy_clade_table_node_support(dphy_ctx* ctx, dphy_clade_table* tab, dphy_for
   if ((st = check_sizes(ctx, tab, fo, &Nt)) != DPHY_OK) return st;
   cudaSetDevice(ctx->device);
   KeyScratch ks(ctx->stream);
-  const size_t b_mean = al(sizeof(int64_t) * Nt);
-  if ((st = clade_keys(ctx, fo, tab->d_tips, 0, b_mean + sizeof(double) * Nt, ks)) != DPHY_OK) return st;
-  int64_t* d_count = (int64_t*)ks.extra;
-  double* d_mean = (double*)(ks.extra + b_mean);
+  Slab ex;
+  const int b_count = ex.reserve(sizeof(int64_t) * Nt), b_mean = ex.reserve(sizeof(double) * Nt);
+  if ((st = clade_keys(ctx, fo, tab->d_tips, 0, ex.total, ks)) != DPHY_OK) return st;
+  int64_t* d_count = ex.at<int64_t>(ks.extra, b_count);
+  double* d_mean = ex.at<double>(ks.extra, b_mean);
   clade_node_support_kernel<<<blocks(Nt), 256, 0, ctx->stream>>>(fo->h, tree, ks.h, view_of(tab), d_count, d_mean);
   ++ctx->launches;
   DPHY_CUDA(ctx, cudaGetLastError());

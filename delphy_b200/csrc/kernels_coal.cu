@@ -106,9 +106,6 @@ __global__ void __launch_bounds__(kTile) coal_tree_sum_kernel(ForestDev f, const
   if (threadIdx.x == 0) out[blockIdx.x] = v;
 }
 
-size_t al(size_t x) { return (x + 255) / 256 * 256; }
-int bits_for(int max_value) { int b = 1; while (b < 31 && (1 << b) <= max_value) ++b; return b; }
-
 }  // namespace
 }  // namespace dphy
 
@@ -132,18 +129,20 @@ int dphy_forest_log_coalescent_prior(dphy_ctx* ctx, dphy_forest* fo, double n0, 
   if (T > 1)
     DPHY_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, cub2_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (const int32_t*)nullptr,
                                                    (int32_t*)nullptr, N, 0, tree_bits, ctx->stream));
-  const size_t b_ts = 0, b_ev = b_ts + al(sizeof(double) * N), b_ev2 = b_ev + al(sizeof(int32_t) * N);
-  const size_t b_key = b_ev2 + al(sizeof(int32_t) * N), b_key2 = b_key + al(sizeof(int32_t) * N);
-  const size_t b_tsum = b_key2 + al(sizeof(int32_t) * N), b_tpart = b_tsum + al(sizeof(int32_t) * tiles);
-  const size_t b_tt = b_tpart + al(sizeof(double) * tiles), b_out = b_tt + al(sizeof(int32_t) * (tiles / 8192 + 2));
-  const size_t b_cub = b_out + al(sizeof(double) * T), total = b_cub + al(std::max(cub_bytes, cub2_bytes));
-  char* d = nullptr;
-  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(coalescent prior)");
-  double* ts = (double*)(d + b_ts);
-  int32_t* ev = (int32_t*)(d + b_ev); int32_t* ev2 = (int32_t*)(d + b_ev2);
-  int32_t* key = (int32_t*)(d + b_key); int32_t* key2 = (int32_t*)(d + b_key2);
-  int32_t* tsum = (int32_t*)(d + b_tsum); double* tpart = (double*)(d + b_tpart); int32_t* tt = (int32_t*)(d + b_tt);
-  double* d_out = (double*)(d + b_out); void* cub_tmp = d + b_cub;
+  Slab slab;
+  const int b_ts = slab.reserve(sizeof(double) * N), b_ev = slab.reserve(sizeof(int32_t) * N), b_ev2 = slab.reserve(sizeof(int32_t) * N);
+  const int b_key = slab.reserve(sizeof(int32_t) * N), b_key2 = slab.reserve(sizeof(int32_t) * N);
+  const int b_tsum = slab.reserve(sizeof(int32_t) * tiles), b_tpart = slab.reserve(sizeof(double) * tiles);
+  const int b_tt = slab.reserve(sizeof(int32_t) * (tiles / 8192 + 2)), b_out = slab.reserve(sizeof(double) * T);
+  const int b_cub = slab.reserve(std::max(cub_bytes, cub2_bytes));
+  DevBlock blk(ctx->stream);
+  if (!blk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(coalescent prior)");
+  char* d = blk.p;
+  double* ts = slab.at<double>(d, b_ts);
+  int32_t* ev = slab.at<int32_t>(d, b_ev); int32_t* ev2 = slab.at<int32_t>(d, b_ev2);
+  int32_t* key = slab.at<int32_t>(d, b_key); int32_t* key2 = slab.at<int32_t>(d, b_key2);
+  int32_t* tsum = slab.at<int32_t>(d, b_tsum); double* tpart = slab.at<double>(d, b_tpart); int32_t* tt = slab.at<int32_t>(d, b_tt);
+  double* d_out = slab.at<double>(d, b_out); void* cub_tmp = slab.at<char>(d, b_cub);
   const unsigned nb = (unsigned)((N + 255) / 256);
   coal_iota_kernel<<<nb, 256, 0, ctx->stream>>>(ev2, N);
   // every CUB sort below is counted as one launch
@@ -171,7 +170,6 @@ int dphy_forest_log_coalescent_prior(dphy_ctx* ctx, dphy_forest* fo, double n0, 
   }
   if (st == DPHY_OK) st = check_cuda(ctx, cudaMemcpyAsync(out, d_out, sizeof(double) * T, cudaMemcpyDeviceToHost, ctx->stream), "coalescent prior D2H");
   if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "coalescent prior");
-  cudaFreeAsync(d, ctx->stream);
   return st;
 }
 

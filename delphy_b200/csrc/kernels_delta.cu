@@ -151,8 +151,6 @@ int launch_raw_set_node_times(dphy_ctx* ctx, dphy_forest* fo, int tree, const in
 using namespace dphy;
 
 namespace {
-size_t al256(size_t x) { return (x + 255) / 256 * 256; }
-
 // per-node list lengths, host order, fetched once from the resident raw offsets
 int ensure_host_counts(dphy_ctx* ctx, dphy_forest* fo) {
   const int nt = fo->h.num_trees;
@@ -207,14 +205,14 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
   if (!any) return DPHY_OK;
 
   // ---- pack rows + payload into the pinned slab, one H2D ----------------------------------------------------------------------------------
-  const size_t o_rows = 0, o_msite = al256(o_rows + sizeof(RowDev) * std::max(1, count)), o_mfrom = al256(o_msite + 4 * pm),
-               o_mto = al256(o_mfrom + pm), o_mt = al256(o_mto + pm), o_is = al256(o_mt + 8 * pm), o_ie = al256(o_is + 4 * pi),
-               o_fsite = al256(o_ie + 4 * pi), o_ffrom = al256(o_fsite + 4 * pf), total = al256(o_ffrom + pf);
-  void* hbv = nullptr;
-  st = acquire_pinned(ctx, total, &hbv);
-  if (st != DPHY_OK) return st;
-  char* hb = static_cast<char*>(hbv);
-  RowDev* hrows = reinterpret_cast<RowDev*>(hb + o_rows);
+  Slab pay;
+  const int b_rows = pay.reserve(sizeof(RowDev) * std::max(1, count)), b_msite = pay.reserve(4 * pm), b_mfrom = pay.reserve(pm);
+  const int b_mto = pay.reserve(pm), b_mt = pay.reserve(8 * pm), b_is = pay.reserve(4 * pi), b_ie = pay.reserve(4 * pi);
+  const int b_fsite = pay.reserve(4 * pf), b_ffrom = pay.reserve(pf);
+  PinnedStage pin(ctx, pay.total);
+  if (pin.status != DPHY_OK) return pin.status;
+  char* hb = pin.p;
+  RowDev* hrows = pay.at<RowDev>(hb, b_rows);
   {
     size_t cm = 0, ci = 0, cf = 0;
     // rows grouped tree-major so that each tree's kernels address one contiguous range
@@ -228,36 +226,36 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
       d.n_muts = r.n_muts; d.n_miss = r.n_miss; d.n_fs = r.n_fs; d.pad = 0; d.pad2 = 0;
       d.o_mut = (int32_t)cm; d.o_miss = (int32_t)ci; d.o_fs = (int32_t)cf;
       if (r.n_muts) {
-        std::memcpy(hb + o_msite + 4 * cm, r.mut_site, 4 * (size_t)r.n_muts); std::memcpy(hb + o_mfrom + cm, r.mut_from, r.n_muts);
-        std::memcpy(hb + o_mto + cm, r.mut_to, r.n_muts); std::memcpy(hb + o_mt + 8 * cm, r.mut_t, 8 * (size_t)r.n_muts);
+        std::memcpy(pay.at<int32_t>(hb, b_msite) + cm, r.mut_site, 4 * (size_t)r.n_muts); std::memcpy(pay.at<uint8_t>(hb, b_mfrom) + cm, r.mut_from, r.n_muts);
+        std::memcpy(pay.at<uint8_t>(hb, b_mto) + cm, r.mut_to, r.n_muts); std::memcpy(pay.at<double>(hb, b_mt) + cm, r.mut_t, 8 * (size_t)r.n_muts);
       }
-      if (r.n_miss) { std::memcpy(hb + o_is + 4 * ci, r.miss_start, 4 * (size_t)r.n_miss); std::memcpy(hb + o_ie + 4 * ci, r.miss_end, 4 * (size_t)r.n_miss); }
-      if (r.n_fs) { std::memcpy(hb + o_fsite + 4 * cf, r.fs_site, 4 * (size_t)r.n_fs); std::memcpy(hb + o_ffrom + cf, r.fs_from, r.n_fs); }
+      if (r.n_miss) { std::memcpy(pay.at<int32_t>(hb, b_is) + ci, r.miss_start, 4 * (size_t)r.n_miss); std::memcpy(pay.at<int32_t>(hb, b_ie) + ci, r.miss_end, 4 * (size_t)r.n_miss); }
+      if (r.n_fs) { std::memcpy(pay.at<int32_t>(hb, b_fsite) + cf, r.fs_site, 4 * (size_t)r.n_fs); std::memcpy(pay.at<uint8_t>(hb, b_ffrom) + cf, r.fs_from, r.n_fs); }
       cm += r.n_muts; ci += r.n_miss; cf += r.n_fs;
     }
   }
-  char* d_pay = nullptr;
-  if (cudaMallocAsync((void**)&d_pay, total, ctx->stream) != cudaSuccess) { release_pinned_async(ctx); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(rows)"); }
-  cudaError_t ce = cudaMemcpyAsync(d_pay, hb, total, cudaMemcpyHostToDevice, ctx->stream);
-  release_pinned_async(ctx);
-  if (ce != cudaSuccess) { cudaFreeAsync(d_pay, ctx->stream); return check_cuda(ctx, ce, "H2D rows"); }
+  // payload, link flag, new raw blocks + row maps: consumed by the re-flatten below, freed stream-ordered after it
+  std::vector<DevBlock> scratch;
+  scratch.emplace_back(ctx->stream);
+  if (!scratch.back().alloc(pay.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(rows)");
+  char* d_pay = scratch.back().p;
+  cudaError_t ce = cudaMemcpyAsync(d_pay, hb, pay.total, cudaMemcpyHostToDevice, ctx->stream);
+  pin.reset();
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "H2D rows");
   RowPayloadDev P{};
-  P.rows = reinterpret_cast<const RowDev*>(d_pay + o_rows);
-  P.mut_site = reinterpret_cast<const int32_t*>(d_pay + o_msite); P.mut_from = reinterpret_cast<const uint8_t*>(d_pay + o_mfrom);
-  P.mut_to = reinterpret_cast<const uint8_t*>(d_pay + o_mto); P.mut_t = reinterpret_cast<const double*>(d_pay + o_mt);
-  P.miss_start = reinterpret_cast<const int32_t*>(d_pay + o_is); P.miss_end = reinterpret_cast<const int32_t*>(d_pay + o_ie);
-  P.fs_site = reinterpret_cast<const int32_t*>(d_pay + o_fsite); P.fs_from = reinterpret_cast<const uint8_t*>(d_pay + o_ffrom);
+  P.rows = pay.at<const RowDev>(d_pay, b_rows);
+  P.mut_site = pay.at<const int32_t>(d_pay, b_msite); P.mut_from = pay.at<const uint8_t>(d_pay, b_mfrom);
+  P.mut_to = pay.at<const uint8_t>(d_pay, b_mto); P.mut_t = pay.at<const double>(d_pay, b_mt);
+  P.miss_start = pay.at<const int32_t>(d_pay, b_is); P.miss_end = pay.at<const int32_t>(d_pay, b_ie);
+  P.fs_site = pay.at<const int32_t>(d_pay, b_fsite); P.fs_from = pay.at<const uint8_t>(d_pay, b_ffrom);
 
   // ---- rebuild the raw arrays of every changed tree on the device ----------------------------------------------------------------------------
   std::vector<dphy_emat_host> views(nt);
   std::vector<TreeTotals> totals(nt);
-  std::vector<void*> scratch;       // new raw blocks + row maps: consumed by the re-flatten below, freed stream-ordered after it
-  scratch.push_back(d_pay);
-  auto free_scratch = [&]() { for (void* p : scratch) cudaFreeAsync(p, ctx->stream); };
   // one word: set by a row whose links differ from its node's current ones
-  uint32_t* d_links = nullptr;
-  if (cudaMallocAsync((void**)&d_links, 256, ctx->stream) != cudaSuccess) { free_scratch(); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(apply_rows flag)"); }
-  scratch.push_back(d_links);
+  scratch.emplace_back(ctx->stream);
+  if (!scratch.back().alloc(256)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(apply_rows flag)");
+  uint32_t* d_links = reinterpret_cast<uint32_t*>(scratch.back().p);
   cudaMemsetAsync(d_links, 0, sizeof(uint32_t), ctx->stream);
   bool root_changed = false;
   int row0 = 0;
@@ -270,14 +268,15 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
     dphy_emat_host& e = views[k];
     std::memset(&e, 0, sizeof(e));
     e.num_nodes = n; e.root = new_roots ? new_roots[k] : R.root; e.includes_run_root = fo->trees[k].includes_run_root;
-    if (e.root < 0 || e.root >= n) { free_scratch(); return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "apply_rows: new root out of range"); }
-    int64_t M = R.num_muts, I = R.num_ivls, F = R.num_fs;
+    if (e.root < 0 || e.root >= n) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "apply_rows: new root out of range");
+    // the host mirror of the list lengths is updated only once the rebuild has succeeded (a node has at most one row per tree)
+    int64_t M = R.num_muts, I = R.num_ivls, F = R.num_fs, root_m = fo->cnt_mut[k][e.root];
     for (int j : by_tree[k]) {
       const dphy_node_row& r = rows[j];
       M += r.n_muts - fo->cnt_mut[k][r.node]; I += r.n_miss - fo->cnt_miss[k][r.node]; F += r.n_fs - fo->cnt_fs[k][r.node];
-      fo->cnt_mut[k][r.node] = r.n_muts; fo->cnt_miss[k][r.node] = r.n_miss; fo->cnt_fs[k][r.node] = r.n_fs;
+      if (r.node == e.root) root_m = r.n_muts;
     }
-    totals[k] = {M, I, F, fo->cnt_mut[k][e.root]};
+    totals[k] = {M, I, F, root_m};
     const int nrows = (int)by_tree[k].size();
     if (nrows == 0) {
       // untouched tree: re-flattened from the arrays it already has
@@ -287,25 +286,23 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
       e.fs_off = R.fs_off; e.fs_site = R.fs_site; e.fs_from = R.fs_from;
       continue;
     }
-    size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t at = o; o = al256(o + std::max<size_t>(bytes, 1)); return at; };
-    const size_t a_par = take(4 * (size_t)n), a_c0 = take(4 * (size_t)n), a_c1 = take(4 * (size_t)n), a_t = take(8 * (size_t)n);
-    const size_t a_moff = take(4 * ((size_t)n + 1)), a_msite = take(4 * M), a_mfrom = take(M), a_mto = take(M), a_mt = take(8 * M);
-    const size_t a_ioff = take(4 * ((size_t)n + 1)), a_is = take(4 * I), a_ie = take(4 * I);
-    const size_t a_foff = take(4 * ((size_t)n + 1)), a_fsite = take(4 * F), a_ffrom = take(F), a_map = take(4 * (size_t)n);
+    Slab raw;
+    const int a_par = raw.reserve(4 * (size_t)n), a_c0 = raw.reserve(4 * (size_t)n), a_c1 = raw.reserve(4 * (size_t)n), a_t = raw.reserve(8 * (size_t)n);
+    const int a_moff = raw.reserve(4 * ((size_t)n + 1)), a_msite = raw.reserve(4 * M), a_mfrom = raw.reserve(M), a_mto = raw.reserve(M), a_mt = raw.reserve(8 * M);
+    const int a_ioff = raw.reserve(4 * ((size_t)n + 1)), a_is = raw.reserve(4 * I), a_ie = raw.reserve(4 * I);
+    const int a_foff = raw.reserve(4 * ((size_t)n + 1)), a_fsite = raw.reserve(4 * F), a_ffrom = raw.reserve(F), a_map = raw.reserve(4 * (size_t)n);
     const int ntiles = (n + kDeltaTile - 1) / kDeltaTile;
-    const size_t a_tt = take(4 * 3 * (size_t)ntiles);
-    char* nb = nullptr;
-    if (cudaMallocAsync((void**)&nb, o, ctx->stream) != cudaSuccess) { free_scratch(); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(raw rebuild)"); }
-    scratch.push_back(nb);
+    const int a_tt = raw.reserve(4 * 3 * (size_t)ntiles);
+    scratch.emplace_back(ctx->stream);
+    if (!scratch.back().alloc(raw.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(raw rebuild)");
+    char* nb = scratch.back().p;
     RawTreeOut out{};
-    out.parent = (int32_t*)(nb + a_par); out.child0 = (int32_t*)(nb + a_c0); out.child1 = (int32_t*)(nb + a_c1); out.t = (double*)(nb + a_t);
-    out.mut_off = (int32_t*)(nb + a_moff); out.mut_site = (int32_t*)(nb + a_msite); out.mut_from = (uint8_t*)(nb + a_mfrom);
-    out.mut_to = (uint8_t*)(nb + a_mto); out.mut_t = (double*)(nb + a_mt);
-    out.miss_off = (int32_t*)(nb + a_ioff); out.miss_start = (int32_t*)(nb + a_is); out.miss_end = (int32_t*)(nb + a_ie);
-    out.fs_off = (int32_t*)(nb + a_foff); out.fs_site = (int32_t*)(nb + a_fsite); out.fs_from = (uint8_t*)(nb + a_ffrom);
-    int32_t* row_of = (int32_t*)(nb + a_map);
-    jobs.push_back({R, out, row_of, (int32_t*)(nb + a_tt), n, ntiles, row0, nrows});
+    out.parent = raw.at<int32_t>(nb, a_par); out.child0 = raw.at<int32_t>(nb, a_c0); out.child1 = raw.at<int32_t>(nb, a_c1); out.t = raw.at<double>(nb, a_t);
+    out.mut_off = raw.at<int32_t>(nb, a_moff); out.mut_site = raw.at<int32_t>(nb, a_msite); out.mut_from = raw.at<uint8_t>(nb, a_mfrom);
+    out.mut_to = raw.at<uint8_t>(nb, a_mto); out.mut_t = raw.at<double>(nb, a_mt);
+    out.miss_off = raw.at<int32_t>(nb, a_ioff); out.miss_start = raw.at<int32_t>(nb, a_is); out.miss_end = raw.at<int32_t>(nb, a_ie);
+    out.fs_off = raw.at<int32_t>(nb, a_foff); out.fs_site = raw.at<int32_t>(nb, a_fsite); out.fs_from = raw.at<uint8_t>(nb, a_ffrom);
+    jobs.push_back({R, out, raw.at<int32_t>(nb, a_map), raw.at<int32_t>(nb, a_tt), n, ntiles, row0, nrows});
     row0 += nrows;
     e.parent = out.parent; e.child0 = out.child0; e.child1 = out.child1; e.t = out.t;
     e.mut_off = out.mut_off; e.mut_site = out.mut_site; e.mut_from = out.mut_from; e.mut_to = out.mut_to; e.mut_t = out.mut_t;
@@ -352,10 +349,12 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
   const bool same_links = links == 0u && !root_changed;
   // ---- re-flatten from the device-resident arrays (the same kernels as an upload; validation included) ----------------------------------------------
   if (st == DPHY_OK) st = rebuild_forest_from_device(ctx, fo, views.data(), totals.data(), same_links);
-  free_scratch();
-  if (st != DPHY_OK) {
-    // the forest is unchanged (the rebuild swaps only on success), but the host mirror of the list lengths is now ahead of it
-    fo->cnt_mut.clear(); fo->cnt_miss.clear(); fo->cnt_fs.clear();
-  }
-  return st;
+  scratch.clear();
+  if (st != DPHY_OK) return st;
+  for (int k = 0; k < nt; ++k)
+    for (int j : by_tree[k]) {
+      const dphy_node_row& r = rows[j];
+      fo->cnt_mut[k][r.node] = r.n_muts; fo->cnt_miss[k][r.node] = r.n_miss; fo->cnt_fs[k][r.node] = r.n_fs;
+    }
+  return DPHY_OK;
 }

@@ -499,8 +499,6 @@ __global__ void __launch_bounds__(kPlaceWarps * 32, 2) place_samples_kernel(Plac
 }
 
 namespace {
-size_t al(size_t x) { return (x + 255) / 256 * 256; }
-int bits_for(int64_t max_value) { int b = 1; while (b < 31 && ((int64_t)1 << b) <= max_value) ++b; return b; }
 
 // the per-tree index: built by the first placement on the tree, freed with the forest (dphy_forest_apply_rows swaps in a fresh forest,
 // so a rebuilt tree gets a fresh index; dphy_forest_set_node_times changes no entry, the times are read when the records are made)
@@ -521,21 +519,19 @@ int ensure_place_index(dphy_ctx* ctx, dphy_forest* fo, int tree) {
   int64_t P2 = 1;
   while (P2 < R) P2 <<= 1;
   // resident: site_off [L+1], rec [M], seg [2 P2]; temporaries (freed once built): fill [L], diff [R+2], scan tiles
-  const size_t b_so = 0, b_rec = al(sizeof(int32_t) * (L + 1)), b_seg = b_rec + al(sizeof(int4) * std::max<int64_t>(M, 1));
-  const size_t total = b_seg + al(sizeof(int2) * 2 * P2);
-  const size_t b_fill = 0, b_diff = al(sizeof(int32_t) * L), b_tt = b_diff + al(sizeof(int32_t) * (R + 2));
-  const size_t tmp_bytes = b_tt + al(sizeof(int32_t) * ((std::max<int64_t>(L, R + 1) + 1) / 8192 + 2));
-  char* d = nullptr;
-  char* tmp = nullptr;
-  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index)");
-  if (cudaMallocAsync((void**)&tmp, tmp_bytes, ctx->stream) != cudaSuccess) {
-    cudaFreeAsync(d, ctx->stream);
-    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index scratch)");
-  }
-  int32_t* so = (int32_t*)(d + b_so); int4* rec = (int4*)(d + b_rec); int2* seg = (int2*)(d + b_seg);
-  int32_t* fill = (int32_t*)(tmp + b_fill); int32_t* diff = (int32_t*)(tmp + b_diff); int32_t* tt = (int32_t*)(tmp + b_tt);
-  int st = check_cuda(ctx, cudaMemsetAsync(d, 0, b_rec, ctx->stream), "place index memset");
-  if (st == DPHY_OK) st = check_cuda(ctx, cudaMemsetAsync(tmp, 0, b_tt, ctx->stream), "place index memset");
+  Slab res, work;
+  const int b_so = res.reserve(sizeof(int32_t) * (L + 1)), b_rec = res.reserve(sizeof(int4) * std::max<int64_t>(M, 1));
+  const int b_seg = res.reserve(sizeof(int2) * 2 * P2);
+  const int b_fill = work.reserve(sizeof(int32_t) * L), b_diff = work.reserve(sizeof(int32_t) * (R + 2));
+  const int b_tt = work.reserve(sizeof(int32_t) * ((std::max<int64_t>(L, R + 1) + 1) / 8192 + 2));
+  DevBlock d(ctx->stream), tmp(ctx->stream);
+  if (!d.alloc(res.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index)");
+  if (!tmp.alloc(work.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place index scratch)");
+  int32_t* so = res.at<int32_t>(d.p, b_so); int4* rec = res.at<int4>(d.p, b_rec); int2* seg = res.at<int2>(d.p, b_seg);
+  int32_t* fill = work.at<int32_t>(tmp.p, b_fill); int32_t* diff = work.at<int32_t>(tmp.p, b_diff); int32_t* tt = work.at<int32_t>(tmp.p, b_tt);
+  // site_off, fill and diff start at zero
+  int st = check_cuda(ctx, cudaMemsetAsync(d.p, 0, res.blocks[b_rec].off, ctx->stream), "place index memset");
+  if (st == DPHY_OK) st = check_cuda(ctx, cudaMemsetAsync(tmp.p, 0, work.blocks[b_tt].off, ctx->stream), "place index memset");
   if (st == DPHY_OK) {
     const int m0 = h_mo[0], Mi = (int)M;
     if (Mi > 0) place_site_hist_kernel<<<(Mi + 255) / 256, 256, 0, ctx->stream>>>(fo->h, m0, Mi, so);
@@ -553,12 +549,12 @@ int ensure_place_index(dphy_ctx* ctx, dphy_forest* fo, int tree) {
   std::vector<int32_t> h_so(L + 1);
   if (st == DPHY_OK) st = check_cuda(ctx, cudaMemcpyAsync(h_so.data(), so, sizeof(int32_t) * (L + 1), cudaMemcpyDeviceToHost, ctx->stream), "D2H");
   if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "place index build");
-  cudaFreeAsync(tmp, ctx->stream);
-  if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return st; }
-  fo->allocs.push_back(d);
-  fo->bytes += total;
+  tmp.reset();
+  if (st != DPHY_OK) return st;
+  fo->allocs.push_back(d.release());
+  fo->bytes += res.total;
   X.R = (int32_t)R; X.P2 = (int32_t)P2; X.L = L;
-  X.site_off = so; X.rec = rec; X.seg = seg; X.bytes = total;
+  X.site_off = so; X.rec = rec; X.seg = seg; X.bytes = res.total;
   X.h_site_off = std::move(h_so);
   return DPHY_OK;
 }
@@ -604,33 +600,27 @@ int ensure_dated_index(dphy_ctx* ctx, dphy_forest* fo, int tree, uint64_t ver) {
                                                  (int32_t*)nullptr, R, 0, 64, ctx->stream));
   DPHY_CUDA(ctx, cub::DeviceScan::InclusiveScanByKey(nullptr, scan_bytes, thrust::counting_iterator<int>(0), (const DatedAcc*)nullptr,
                                                      (DatedAcc*)nullptr, DatedComb{}, P2, SameNode{1}, ctx->stream));
-  const size_t b_lc = al(sizeof(double) * R), b_pre = b_lc + al(sizeof(int32_t) * (size_t)lg * P2);
-  const size_t total = b_pre + al(sizeof(int2) * (size_t)lg * P2);
+  Slab res, work;
+  const int b_tkey = res.reserve(sizeof(double) * R), b_lc = res.reserve(sizeof(int32_t) * (size_t)lg * P2);
+  const int b_pre = res.reserve(sizeof(int2) * (size_t)lg * P2);
   // temporaries: unsorted keys, region indices, two level lists, scan input and output, CUB's storage
-  const size_t b_idx = al(sizeof(double) * R), b_l0 = b_idx + al(sizeof(int32_t) * R), b_l1 = b_l0 + al(sizeof(int32_t) * P2);
-  const size_t b_vin = b_l1 + al(sizeof(int32_t) * P2), b_vout = b_vin + al(sizeof(DatedAcc) * P2), b_cub = b_vout + al(sizeof(DatedAcc) * P2);
-  const size_t tmp_bytes = b_cub + al(std::max(sort_bytes, scan_bytes));
-  char* d = (char*)X.tkey;
-  const bool fresh = d == nullptr;
-  if (fresh && cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) {
-    cudaGetLastError();
-    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index)");
-  }
-  char* tmp = nullptr;
-  if (cudaMallocAsync((void**)&tmp, tmp_bytes, ctx->stream) != cudaSuccess) {
-    cudaGetLastError();
-    if (fresh) cudaFreeAsync(d, ctx->stream);
-    return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index scratch)");
-  }
+  const int b_key = work.reserve(sizeof(double) * R), b_idx = work.reserve(sizeof(int32_t) * R), b_l0 = work.reserve(sizeof(int32_t) * P2);
+  const int b_l1 = work.reserve(sizeof(int32_t) * P2), b_vin = work.reserve(sizeof(DatedAcc) * P2), b_vout = work.reserve(sizeof(DatedAcc) * P2);
+  const int b_cub = work.reserve(std::max(sort_bytes, scan_bytes));
+  DevBlock d(ctx->stream), tmp(ctx->stream);
+  const bool fresh = X.tkey == nullptr;
+  if (fresh && !d.alloc(res.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index)");
+  if (!tmp.alloc(work.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(dated place index scratch)");
   if (fresh) {
-    fo->allocs.push_back(d);
-    fo->bytes += total;
-    X.tkey = (double*)d; X.lc = (int32_t*)(d + b_lc); X.pre = (int2*)(d + b_pre); X.dated_bytes = total; X.lg = lg;
+    fo->allocs.push_back(d.release());
+    fo->bytes += res.total;
+    void* base = fo->allocs.back();
+    X.tkey = res.at<double>(base, b_tkey); X.lc = res.at<int32_t>(base, b_lc); X.pre = res.at<int2>(base, b_pre); X.dated_bytes = res.total; X.lg = lg;
   }
   X.dated_at = ~0ull;                       // not valid until the build below has finished
-  double* key = (double*)tmp; int32_t* idx = (int32_t*)(tmp + b_idx);
-  int32_t* list = (int32_t*)(tmp + b_l0); int32_t* next = (int32_t*)(tmp + b_l1);
-  DatedAcc* vin = (DatedAcc*)(tmp + b_vin); DatedAcc* vout = (DatedAcc*)(tmp + b_vout); void* cub_tmp = tmp + b_cub;
+  double* key = work.at<double>(tmp.p, b_key); int32_t* idx = work.at<int32_t>(tmp.p, b_idx);
+  int32_t* list = work.at<int32_t>(tmp.p, b_l0); int32_t* next = work.at<int32_t>(tmp.p, b_l1);
+  DatedAcc* vin = work.at<DatedAcc>(tmp.p, b_vin); DatedAcc* vout = work.at<DatedAcc>(tmp.p, b_vout); void* cub_tmp = work.at<char>(tmp.p, b_cub);
   place_tkey_kernel<<<(T.num_nodes + 255) / 256, 256, 0, ctx->stream>>>(fo->h, T.node_base, T.num_nodes, key, idx);
   if (P2 > R) place_pad_list_kernel<<<(P2 - R + 255) / 256, 256, 0, ctx->stream>>>(list, R, P2);
   // every CUB call below is counted as one launch
@@ -651,7 +641,7 @@ int ensure_dated_index(dphy_ctx* ctx, dphy_forest* fo, int tree, uint64_t ver) {
   int st = check_cuda(ctx, ce, "dated place index");
   if (st == DPHY_OK) st = check_cuda(ctx, cudaGetLastError(), "dated place index kernels");
   if (st == DPHY_OK) st = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "dated place index build");
-  cudaFreeAsync(tmp, ctx->stream);
+  tmp.reset();
   if (st == DPHY_OK) X.dated_at = ver;
   return st;
 }
@@ -722,49 +712,52 @@ int place_samples(dphy_ctx* ctx, dphy_forest* fo, int32_t tree, const dphy_sampl
   }
   cuts.push_back(S);
   // ---- inputs through the pinned slab; outputs back through it ----
-  const size_t b_doff = 0, b_moff = al(4 * (size_t)(S + 1)), b_ds = b_moff + al(4 * (size_t)(S + 1)), b_dt = b_ds + al(4 * (size_t)D);
-  const size_t b_ms = b_dt + al((size_t)D), b_me = b_ms + al(4 * (size_t)I), b_scr = b_me + al(4 * (size_t)I);
-  const size_t b_tx = b_scr + al(8 * (size_t)(S + 1)), in_bytes = b_tx + (dated ? al(8 * (size_t)S) : 0);
-  const size_t b_out = in_bytes, b_best = b_out + al(sizeof(dphy_placement) * (size_t)S);
-  const size_t io_bytes = b_best + al(sizeof(dphy_candidate_region) * (size_t)S * max_best);
-  const size_t b_scratch = io_bytes, total = b_scratch + al(4 * (size_t)max_words);
-  char* d = nullptr;
-  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place)");
-  void* hv = nullptr;
-  st = acquire_pinned(ctx, io_bytes, &hv);
-  if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return st; }
-  char* h = (char*)hv;
-  int32_t* h_doff = (int32_t*)(h + b_doff); int32_t* h_moff = (int32_t*)(h + b_moff);
+  // [inputs | outputs] cross through the pinned slab, the per-sample scratch stays on the device
+  Slab slab;
+  const int b_doff = slab.reserve(4 * (size_t)(S + 1)), b_moff = slab.reserve(4 * (size_t)(S + 1)), b_ds = slab.reserve(4 * (size_t)D);
+  const int b_dt = slab.reserve((size_t)D), b_ms = slab.reserve(4 * (size_t)I), b_me = slab.reserve(4 * (size_t)I);
+  const int b_scr = slab.reserve(8 * (size_t)(S + 1)), b_tx = dated ? slab.reserve(8 * (size_t)S) : -1;
+  const size_t in_bytes = slab.total;
+  const int b_out = slab.reserve(sizeof(dphy_placement) * (size_t)S), b_best = slab.reserve(sizeof(dphy_candidate_region) * (size_t)S * max_best);
+  const size_t io_bytes = slab.total;
+  const int b_scratch = slab.reserve(4 * (size_t)max_words);
+  DevBlock blk(ctx->stream);
+  if (!blk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(place)");
+  char* d = blk.p;
+  PinnedStage pin(ctx, io_bytes);
+  if (pin.status != DPHY_OK) return pin.status;
+  char* h = pin.p;
+  int32_t* h_doff = slab.at<int32_t>(h, b_doff); int32_t* h_moff = slab.at<int32_t>(h, b_moff);
   for (int k = 0; k <= S; ++k) { h_doff[k] = dof[k] - dof[0]; h_moff[k] = mof[k] - mof[0]; }
-  if (D) { std::memcpy(h + b_ds, set->delta_site + dof[0], 4 * D); std::memcpy(h + b_dt, set->delta_to + dof[0], D); }
-  if (I) { std::memcpy(h + b_ms, set->miss_start + mof[0], 4 * I); std::memcpy(h + b_me, set->miss_end + mof[0], 4 * I); }
-  std::memcpy(h + b_scr, scr.data(), 8 * (size_t)(S + 1));
-  if (dated) std::memcpy(h + b_tx, t_X, 8 * (size_t)S);
+  if (D) { std::memcpy(slab.at<char>(h, b_ds), set->delta_site + dof[0], 4 * D); std::memcpy(slab.at<char>(h, b_dt), set->delta_to + dof[0], D); }
+  if (I) { std::memcpy(slab.at<char>(h, b_ms), set->miss_start + mof[0], 4 * I); std::memcpy(slab.at<char>(h, b_me), set->miss_end + mof[0], 4 * I); }
+  std::memcpy(slab.at<char>(h, b_scr), scr.data(), 8 * (size_t)(S + 1));
+  if (dated) std::memcpy(slab.at<char>(h, b_tx), t_X, 8 * (size_t)S);
   cudaError_t ce = cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
   PlaceParams P;
   std::memset(&P, 0, sizeof(P));
   P.f = fo->h; P.nb = T.node_base; P.N = T.num_nodes; P.R = X.R; P.P2 = X.P2; P.L = L;
   P.site_bits = bits_for(L); P.pos_bits = bits_for(X.R); P.can_change_root = can_change_root != 0; P.max_best = max_best;
   P.site_off = X.site_off; P.rec = X.rec; P.seg = X.seg; P.ref = fo->sites[T.sites_id]->d_ref;
-  if (dated) P.t_X = (const double*)(d + b_tx);
+  if (dated) P.t_X = slab.at<const double>(d, b_tx);
   if (use_dated) { P.tkey = X.tkey; P.lc = X.lc; P.pre = X.pre; P.lg = X.lg; }
-  P.delta_off = (const int32_t*)(d + b_doff); P.delta_site = (const int32_t*)(d + b_ds); P.delta_to = (const uint8_t*)(d + b_dt);
-  P.miss_off = (const int32_t*)(d + b_moff); P.miss_start = (const int32_t*)(d + b_ms); P.miss_end = (const int32_t*)(d + b_me);
-  P.scr_off = (const int64_t*)(d + b_scr); P.scratch = (uint32_t*)(d + b_scratch);
-  P.out = (dphy_placement*)(d + b_out); P.best = (dphy_candidate_region*)(d + b_best);
+  P.delta_off = slab.at<const int32_t>(d, b_doff); P.delta_site = slab.at<const int32_t>(d, b_ds); P.delta_to = slab.at<const uint8_t>(d, b_dt);
+  P.miss_off = slab.at<const int32_t>(d, b_moff); P.miss_start = slab.at<const int32_t>(d, b_ms); P.miss_end = slab.at<const int32_t>(d, b_me);
+  P.scr_off = slab.at<const int64_t>(d, b_scr); P.scratch = slab.at<uint32_t>(d, b_scratch);
+  P.out = slab.at<dphy_placement>(d, b_out); P.best = slab.at<dphy_candidate_region>(d, b_best);
   for (size_t c = 0; c + 1 < cuts.size() && ce == cudaSuccess; ++c) {
     P.s0 = cuts[c]; P.s1 = cuts[c + 1];
     place_samples_kernel<<<(P.s1 - P.s0 + kPlaceWarps - 1) / kPlaceWarps, kPlaceWarps * 32, 0, ctx->stream>>>(P);
     ++ctx->launches;
     ce = cudaGetLastError();
   }
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(h + b_out, d + b_out, io_bytes - b_out, cudaMemcpyDeviceToHost, ctx->stream);
+  const size_t out_at = slab.blocks[b_out].off;
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(h + out_at, d + out_at, io_bytes - out_at, cudaMemcpyDeviceToHost, ctx->stream);
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-  cudaFreeAsync(d, ctx->stream);
-  if (ce != cudaSuccess) { release_pinned_async(ctx); return check_cuda(ctx, ce, "place samples"); }
-  std::memcpy(out, h + b_out, sizeof(dphy_placement) * (size_t)S);
-  if (max_best > 0) std::memcpy(best, h + b_best, sizeof(dphy_candidate_region) * (size_t)S * max_best);
-  release_pinned_async(ctx);
+  blk.reset();
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "place samples");
+  std::memcpy(out, slab.at<char>(h, b_out), sizeof(dphy_placement) * (size_t)S);
+  if (max_best > 0) std::memcpy(best, slab.at<char>(h, b_best), sizeof(dphy_candidate_region) * (size_t)S * max_best);
   return DPHY_OK;
 }
 }  // namespace

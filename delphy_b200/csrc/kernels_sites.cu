@@ -195,10 +195,9 @@ int launch_sites_derive(dphy_ctx* ctx, dphy_sites* s, bool with_nu_tables) {
 // mu / pi / q changed on every table of `tables` (site rates untouched): one launch, one cluster per table
 int launch_sites_derive_many(dphy_ctx* ctx, dphy_sites* const* tables, int n) {
   if (n <= 0) return DPHY_OK;
-  void* hbv = nullptr;
-  int st = acquire_pinned(ctx, sizeof(DeriveArgs) * (size_t)n, &hbv);
-  if (st != DPHY_OK) return st;
-  DeriveArgs* h = static_cast<DeriveArgs*>(hbv);
+  PinnedStage pin(ctx, sizeof(DeriveArgs) * (size_t)n);
+  if (pin.status != DPHY_OK) return pin.status;
+  DeriveArgs* h = reinterpret_cast<DeriveArgs*>(pin.p);
   for (int k = 0; k < n; ++k) {
     dphy_sites* s = tables[k];
     DeriveArgs& a = h[k];
@@ -211,7 +210,7 @@ int launch_sites_derive_many(dphy_ctx* ctx, dphy_sites* const* tables, int n) {
   DeriveArgs* d = static_cast<DeriveArgs*>(ctx->arena.alloc(sizeof(DeriveArgs) * (size_t)n));
   if (!d) { ctx->arena.release(mark); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "arena exhausted (set_evo_many)"); }
   cudaError_t ce = cudaMemcpyAsync(d, h, sizeof(DeriveArgs) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream);
-  release_pinned_async(ctx);
+  pin.reset();
   if (ce == cudaSuccess) {
     sites_derive_many_kernel<<<kClusterCtas * n, kScanThreads, 0, ctx->stream>>>(d);
     ctx->launches += 1;

@@ -28,6 +28,7 @@
 #include <cstddef>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <math_constants.h>
 #include <new>
 #include <vector>
@@ -1426,33 +1427,39 @@ static int spr_join_tail(dphy_ctx* ctx, dphy_spr_batch* b) {
 }
 
 namespace {
-size_t al(size_t x) { return (x + 255) / 256 * 256; }
-
 // the study-independent tables of the event-scan path: built by the first grouped batch on a forest, freed with it
 int ensure_spr_tables(dphy_ctx* ctx, dphy_forest* fo) {
   if (fo->d_spr_eopen) return DPHY_OK;
   const size_t N = (size_t)fo->h.num_nodes, M = (size_t)fo->total_muts;
-  const size_t b_eopen = 0, b_tnode = al(sizeof(int32_t) * N), b_ev = b_tnode + al(sizeof(int32_t) * (N + M + 1));
   int max_nodes = 1;
   for (const TreeDev& T : fo->trees) max_nodes = std::max(max_nodes, T.num_nodes);
   const int max_tiles = (max_nodes + kPmTile - 1) / kPmTile;
-  const size_t b_pm = b_ev + al(sizeof(int32_t) * (2 * M + 1)), b_tt = b_pm + al(sizeof(int32_t) * N);
-  const size_t total = b_tt + al(sizeof(int32_t) * (size_t)max_tiles * fo->h.num_trees);
-  char* d = nullptr;
-  if (cudaMallocAsync((void**)&d, total, ctx->stream) != cudaSuccess) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(spr tables)");
-  int32_t* pm = (int32_t*)(d + b_pm);
-  int32_t* tt = (int32_t*)(d + b_tt);
+  Slab slab;
+  const int b_eopen = slab.reserve(sizeof(int32_t) * N), b_tnode = slab.reserve(sizeof(int32_t) * (N + M + 1));
+  const int b_ev = slab.reserve(sizeof(int32_t) * (2 * M + 1)), b_pm = slab.reserve(sizeof(int32_t) * N);
+  const int b_tt = slab.reserve(sizeof(int32_t) * (size_t)max_tiles * fo->h.num_trees);
+  DevBlock blk(ctx->stream);
+  if (!blk.alloc(slab.total)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "cudaMallocAsync(spr tables)");
+  char* d = blk.p;
+  int32_t* pm = slab.at<int32_t>(d, b_pm);
+  int32_t* tt = slab.at<int32_t>(d, b_tt);
   spr_tab_pm_kernel<<<dim3(max_tiles, fo->h.num_trees), 1024, 0, ctx->stream>>>(fo->h, pm, tt, max_tiles);
-  spr_tab_fill_kernel<<<dim3((max_nodes + 255) / 256, fo->h.num_trees), 256, 0, ctx->stream>>>(fo->h, pm, tt, max_tiles, (int32_t*)(d + b_eopen),
-                                                                                             (int32_t*)(d + b_tnode), (int32_t*)(d + b_ev));
+  spr_tab_fill_kernel<<<dim3((max_nodes + 255) / 256, fo->h.num_trees), 256, 0, ctx->stream>>>(fo->h, pm, tt, max_tiles, slab.at<int32_t>(d, b_eopen),
+                                                                                             slab.at<int32_t>(d, b_tnode), slab.at<int32_t>(d, b_ev));
   ctx->launches += 2;
   const int st = check_cuda(ctx, cudaGetLastError(), "spr table kernels launch");
-  if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); return st; }
-  fo->allocs.push_back(d);
-  fo->bytes += total;
-  fo->d_spr_eopen = (int32_t*)(d + b_eopen); fo->d_spr_tnode = (int32_t*)(d + b_tnode); fo->d_spr_ev = (int32_t*)(d + b_ev);
+  if (st != DPHY_OK) return st;
+  fo->allocs.push_back(blk.release());
+  fo->bytes += slab.total;
+  fo->d_spr_eopen = slab.at<int32_t>(d, b_eopen); fo->d_spr_tnode = slab.at<int32_t>(d, b_tnode); fo->d_spr_ev = slab.at<int32_t>(d, b_ev);
   return DPHY_OK;
 }
+
+// dphy_spr_batch_destroy as a deleter: a batch under construction is released by it on every early return
+struct BatchDestroy {
+  dphy_ctx* ctx;
+  void operator()(dphy_spr_batch* b) const { dphy_spr_batch_destroy(ctx, b); }
+};
 }
 
 extern "C" {
@@ -1463,7 +1470,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   cudaSetDevice(ctx->device);
   int st = refresh_sites(ctx, fo);
   if (st != DPHY_OK) return st;
-  auto* b = new (std::nothrow) dphy_spr_batch();
+  std::unique_ptr<dphy_spr_batch, BatchDestroy> b(new (std::nothrow) dphy_spr_batch(), BatchDestroy{ctx});
   if (!b) return DPHY_ERR_OUT_OF_MEMORY;
   b->num = n; b->forest = fo;
   b->host.resize(n);
@@ -1471,7 +1478,10 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   bool any_frontier = false, any_swept_limited = false;
   int num_bounded = 0;
   for (int i = 0; i < n; ++i) num_bounded += reqs[i].max_muts_from_start != INT_MAX;
+  // the batch's slab: per-group and per-study arrays, then the path targets.  Their offsets from b->dev.slab go straight into the
+  // group and study records, so a running offset lays them out (a Slab's block records cost measurable host time at 1,024 studies)
   size_t off = 0;
+  auto take = [&](size_t bytes) { const size_t at = off; off = align_up(off + bytes); return (int64_t)at; };
   std::vector<std::pair<size_t, const void*>> copies;   // (slab offset, host ptr) with sizes below
   std::vector<size_t> copy_bytes;
   // ---- grouping: full (unbounded) studies of the same tree go 32 at a time through the lanes-are-studies kernels ----------------
@@ -1479,7 +1489,6 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   constexpr int kMinGroup = 24;     // a group costs the same for 1 or 32 lanes: below ~24 studies the per-study kernels are cheaper
   // DPHY_SPR_GROUPED=0: every study on the per-study kernels
   static const bool use_groups = [] { const char* e = getenv("DPHY_SPR_GROUPED"); return !(e && atoi(e) == 0); }();
-  const bool g2 = use_groups;
   std::vector<int> group_of(n, -1), lane_of(n, 0);
   std::vector<SprGroupDev> groups;
   if (use_groups) {
@@ -1499,25 +1508,25 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
         G.mut_base = (int32_t)mut_base[k];
         G.num = (int32_t)std::min<size_t>(kGroup, v.size() - g0);
         for (int l = 0; l < G.num; ++l) { G.study[l] = v[g0 + l]; group_of[v[g0 + l]] = (int)groups.size(); lane_of[v[g0 + l]] = l; }
-        G.off_xT = off; off = al(off + (size_t)G.L * kGroup);
+        G.off_xT = take((size_t)G.L * kGroup);
         {
           const int64_t M = fo->tree_muts[k];
-          if (2 * M + 1 + kEvChunk > INT_MAX || (int64_t)T.num_nodes + M + 64 > INT_MAX) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: tree too large"); }
+          if (2 * M + 1 + kEvChunk > INT_MAX || (int64_t)T.num_nodes + M + 64 > INT_MAX) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: tree too large");
           G.num_muts = (int32_t)M; G.num_templates = (int32_t)(T.num_nodes + M);
           G.num_ev_chunks = (int32_t)(2 * M / kEvChunk + 1);           // rows 0 .. 2M
           G.num_t_chunks = (G.num_templates + 31) / 32;                // + one empty chunk, so that KB(N) always has a row
-          G.off_S = off; off = al(off + (size_t)G.num_ev_chunks * kEvChunk * kGroup);
-          G.off_aggS = off; off = al(off + sizeof(int32_t) * ((size_t)G.num_ev_chunks + 1) * kGroup);
-          G.off_mask = off; off = al(off + sizeof(uint32_t) * ((size_t)G.num_t_chunks + 1) * kGroup);
-          G.off_aggK = off; off = al(off + sizeof(int32_t) * ((size_t)G.num_t_chunks + 2) * kGroup);
-          G.off_cbase = off; off = al(off + sizeof(int2) * ((size_t)G.num_t_chunks + 1) * kGroup);
-          G.off_consts = off; off = al(off + 32 * kGroup + sizeof(int32_t) * kGroup);      // G2Const [32] + root_keep [32]
-          G.off_outs = off; off = al(off + 64 * kGroup);
+          G.off_S = take((size_t)G.num_ev_chunks * kEvChunk * kGroup);
+          G.off_aggS = take(sizeof(int32_t) * ((size_t)G.num_ev_chunks + 1) * kGroup);
+          G.off_mask = take(sizeof(uint32_t) * ((size_t)G.num_t_chunks + 1) * kGroup);
+          G.off_aggK = take(sizeof(int32_t) * ((size_t)G.num_t_chunks + 2) * kGroup);
+          G.off_cbase = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1) * kGroup);
+          G.off_consts = take(32 * kGroup + sizeof(int32_t) * kGroup);      // G2Const [32] + root_keep [32]
+          G.off_outs = take(64 * kGroup);
           if (g0 == 0) {
-            G.trec_owner = 1; G.off_trec = off; off = al(off + 48 * (size_t)G.num_templates);
-            G.off_csort = off; off = al(off + sizeof(double) * 32 * ((size_t)G.num_t_chunks + 1));
-            G.off_cpm = off; off = al(off + sizeof(uint32_t) * 32 * ((size_t)G.num_t_chunks + 1));
-            G.off_cq = off; off = al(off + sizeof(int2) * ((size_t)G.num_t_chunks + 1));
+            G.trec_owner = 1; G.off_trec = take(48 * (size_t)G.num_templates);
+            G.off_csort = take(sizeof(double) * 32 * ((size_t)G.num_t_chunks + 1));
+            G.off_cpm = take(sizeof(uint32_t) * 32 * ((size_t)G.num_t_chunks + 1));
+            G.off_cq = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1));
           } else {
             const SprGroupDev& G0 = groups[groups.size() - g0 / kGroup];
             G.trec_owner = 0; G.off_trec = G0.off_trec; G.off_csort = G0.off_csort; G.off_cpm = G0.off_cpm; G.off_cq = G0.off_cq;
@@ -1530,24 +1539,22 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   // (raw log-weights inside the grouped emit were measured slower than the dense weights pass over the stored heads: the two logs
   // per region then run at the emit's ~45 % lane utilisation and low occupancy, 1.26 ms vs 0.68 + 0.23 ms per 128 studies)
   // The event-scan emit computes the raw log-weights itself (DPHY_SPR_FUSE_WEIGHTS=0: dense pass over the stored heads instead)
-  static const bool fuse_env = [] { const char* e = getenv("DPHY_SPR_FUSE_WEIGHTS"); return !(e && atoi(e) == 0); }();
-  const bool fuse_weights = g2 && fuse_env;
+  static const bool fuse_weights = [] { const char* e = getenv("DPHY_SPR_FUSE_WEIGHTS"); return !(e && atoi(e) == 0); }();
   for (int i = 0; i < n; ++i) {
     const dphy_spr_request& r = reqs[i];
     SprStudy& S = b->host[i];
     std::memset(&S, 0, sizeof(S));
-    if (r.tree < 0 || r.tree >= fo->h.num_trees) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: tree index out of range"); }
+    if (r.tree < 0 || r.tree >= fo->h.num_trees) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: tree index out of range");
     const TreeDev& T = fo->trees[r.tree];
     const int L = fo->sites[T.sites_id]->L;
-    if (r.X < -1 || r.X >= T.num_nodes) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X out of range"); }
-    if (r.X == T.root_id) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: X must not be the root (CHECK_NE(X, tree->root))"); }
-    if (r.start_branch < 0 || r.start_branch >= T.num_nodes) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: start branch out of range"); }
-    if (r.start_branch == r.X) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: start region is on branch X"); }
-    if (!(r.lambda_X >= 0.0)) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: lambda_X must be >= 0 (0: enumerate only)"); }
-    if (r.x_state_mode < DPHY_SPR_X_FROM_TREE || r.x_state_mode > DPHY_SPR_X_REL_START) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: unknown x_state_mode"); }
-    if ((r.x_state_mode != DPHY_SPR_X_FROM_TREE || r.X < 0) && ((r.n_x_deltas > 0 && (!r.x_delta_site || !r.x_delta_to)) || (r.n_x_missing > 0 && (!r.x_missing_start || !r.x_missing_end)) || r.n_x_deltas < 0 || r.n_x_missing < 0)) {
-      delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: explicit X state without its arrays");
-    }
+    if (r.X < -1 || r.X >= T.num_nodes) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X out of range");
+    if (r.X == T.root_id) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: X must not be the root (CHECK_NE(X, tree->root))");
+    if (r.start_branch < 0 || r.start_branch >= T.num_nodes) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: start branch out of range");
+    if (r.start_branch == r.X) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: start region is on branch X");
+    if (!(r.lambda_X >= 0.0)) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: lambda_X must be >= 0 (0: enumerate only)");
+    if (r.x_state_mode < DPHY_SPR_X_FROM_TREE || r.x_state_mode > DPHY_SPR_X_REL_START) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: unknown x_state_mode");
+    if ((r.x_state_mode != DPHY_SPR_X_FROM_TREE || r.X < 0) && ((r.n_x_deltas > 0 && (!r.x_delta_site || !r.x_delta_to)) || (r.n_x_missing > 0 && (!r.x_missing_start || !r.x_missing_end)) || r.n_x_deltas < 0 || r.n_x_missing < 0))
+      return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: explicit X state without its arrays");
     S.tree = r.tree; S.X = r.X; S.start_branch = r.start_branch; S.start_mut_idx = r.start_mut_idx;
     S.init_min_muts = r.init_min_muts; S.limit = r.max_muts_from_start; S.can_change_root = r.can_change_root != 0;
     S.t_X = r.t_X; S.lambda_X = r.lambda_X; S.f = r.annealing_factor; S.t_max_tip = r.t_max_tip;
@@ -1555,9 +1562,9 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     const bool explicit_x = S.x_mode != DPHY_SPR_X_FROM_TREE;
     S.n_x_deltas = explicit_x ? r.n_x_deltas : 0; S.n_x_missing = explicit_x ? r.n_x_missing : 0;
     for (int k = 0; k < S.n_x_deltas; ++k)
-      if (r.x_delta_site[k] < 0 || r.x_delta_site[k] >= L || r.x_delta_to[k] > 3) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X delta out of range"); }
+      if (r.x_delta_site[k] < 0 || r.x_delta_site[k] >= L || r.x_delta_to[k] > 3) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X delta out of range");
     for (int k = 0; k < S.n_x_missing; ++k)
-      if (r.x_missing_start[k] < 0 || r.x_missing_end[k] > L || r.x_missing_start[k] >= r.x_missing_end[k]) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X missing interval out of range"); }
+      if (r.x_missing_start[k] < 0 || r.x_missing_end[k] > L || r.x_missing_start[k] >= r.x_missing_end[k]) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X missing interval out of range");
     const int N = T.num_nodes;
     const bool grouped = group_of[i] >= 0;
     // bounded studies of a small radius walk their ball (kernels_spr_frontier.cuh; DPHY_SPR_FRONTIER=0: the per-study sweeps instead)
@@ -1571,7 +1578,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     any_swept_limited |= !grouped && !frontier && r.max_muts_from_start != INT_MAX;
     S.h_stride = grouped ? kGroup : (frontier ? 0 : 1); S.tile_shift = grouped ? 5 : 8;
     S.num_htiles = grouped ? 1 : T.num_tiles;
-    if (grouped && g2) {
+    if (grouped) {
       const SprGroupDev& G = groups[group_of[i]];
       S.g2 = 1; S.g2_lane = lane_of[i]; S.g2_mut_base = G.mut_base; S.g2_num_templates = G.num_templates;
       S.off_g2S = G.off_S; S.off_g2aggS = G.off_aggS; S.off_g2mask = G.off_mask; S.off_g2aggK = G.off_aggK; S.off_g2cbase = G.off_cbase;
@@ -1581,35 +1588,35 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     if (!grouped && !frontier) max_tiles256 = std::max(max_tiles256, T.num_tiles);
     // exact upper bound on regions: every non-root node has n+1 regions, the root has 1
     const int64_t cap64 = (int64_t)N + fo->tree_muts[r.tree] + 1;
-    if (cap64 > INT_MAX) { delete b; return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: region capacity overflow"); }
+    if (cap64 > INT_MAX) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: region capacity overflow");
     S.region_cap = (int32_t)cap64;
     S.path_cap = fo->tree_max_depth[r.tree] + 2;
-    S.off_xtab = off; off = al(off + L);
-    S.off_xkey = off; off = al(off + sizeof(uint32_t) * (size_t)L);
-    S.off_path = off; off = al(off + sizeof(int32_t) * S.path_cap);
-    S.off_xpath = off; off = al(off + sizeof(int32_t) * S.path_cap);
-    S.off_pae = off; off = al(off + sizeof(int2) * S.path_cap);
-    if (grouped && g2) {
+    S.off_xtab = take(L);
+    S.off_xkey = take(sizeof(uint32_t) * (size_t)L);
+    S.off_path = take(sizeof(int32_t) * S.path_cap);
+    S.off_xpath = take(sizeof(int32_t) * S.path_cap);
+    S.off_pae = take(sizeof(int2) * S.path_cap);
+    if (grouped) {
       S.off_H = 0; S.off_C = 0; S.off_KB = 0;          // unused: H and KB are read off the group's event rows / keep masks
     } else {
-      S.off_H = off; off = al(off + sizeof(int32_t) * N);
-      S.off_C = off; off = al(off + sizeof(int32_t) * N);
-      S.off_KB = off; off = al(off + sizeof(int32_t) * (N + 1));
+      S.off_H = take(sizeof(int32_t) * N);
+      S.off_C = take(sizeof(int32_t) * N);
+      S.off_KB = take(sizeof(int32_t) * (N + 1));
     }
-    S.off_seg = off; off = al(off + sizeof(int32_t) * kSegStride * (size_t)S.path_cap);
-    S.off_hang = off; if (grouped && g2) off = al(off + sizeof(int32_t) * (size_t)S.path_cap);
+    S.off_seg = take(sizeof(int32_t) * kSegStride * (size_t)S.path_cap);
+    S.off_hang = grouped ? take(sizeof(int32_t) * (size_t)S.path_cap) : (int64_t)off;
     // chunks that straddle a segment boundary of the study: at most two per path node
-    S.hmix_cap = (grouped && g2) ? 2 * S.path_cap + 2 : 0;
-    S.off_hmix = off; off = al(off + sizeof(int32_t) * 32 * (size_t)S.hmix_cap);
-    S.off_part = off; off = al(off + sizeof(double) * kNormBlocks);
-    S.off_tj = off; off = al(off + sizeof(int2) * (size_t)T.num_tiles);       // classify() of the first / last node of every tile
-    S.off_xd_site = off; off = al(off + sizeof(int32_t) * std::max(1, S.n_x_deltas));
-    S.off_xd_to = off; off = al(off + std::max(1, S.n_x_deltas));
-    S.off_xm_start = off; off = al(off + sizeof(int32_t) * std::max(1, S.n_x_missing));
-    S.off_xm_end = off; off = al(off + sizeof(int32_t) * std::max(1, S.n_x_missing));
-    S.off_regions = off; off = al(off + sizeof(RegionHead) * (size_t)S.region_cap);
-    S.off_nw = off; off = al(off + sizeof(double2) * (size_t)S.region_cap);
-    S.off_lw = off; off = al(off + sizeof(double) * (size_t)S.region_cap);     // raw log-weights between emit and normalise
+    S.hmix_cap = grouped ? 2 * S.path_cap + 2 : 0;
+    S.off_hmix = take(sizeof(int32_t) * 32 * (size_t)S.hmix_cap);
+    S.off_part = take(sizeof(double) * kNormBlocks);
+    S.off_tj = take(sizeof(int2) * (size_t)T.num_tiles);       // classify() of the first / last node of every tile
+    S.off_xd_site = take(sizeof(int32_t) * std::max(1, S.n_x_deltas));
+    S.off_xd_to = take(std::max(1, S.n_x_deltas));
+    S.off_xm_start = take(sizeof(int32_t) * std::max(1, S.n_x_missing));
+    S.off_xm_end = take(sizeof(int32_t) * std::max(1, S.n_x_missing));
+    S.off_regions = take(sizeof(RegionHead) * (size_t)S.region_cap);
+    S.off_nw = take(sizeof(double2) * (size_t)S.region_cap);
+    S.off_lw = take(sizeof(double) * (size_t)S.region_cap);     // raw log-weights between emit and normalise
     if (S.n_x_deltas) {
       copies.push_back({(size_t)S.off_xd_site, r.x_delta_site}); copy_bytes.push_back(sizeof(int32_t) * S.n_x_deltas);
       copies.push_back({(size_t)S.off_xd_to, r.x_delta_to}); copy_bytes.push_back(S.n_x_deltas);
@@ -1633,25 +1640,23 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
       first += (int32_t)by[k].size();
     }
   }
-  const size_t off_porder = off; off = al(off + sizeof(int32_t) * std::max(1, n));
-  const size_t off_ptrees = off; off = al(off + sizeof(SprPathTree) * std::max<size_t>(1, path_trees.size()));
-  const size_t off_traw = off; off = al(off + sizeof(int32_t) * 2 * std::max(1, n));
-  const size_t off_tgt = off; off = al(off + sizeof(SprPathTarget) * 2 * std::max(1, n));
-  const size_t off_taux = off; off = al(off + sizeof(SprPathTargetAux) * 2 * std::max(1, n));
+  const size_t off_porder = take(sizeof(int32_t) * std::max(1, n));
+  const size_t off_ptrees = take(sizeof(SprPathTree) * std::max<size_t>(1, path_trees.size()));
+  const size_t off_traw = take(sizeof(int32_t) * 2 * std::max(1, n));
+  const size_t off_tgt = take(sizeof(SprPathTarget) * 2 * std::max(1, n));
+  const size_t off_taux = take(sizeof(SprPathTargetAux) * 2 * std::max(1, n));
   if (n > 0) {
     copies.push_back({off_porder, path_order.data()}); copy_bytes.push_back(sizeof(int32_t) * n);
     copies.push_back({off_ptrees, path_trees.data()}); copy_bytes.push_back(sizeof(SprPathTree) * path_trees.size());
   }
-  const size_t slab_bytes = off;
-  const size_t b_studies = 0;
-  const size_t b_agg = al(b_studies + sizeof(SprStudy) * std::max(1, n));
-  const size_t b_flag = al(b_agg + sizeof(int32_t) * 3 * ((size_t)max_tiles + 1) * std::max(1, n));
-  const size_t b_ticket = al(b_flag + 256);
-  const size_t b_groups = al(b_ticket + sizeof(uint32_t) * 4 * std::max(1, n));
-  const size_t b_slab = al(b_groups + sizeof(SprGroupDev) * std::max<size_t>(1, groups.size()));
-  const size_t total = b_slab + slab_bytes;
+  // the block: studies, look-back workspaces, flags + tickets, groups, then the slab
+  Slab hdr;
+  const int b_studies = hdr.reserve(sizeof(SprStudy) * std::max(1, n));
+  const int b_agg = hdr.reserve(sizeof(int32_t) * 3 * ((size_t)max_tiles + 1) * std::max(1, n));
+  const int b_flag = hdr.reserve(256), b_ticket = hdr.reserve(sizeof(uint32_t) * 4 * std::max(1, n));
+  const int b_groups = hdr.reserve(sizeof(SprGroupDev) * std::max<size_t>(1, groups.size()));
+  const size_t total = hdr.total + off;
   char* d = nullptr;
-  cudaError_t ce = cudaSuccess;
   size_t block_bytes = total;
   // a block left by an earlier batch (see dphy_ctx::spr_blocks): the oldest one that is large enough, once two are waiting
   if (ctx->spr_blocks.size() >= 2) {
@@ -1664,49 +1669,51 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
       break;
     }
   }
-  if (!d) ce = cudaMallocAsync((void**)&d, total, ctx->stream);
-  if (ce != cudaSuccess) { delete b; return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, std::string("cudaMallocAsync(spr batch): ") + cudaGetErrorString(ce)); }
-  b->d_block = d; b->bytes = block_bytes;
-  b->dev.studies = (SprStudy*)(d + b_studies);
-  b->dev.tile_agg = (int32_t*)(d + b_agg);
-  b->dev.tile_flag = (uint32_t*)(d + b_flag);
-  b->dev.ticket = (uint32_t*)(d + b_ticket);
-  b->dev.slab = d + b_slab;
+  if (!d) {
+    DevBlock blk(ctx->stream);
+    cudaError_t ce = cudaSuccess;
+    if (!blk.alloc(total, &ce)) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, std::string("cudaMallocAsync(spr batch): ") + cudaGetErrorString(ce));
+    d = blk.release();
+  }
+  b->d_block = d; b->bytes = block_bytes;     // from here on freed (or parked) by dphy_spr_batch_destroy
+  b->dev.studies = hdr.at<SprStudy>(d, b_studies);
+  b->dev.tile_agg = hdr.at<int32_t>(d, b_agg);
+  b->dev.tile_flag = hdr.at<uint32_t>(d, b_flag);
+  b->dev.ticket = hdr.at<uint32_t>(d, b_ticket);
+  b->dev.slab = d + hdr.total;
   b->dev.num_studies = n; b->dev.max_tiles = max_tiles; b->dev.epoch = 1;
   b->dev.g2_eopen = nullptr; b->dev.g2_tnode = nullptr; b->dev.g2_ev = nullptr; b->dev.g2_mut_off = fo->h.mut_off;
-  if (g2 && !groups.empty()) {
+  if (!groups.empty()) {
     st = ensure_spr_tables(ctx, fo);
-    if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); delete b; return st; }
+    if (st != DPHY_OK) return st;
     b->dev.g2_eopen = fo->d_spr_eopen; b->dev.g2_tnode = fo->d_spr_tnode; b->dev.g2_ev = fo->d_spr_ev;
   }
   { static const bool dry = [] { const char* e = getenv("DPHY_SPR_DRY"); return e && atoi(e) != 0; }(); if (dry) b->dev.epoch = 777u; }
-  b->d_groups = (SprGroupDev*)(d + b_groups); b->num_groups = (int32_t)groups.size();
-  if (n == 0) { *out = b; return DPHY_OK; }
+  b->d_groups = hdr.at<SprGroupDev>(d, b_groups); b->num_groups = (int32_t)groups.size();
+  if (n == 0) { *out = b.release(); return DPHY_OK; }
   // flags + tickets start at zero; studies + X overlays uploaded through the pinned staging buffer
-  ce = cudaMemsetAsync(d + b_flag, 0, b_groups - b_flag, ctx->stream);
-  size_t stage = sizeof(SprStudy) * n + al(sizeof(SprGroupDev) * groups.size());
-  for (size_t cb : copy_bytes) stage += al(cb);
+  cudaError_t ce = cudaMemsetAsync(hdr.at<char>(d, b_flag), 0, hdr.blocks[b_groups].off - hdr.blocks[b_flag].off, ctx->stream);
+  size_t stage = sizeof(SprStudy) * n + align_up(sizeof(SprGroupDev) * groups.size());
+  for (size_t cb : copy_bytes) stage += align_up(cb);
   if (ce == cudaSuccess) {
-    void* hbv = nullptr;
-    st = acquire_pinned(ctx, stage, &hbv);
-    if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); delete b; return st; }
-    char* hb = (char*)hbv;
+    PinnedStage pin(ctx, stage);
+    if (pin.status != DPHY_OK) return pin.status;
+    char* hb = pin.p;
     std::memcpy(hb, b->host.data(), sizeof(SprStudy) * n);
     ce = cudaMemcpyAsync(b->dev.studies, hb, sizeof(SprStudy) * n, cudaMemcpyHostToDevice, ctx->stream);
     size_t so = sizeof(SprStudy) * n;
     if (!groups.empty() && ce == cudaSuccess) {
       std::memcpy(hb + so, groups.data(), sizeof(SprGroupDev) * groups.size());
       ce = cudaMemcpyAsync(b->d_groups, hb + so, sizeof(SprGroupDev) * groups.size(), cudaMemcpyHostToDevice, ctx->stream);
-      so += al(sizeof(SprGroupDev) * groups.size());
+      so += align_up(sizeof(SprGroupDev) * groups.size());
     }
     for (size_t k = 0; k < copies.size() && ce == cudaSuccess; ++k) {
       std::memcpy(hb + so, copies[k].second, copy_bytes[k]);
       ce = cudaMemcpyAsync(b->dev.slab + copies[k].first, hb + so, copy_bytes[k], cudaMemcpyHostToDevice, ctx->stream);
-      so += al(copy_bytes[k]);
+      so += align_up(copy_bytes[k]);
     }
-    release_pinned_async(ctx);
   }
-  if (ce != cudaSuccess) { cudaFreeAsync(d, ctx->stream); delete b; return check_cuda(ctx, ce, "spr batch upload"); }
+  if (ce != cudaSuccess) return check_cuda(ctx, ce, "spr batch upload");
   int max_nodes = 1, group_L = 1;
   for (int i = 0; i < n; ++i) max_nodes = std::max(max_nodes, fo->trees[reqs[i].tree].num_nodes);
   for (const SprGroupDev& G : groups) group_L = std::max(group_L, G.L);
@@ -1720,12 +1727,12 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
                                                                          (SprPathTarget*)(sl + off_tgt), (SprPathTargetAux*)(sl + off_taux));
     // fork: what depends on the tree and the studies' positions alone (constants, template records, keep masks) runs on the side stream
     // while the main stream walks the latency-bound chain paths -> X tables -> event scan
-    if (ng > 0 && g2 && use_aux) {
+    if (ng > 0 && use_aux) {
       if (!ctx->aux_stream) {
         if (cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
             cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) != cudaSuccess) {
-          cudaFreeAsync(d, ctx->stream); delete b; return set_error(ctx, DPHY_ERR_CUDA, "spr: side stream");
+          return set_error(ctx, DPHY_ERR_CUDA, "spr: side stream");
         }
       }
       cudaEventRecord(ctx->ev_fork, ctx->stream);
@@ -1744,7 +1751,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     g2_templates = std::max(g2_templates, G.num_templates);
   }
   const dim3 grid_g2t((g2_t_chunks + kG2Warps - 1) / kG2Warps, std::max(ng, 1));
-  if (ng > 0 && g2) {
+  if (ng > 0) {
     cudaStream_t side = use_aux ? ctx->aux_stream : ctx->stream;
     spr_xT_kernel<<<dim3((group_L + 255) / 256, ng), 256, 0, ctx->stream>>>(b->dev, b->d_groups);
     spr_g2_consts_kernel<<<ng, kGroup, 0, side>>>(fo->h, b->dev, b->d_groups);
@@ -1779,7 +1786,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     any_weighted |= b->host[i].lambda_X > 0.0;
     any_unfused |= b->host[i].lambda_X > 0.0 && !b->host[i].weights_fused;
   }
-  const bool g2_emit = ng > 0 && g2;
+  const bool g2_emit = ng > 0;
   if (g2_emit) { spr_g2_bases_kernel<<<dim3(kGroup, ng, kBasesSlices), kBasesThreads, 0, ctx->stream>>>(b->dev, b->d_groups); ++launched; }
   // The bulk passes of a batch -- the template emit (heads + raw log-weights: issue- and bandwidth-bound), the dense weights pass if
   // any, the normalisation (bandwidth-bound) -- read the forest and write only the batch's own block: they go to the TAIL stream, so
@@ -1803,13 +1810,13 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     return DPHY_OK;
   };
   if (g2_emit) {
-    if (use_tail && tail_mode >= 2) { st = fork_tail(); if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); delete b; return st; } }
+    if (use_tail && tail_mode >= 2) { st = fork_tail(); if (st != DPHY_OK) return st; }
     if (fuse_weights) spr_g2_emit_kernel<2><<<grid_g2t, kG2Warps * 32, 0, ts>>>(fo->h, b->dev, b->d_groups);
     else spr_g2_emit_kernel<1><<<grid_g2t, kG2Warps * 32, 0, ts>>>(fo->h, b->dev, b->d_groups);
     ++launched;
   }
   if (any_weighted) {
-    if (use_tail) { st = fork_tail(); if (st != DPHY_OK) { cudaFreeAsync(d, ctx->stream); delete b; return st; } }
+    if (use_tail) { st = fork_tail(); if (st != DPHY_OK) return st; }
     if (any_unfused) { spr_weights_kernel<<<dim3(kWeightBlocks, n), 256, 0, ts>>>(fo->h, b->dev); ++launched; }
     spr_normalize_kernel<<<dim3(kNormBlocks, n), 256, 0, ts>>>(b->dev);
     ++launched;
@@ -1818,8 +1825,8 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   if (ts != ctx->stream) { cudaEventRecord(b->ev_done, ctx->tail_stream); b->tail_pending = true; ctx->tail_dirty = true; }
   ctx->launches += launched;
   st = check_cuda(ctx, cudaGetLastError(), "spr kernels launch");
-  if (st != DPHY_OK) { dphy_spr_batch_destroy(ctx, b); return st; }
-  *out = b;
+  if (st != DPHY_OK) return st;
+  *out = b.release();
   return DPHY_OK;
 }
 
@@ -1931,16 +1938,15 @@ int dphy_spr_batch_set_weights(dphy_ctx* ctx, dphy_spr_batch* b, const dphy_spr_
   { const int js = spr_join_tail(ctx, b); if (js != DPHY_OK) return js; }
   for (int i = 0; i < b->num; ++i)
     if (!(params[i].lambda_X > 0.0)) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: lambda_X must be > 0");
-  void* hbv = nullptr;
-  int st = acquire_pinned(ctx, sizeof(double) * 3 * b->num, &hbv);
-  if (st != DPHY_OK) return st;
-  double* hb = (double*)hbv;
+  PinnedStage pin(ctx, sizeof(double) * 3 * b->num);
+  if (pin.status != DPHY_OK) return pin.status;
+  double* hb = reinterpret_cast<double*>(pin.p);
   for (int i = 0; i < b->num; ++i) { hb[3 * i] = params[i].lambda_X; hb[3 * i + 1] = params[i].annealing_factor; hb[3 * i + 2] = params[i].t_max_tip; }
   const size_t mark = ctx->arena.mark();
   double* d_wp = (double*)ctx->arena.alloc(sizeof(double) * 3 * b->num);
-  if (!d_wp) { release_pinned_async(ctx); return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "arena exhausted (spr weights)"); }
+  if (!d_wp) return set_error(ctx, DPHY_ERR_OUT_OF_MEMORY, "arena exhausted (spr weights)");
   cudaError_t ce = cudaMemcpyAsync(d_wp, hb, sizeof(double) * 3 * b->num, cudaMemcpyHostToDevice, ctx->stream);
-  release_pinned_async(ctx);
+  pin.reset();
   if (ce == cudaSuccess) {
     spr_set_weight_params_kernel<<<(b->num + 127) / 128, 128, 0, ctx->stream>>>(b->forest->h, b->dev, d_wp);
     spr_weights_kernel<<<dim3(kWeightBlocks, b->num), 256, 0, ctx->stream>>>(b->forest->h, b->dev);

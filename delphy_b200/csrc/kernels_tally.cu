@@ -19,6 +19,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <optional>
 
 namespace dphy {
 
@@ -447,18 +448,20 @@ int dphy_forest_calc_site_tallies(dphy_ctx* ctx, dphy_forest* fo, int64_t ld, do
   // host for every row), then are copied out to the caller's rows
   auto drain = [&]() {
     size_t total = 0;
-    for (const auto& c : ctx->deferred_d2h) total += (c.bytes + 255) & ~(size_t)255;
-    void* hb = nullptr;
-    int r = total ? acquire_pinned(ctx, total, &hb) : DPHY_OK;
+    for (const auto& c : ctx->deferred_d2h) total += align_up(c.bytes);
+    std::optional<PinnedStage> pin;
+    if (total) pin.emplace(ctx, total);
+    int r = pin ? pin->status : DPHY_OK;
+    char* hb = pin ? pin->p : nullptr;
     size_t off = 0;
     for (const auto& c : ctx->deferred_d2h) {
-      if (r == DPHY_OK) r = check_cuda(ctx, cudaMemcpyAsync(static_cast<char*>(hb) + off, c.src, c.bytes, cudaMemcpyDeviceToHost, ctx->stream), "site tallies D2H");
-      off += (c.bytes + 255) & ~(size_t)255;
+      if (r == DPHY_OK) r = check_cuda(ctx, cudaMemcpyAsync(hb + off, c.src, c.bytes, cudaMemcpyDeviceToHost, ctx->stream), "site tallies D2H");
+      off += align_up(c.bytes);
     }
     const int r2 = check_cuda(ctx, cudaStreamSynchronize(ctx->stream), "site tallies");
     if (r == DPHY_OK && r2 == DPHY_OK) {
       off = 0;
-      for (const auto& c : ctx->deferred_d2h) { std::memcpy(c.dst, static_cast<char*>(hb) + off, c.bytes); off += (c.bytes + 255) & ~(size_t)255; }
+      for (const auto& c : ctx->deferred_d2h) { std::memcpy(c.dst, hb + off, c.bytes); off += align_up(c.bytes); }
     }
     ctx->deferred_d2h.clear();
     ctx->arena.release(mark);

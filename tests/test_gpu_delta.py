@@ -3,6 +3,8 @@ fresh upload of the edited trees -- integers (nsmn, num_muts*, SPR regions and t
 1e-12 -- after 1,000 random edits of the kinds the reference's local moves make: node displacements (core/subrun.cpp:223-231),
 branch reforms (one branch's mutation list rewritten, :316-319) and SPR regrafts (topology + times around P,
 core/spr_move.cpp:1101-1156), including regrafts that change the root."""
+import copy
+
 import numpy as np
 import pytest
 
@@ -218,6 +220,42 @@ def test_a_thousand_random_edits_match_fresh_uploads():
         with pytest.raises(db.DphyError):
             fo.apply_rows([bad])
         np.testing.assert_array_equal(fo.log_G()[2], before)
+        fo.close()
+        for t in tables:
+            t.close()
+
+
+def test_a_refused_call_changes_no_list_length():
+    """A call refused at a later tree (an out-of-range new root for tree 1) after tree 0's row was read must leave the forest's
+    record of tree 0's list lengths as it was: the same row sent again alone then builds exactly the edited forest.  The row
+    shortens a mutation list, so a length recorded by the refused call would size the rebuild for more mutations than it gets."""
+    rng = np.random.default_rng(31)
+    items = [synth(1), synth(0, seed=77, num_tips=120)]
+    with db.Context(0) as ctx:
+        tables = [db.DeviceSites(ctx, it[1]) for it in items]
+        eds = [Editable(it[0]) for it in items]
+        sidx = np.arange(len(items))
+        fo = db.Forest(ctx, [e.flat() for e in eds], tables, sites_index=sidx)
+        for _ in range(10000):                      # a reform may keep or grow the list: draw until one shortens it
+            ed = copy.deepcopy(eds[0])
+            touched = ed.reform(rng, items[0][1].num_sites)
+            if touched and len(ed.muts[min(touched)][0]) < len(eds[0].muts[min(touched)][0]):
+                break
+        else:
+            pytest.fail("no shortening reform drawn")
+        v = min(touched)
+        eds[0] = ed
+        with pytest.raises(db.DphyError):
+            fo.apply_rows([ed.row(0, v)], new_roots=[ed.root, len(eds[1].parent)])
+        fo.apply_rows([ed.row(0, v)], new_roots=[e.root for e in eds])
+        fresh = db.Forest(ctx, [e.flat() for e in eds], tables, sites_index=sidx)
+        for k in range(len(eds)):
+            got, want = fo.download_tree(k), fresh.download_tree(k)
+            assert got.root == want.root
+            for f in F:
+                np.testing.assert_array_equal(getattr(got, f), getattr(want, f), err_msg=f"tree {k}: {f}")
+        np.testing.assert_allclose(fo.log_G()[2], fresh.log_G()[2], rtol=1e-12, atol=0)
+        fresh.close()
         fo.close()
         for t in tables:
             t.close()
