@@ -95,9 +95,8 @@ int dphy_ctx_create(int device, dphy_ctx** out) {
   // kernel of one SPR batch runs next to the latency-bound set-up chain of the next, freed SM slots go to the chain first
   {
     int prio_least = 0, prio_greatest = 0;
-    static const bool prio = [] { const char* e = getenv("DPHY_MAIN_STREAM_PRIORITY"); return !e || atoi(e) != 0; }();
     cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest);
-    if (cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio ? prio_greatest : prio_least) != cudaSuccess) { delete ctx; return DPHY_ERR_CUDA; }
+    if (cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_greatest) != cudaSuccess) { delete ctx; return DPHY_ERR_CUDA; }
   }
   if (cudaEventCreateWithFlags(&ctx->pinned_ev, cudaEventDisableTiming) != cudaSuccess) { cudaStreamDestroy(ctx->stream); delete ctx; return DPHY_ERR_CUDA; }
   cudaDeviceProp prop;

@@ -310,13 +310,12 @@ extern "C" int dphy_forest_apply_rows(dphy_ctx* ctx, dphy_forest* fo, int32_t co
     e.fs_off = out.fs_off; e.fs_site = out.fs_site; e.fs_from = out.fs_from;
   }
   // Every edited tree's sequence is five small kernels (25 - 800 CTAs each): tree j runs on side stream j % 4, forked after the
-  // allocations and the payload upload on the main stream, joined before the re-flatten (DPHY_DELTA_STREAMS=0: all on the main stream)
+  // allocations and the payload upload on the main stream, joined before the re-flatten
   {
     constexpr int kS = dphy_ctx::kTallyStreams;
-    static const bool side = [] { const char* e = getenv("DPHY_DELTA_STREAMS"); return !e || atoi(e) != 0; }();
     cudaStream_t main_stream = ctx->stream;
     bool forked = false;
-    if (side && jobs.size() > 1) {
+    if (jobs.size() > 1) {
       bool ok = true;
       for (int i = 0; i < kS && ok; ++i) {
         if (!ctx->tally_streams[i]) ok = cudaStreamCreateWithFlags(&ctx->tally_streams[i], cudaStreamNonBlocking) == cudaSuccess &&

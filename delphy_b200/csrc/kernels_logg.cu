@@ -47,7 +47,6 @@ struct LogGParams {
   int32_t* sd_n;         // [num_nodes] missing-site count of the straddlers (sparse)
   const int32_t* strad_list;   // device positions of the straddlers
   int32_t num_strad;
-  int32_t debug_mask;    // profiling only (DPHY_DEBUG_MASK): 1 skip mutations, 2 intervals, 4 from-states, 8 closers
 };
 
 constexpr int kNW = kLgThreads / 32;
@@ -240,12 +239,12 @@ __device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm
 constexpr int kIvlBatch = 4;   // missation intervals in flight per node per round
 constexpr int kMutBatch = 2;   // mutations in flight per node per round
 
-template <int kMinBlocks>
-__global__ void __launch_bounds__(kLgThreads, kMinBlocks) emat_log_G_tile_kernel(const LogGParams P, const int32_t* __restrict__ tile_list) {
+// 4 resident CTAs per SM: 64 registers, no spills (5 or 6 CTAs: 48 / 40 registers, 80 / 160 bytes of spill stores)
+__global__ void __launch_bounds__(kLgThreads, 4) emat_log_G_tile_kernel(const LogGParams P, const int32_t* __restrict__ tile_list) {
   __shared__ LogGSmem sm;
   const ForestDev& f = P.f;
   const int tid = threadIdx.x;
-  const int tile = tile_list ? tile_list[blockIdx.x] : (int)blockIdx.x;
+  const int tile = tile_list[blockIdx.x];
   const int4 ct = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile));
   const int4 cl = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile) + 2);
   const int tile_start = ct.x, n_act = ct.y, node_base = ct.z;
@@ -277,7 +276,7 @@ __global__ void __launch_bounds__(kLgThreads, kMinBlocks) emat_log_G_tile_kernel
 
   // ---- per-node sums over the branch lists (list order => deterministic) -----------------------------------------------------------
   // missation intervals: -(cumQ[end] - cumQ[start]); count of sites going missing
-  if (!(P.debug_mask & 2)) {
+  {
     const int c0 = oi[1] - oi[0], c1 = oi[2] - oi[1];
     const int cmax = max(c0, c1);
     for (int j = 0; j < cmax; j += kIvlBatch) {
@@ -299,7 +298,7 @@ __global__ void __launch_bounds__(kLgThreads, kMinBlocks) emat_log_G_tile_kernel
     }
   }
   // mutations: d_i = mu nu (q_to - q_from);  e_i = d_i * t_i + log(mu nu q_from,to)   [g_node = sum e_i - t_P * sum d_i]
-  if (!(P.debug_mask & 1)) {
+  {
     const int c0 = R.om[1] - R.om[0], c1 = R.om[2] - R.om[1];
     const int cmax = max(c0, c1);
     for (int j = 0; j < cmax; j += kMutBatch) {
@@ -331,24 +330,22 @@ __global__ void __launch_bounds__(kLgThreads, kMinBlocks) emat_log_G_tile_kernel
     }
   }
   // from-state overrides of missing sites: folded per-branch state counts when the site rates are uniform, lists otherwise
-  if (!(P.debug_mask & 4)) {
-    if (uni) {
-      for (int k2 = 0; k2 < f.fsw_stride; ++k2) {
-        const double mq = __ldg(S.tab_muq + k2);
-        if (act0) R.dmi[0] += mq * (double)__ldg(f.fsw + (size_t)p0 * f.fsw_stride + k2);
-        if (act1) R.dmi[1] += mq * (double)__ldg(f.fsw + (size_t)(p0 + 1) * f.fsw_stride + k2);
-      }
-    } else {
+  if (uni) {
+    for (int k2 = 0; k2 < f.fsw_stride; ++k2) {
+      const double mq = __ldg(S.tab_muq + k2);
+      if (act0) R.dmi[0] += mq * (double)__ldg(f.fsw + (size_t)p0 * f.fsw_stride + k2);
+      if (act1) R.dmi[1] += mq * (double)__ldg(f.fsw + (size_t)(p0 + 1) * f.fsw_stride + k2);
+    }
+  } else {
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        for (int i = of[k]; i < of[k + 1]; ++i) {
-          const int code = __ldg(f.fs_code + i) & 63;
-          R.dmi[k] -= __ldg(S.munu + __ldg(f.fs_site + i)) * __ldg(S.tab_dq + code);
-        }
+    for (int k = 0; k < 2; ++k) {
+      for (int i = of[k]; i < of[k + 1]; ++i) {
+        const int code = __ldg(f.fs_code + i) & 63;
+        R.dmi[k] -= __ldg(S.munu + __ldg(f.fs_site + i)) * __ldg(S.tab_dq + code);
       }
     }
   }
-  tile_back_half<false>(P, sm, R, tile, tile_start, n_act, node_base, cl.z, (P.debug_mask & 8) ? cl.z : cl.w,
+  tile_back_half<false>(P, sm, R, tile, tile_start, n_act, node_base, cl.z, cl.w,
                         f.post_node + node_base, __ldg(cumQ + S.L));
 }
 
@@ -592,7 +589,6 @@ int launch_log_G_general(dphy_ctx* ctx, dphy_forest* fo) {
   P.sd_n = fo->d_sd_n;
   P.strad_list = fo->d_strad_list;
   P.num_strad = fo->num_strad;
-  { const char* dm = getenv("DPHY_DEBUG_MASK"); P.debug_mask = dm ? atoi(dm) : 0; }
   if (P.num_strad > 0) {
     emat_log_G_straddler_kernel<<<(P.num_strad + 127) / 128, 128, 0, ctx->stream>>>(P);
     ctx->launches += 1;
@@ -600,18 +596,10 @@ int launch_log_G_general(dphy_ctx* ctx, dphy_forest* fo) {
   // The direct-from-global tile kernel: every thread walks the short lists of its own two nodes.  (A TMA-staged persistent variant
   // -- node records / event lists / closer slice brought to shared memory by cp.async.bulk under an mbarrier, two stages deep -- was
   // built and measured in round 1: 281 vs 216 us per 16 x 100k-tip evaluation.  With ~2 events per node, 8 resident CTAs/SM walking
-  // lists keep more loads in flight than two staged tiles per SM; it was removed.)
-  {
-    // resident CTAs per SM (tuning knob DPHY_TILE_OCC = 3 | 4 | 5 | 6)
-    static const int tocc = [] { const char* e = getenv("DPHY_TILE_OCC"); return e ? atoi(e) : 4; }();
-    static const bool ordered = [] { const char* e = getenv("DPHY_TILE_ORDER"); return !e || atoi(e) != 0; }();
-    const int32_t* order = ordered ? fo->d_ctile_order : nullptr;      // full tiles first, the partly filled ones last
-    if (tocc == 3) emat_log_G_tile_kernel<3><<<fo->h.num_ctiles, kLgThreads, 0, ctx->stream>>>(P, order);
-    else if (tocc == 5) emat_log_G_tile_kernel<5><<<fo->h.num_ctiles, kLgThreads, 0, ctx->stream>>>(P, order);
-    else if (tocc == 6) emat_log_G_tile_kernel<6><<<fo->h.num_ctiles, kLgThreads, 0, ctx->stream>>>(P, order);
-    else emat_log_G_tile_kernel<4><<<fo->h.num_ctiles, kLgThreads, 0, ctx->stream>>>(P, order);
-    ctx->launches += 1;
-  }
+  // lists keep more loads in flight than two staged tiles per SM; it was removed.)  Tiles go in fo->d_ctile_order: full tiles
+  // first, the partly filled ones last.
+  emat_log_G_tile_kernel<<<fo->h.num_ctiles, kLgThreads, 0, ctx->stream>>>(P, fo->d_ctile_order);
+  ctx->launches += 1;
   emat_log_G_tree_kernel<<<fo->h.num_trees, kTreeThreads, 0, ctx->stream>>>(P);
   ctx->launches += 1;
   st = check_cuda(ctx, cudaGetLastError(), "emat_log_G kernels launch");

@@ -26,7 +26,6 @@
 #include <climits>
 #include <cmath>
 #include <cstddef>
-#include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <math_constants.h>
@@ -34,6 +33,16 @@
 #include <vector>
 
 namespace dphy {
+
+// SprStudy::error: set on the device by the kernel named, turned into a status and a message by spr_fetch
+enum SprError : int32_t {
+  kSprErrXNoParent = 1,           // spr_init_kernel
+  kSprErrStartMutIdx = 2,         // spr_init_kernel
+  kSprErrStartInXSubtree = 3,     // spr_init_kernel
+  kSprErrPathMuts = 4,            // spr_xtab_kernel: the root path's mutation ordinals must fit 28 bits
+  kSprErrFrontierCap = 5,         // spr_frontier_kernel
+  kSprErrHmixCap = 6,             // spr_g2_bases_kernel
+};
 
 struct SprStudy {
   // ---- inputs (host) ----
@@ -84,7 +93,6 @@ struct SprBatchDev {
   uint32_t* tile_flag;    // unused
   uint32_t* ticket;       // [S][4]
   int32_t num_studies, max_tiles;
-  uint32_t epoch;
   // study-independent tables of the forest for the event-scan path (built once per forest, dphy_forest::d_spr_*)
   const int32_t* g2_eopen;     // [num_nodes]  tree-local index of the event at which the node opens
   const int32_t* g2_tnode;     // [num_nodes + total mutations]  device position of the node of every region template
@@ -167,7 +175,7 @@ __global__ void __launch_bounds__(256) spr_init_kernel(ForestDev f, SprBatchDev 
     int posP = -1, posS = -1, nP = 0, nS = 0, Proot = 0;
     if (posX >= 0) {
       posP = f.parent_pos[posX];
-      if (posP < 0) { S.error = 1; posP = posX; }
+      if (posP < 0) { S.error = kSprErrXNoParent; posP = posX; }
       const int c1 = posP + 1, c0 = posP + 1 + f.subtree_size[posP + 1];
       posS = (posX == c1) ? c0 : c1;
       nP = f.mut_off[posP + 1] - f.mut_off[posP];
@@ -176,8 +184,8 @@ __global__ void __launch_bounds__(256) spr_init_kernel(ForestDev f, SprBatchDev 
     }
     S.posX = posX; S.posP = posP; S.posS = posS; S.nP = nP; S.nS = nS; S.P_is_root = Proot;
     S.pos0 = pos0; S.k0 = S.start_mut_idx; S.n0 = f.mut_off[pos0 + 1] - f.mut_off[pos0];
-    if (S.k0 < 0 || S.k0 > S.n0 || (pos0 == T.node_base && S.k0 != S.n0)) S.error = 2;
-    if (posX >= 0 && pos0 >= posX && pos0 < posX + f.subtree_size[posX]) S.error = 3;   // start inside X's subtree
+    if (S.k0 < 0 || S.k0 > S.n0 || (pos0 == T.node_base && S.k0 != S.n0)) S.error = kSprErrStartMutIdx;
+    if (posX >= 0 && pos0 >= posX && pos0 < posX + f.subtree_size[posX]) S.error = kSprErrStartInXSubtree;   // start inside X's subtree
     S.path_len = min(dep0 + 1, S.path_cap);
     S.xpath_len = posX >= 0 ? min(depX + 1, S.path_cap) : 0;
     traw[2 * (PT.first + w)] = pos0; traw[2 * (PT.first + w) + 1] = posX >= 0 ? posX : INT_MAX;
@@ -323,7 +331,7 @@ __global__ void __launch_bounds__(kSetupThreads) spr_xtab_kernel(ForestDev f, Sp
     int tot;
     const int incl = block_scan_incl<int, kSetupThreads>(cnt, s_ws, &tot);
     const int base = s_carry + incl - cnt;
-    if (base + cnt >= (1 << 28)) S.error = 4;
+    if (base + cnt >= (1 << 28)) S.error = kSprErrPathMuts;
     for (int i = 0; i < cnt; ++i) {
       const int site = f.mut_site[mo + i];
       if (site >= l0 && site < l1) atomicMax(xkey + site, ((uint32_t)(base + i + 1) << 2) | (uint32_t)(f.mut_code[mo + i] & 3));
@@ -1006,8 +1014,8 @@ __device__ __forceinline__ void emit_mut_dc(const ForestDev& f, const EmitSmem& 
   else mut_dc(xtab, f.mut_site[i], f.mut_code[i] & 15, dh, dc);
 }
 
-template <int kMinBlocks>
-__global__ void __launch_bounds__(kTile, kMinBlocks) spr_emit_kernel(ForestDev f, SprBatchDev B) {
+// 4 resident CTAs per SM: 64 registers, 16 bytes of spill stores (5 or 6 CTAs: 48 / 40 registers, 36 / 192 bytes)
+__global__ void __launch_bounds__(kTile, 4) spr_emit_kernel(ForestDev f, SprBatchDev B) {
   __shared__ EmitSmem sm;
   const int study = blockIdx.y;
   const int t0 = blockIdx.x * kEmitSub;        // first kTile-tile of this CTA
@@ -1485,61 +1493,55 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   std::vector<std::pair<size_t, const void*>> copies;   // (slab offset, host ptr) with sizes below
   std::vector<size_t> copy_bytes;
   // ---- grouping: full (unbounded) studies of the same tree go 32 at a time through the lanes-are-studies kernels ----------------
-  // (DPHY_SPR_GROUPED=0 disables)
   constexpr int kMinGroup = 24;     // a group costs the same for 1 or 32 lanes: below ~24 studies the per-study kernels are cheaper
-  // DPHY_SPR_GROUPED=0: every study on the per-study kernels
-  static const bool use_groups = [] { const char* e = getenv("DPHY_SPR_GROUPED"); return !(e && atoi(e) == 0); }();
   std::vector<int> group_of(n, -1), lane_of(n, 0);
   std::vector<SprGroupDev> groups;
-  if (use_groups) {
-    std::vector<std::vector<int>> by_tree(fo->h.num_trees);
-    for (int i = 0; i < n; ++i)
-      if (reqs[i].tree >= 0 && reqs[i].tree < fo->h.num_trees && reqs[i].max_muts_from_start == INT_MAX) by_tree[reqs[i].tree].push_back(i);
-    std::vector<int64_t> mut_base(fo->h.num_trees + 1, 0);
-    for (int k = 0; k < fo->h.num_trees; ++k) mut_base[k + 1] = mut_base[k] + fo->tree_muts[k];
-    for (int k = 0; k < fo->h.num_trees; ++k) {
-      const auto& v = by_tree[k];
-      for (size_t g0 = 0; g0 < v.size(); g0 += kGroup) {
-        if ((int)(v.size() - g0) < kMinGroup) break;       // a thin remainder goes study by study
-        SprGroupDev G;
-        std::memset(&G, 0, sizeof(G));
-        const TreeDev& T = fo->trees[k];
-        G.tree = k; G.node_base = T.node_base; G.num_nodes = T.num_nodes; G.L = fo->sites[T.sites_id]->L;
-        G.mut_base = (int32_t)mut_base[k];
-        G.num = (int32_t)std::min<size_t>(kGroup, v.size() - g0);
-        for (int l = 0; l < G.num; ++l) { G.study[l] = v[g0 + l]; group_of[v[g0 + l]] = (int)groups.size(); lane_of[v[g0 + l]] = l; }
-        G.off_xT = take((size_t)G.L * kGroup);
-        {
-          const int64_t M = fo->tree_muts[k];
-          if (2 * M + 1 + kEvChunk > INT_MAX || (int64_t)T.num_nodes + M + 64 > INT_MAX) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: tree too large");
-          G.num_muts = (int32_t)M; G.num_templates = (int32_t)(T.num_nodes + M);
-          G.num_ev_chunks = (int32_t)(2 * M / kEvChunk + 1);           // rows 0 .. 2M
-          G.num_t_chunks = (G.num_templates + 31) / 32;                // + one empty chunk, so that KB(N) always has a row
-          G.off_S = take((size_t)G.num_ev_chunks * kEvChunk * kGroup);
-          G.off_aggS = take(sizeof(int32_t) * ((size_t)G.num_ev_chunks + 1) * kGroup);
-          G.off_mask = take(sizeof(uint32_t) * ((size_t)G.num_t_chunks + 1) * kGroup);
-          G.off_aggK = take(sizeof(int32_t) * ((size_t)G.num_t_chunks + 2) * kGroup);
-          G.off_cbase = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1) * kGroup);
-          G.off_consts = take(32 * kGroup + sizeof(int32_t) * kGroup);      // G2Const [32] + root_keep [32]
-          G.off_outs = take(64 * kGroup);
-          if (g0 == 0) {
-            G.trec_owner = 1; G.off_trec = take(48 * (size_t)G.num_templates);
-            G.off_csort = take(sizeof(double) * 32 * ((size_t)G.num_t_chunks + 1));
-            G.off_cpm = take(sizeof(uint32_t) * 32 * ((size_t)G.num_t_chunks + 1));
-            G.off_cq = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1));
-          } else {
-            const SprGroupDev& G0 = groups[groups.size() - g0 / kGroup];
-            G.trec_owner = 0; G.off_trec = G0.off_trec; G.off_csort = G0.off_csort; G.off_cpm = G0.off_cpm; G.off_cq = G0.off_cq;
-          }
+  std::vector<std::vector<int>> by_tree(fo->h.num_trees);
+  for (int i = 0; i < n; ++i)
+    if (reqs[i].tree >= 0 && reqs[i].tree < fo->h.num_trees && reqs[i].max_muts_from_start == INT_MAX) by_tree[reqs[i].tree].push_back(i);
+  std::vector<int64_t> mut_base(fo->h.num_trees + 1, 0);
+  for (int k = 0; k < fo->h.num_trees; ++k) mut_base[k + 1] = mut_base[k] + fo->tree_muts[k];
+  for (int k = 0; k < fo->h.num_trees; ++k) {
+    const auto& v = by_tree[k];
+    for (size_t g0 = 0; g0 < v.size(); g0 += kGroup) {
+      if ((int)(v.size() - g0) < kMinGroup) break;       // a thin remainder goes study by study
+      SprGroupDev G;
+      std::memset(&G, 0, sizeof(G));
+      const TreeDev& T = fo->trees[k];
+      G.tree = k; G.node_base = T.node_base; G.num_nodes = T.num_nodes; G.L = fo->sites[T.sites_id]->L;
+      G.mut_base = (int32_t)mut_base[k];
+      G.num = (int32_t)std::min<size_t>(kGroup, v.size() - g0);
+      for (int l = 0; l < G.num; ++l) { G.study[l] = v[g0 + l]; group_of[v[g0 + l]] = (int)groups.size(); lane_of[v[g0 + l]] = l; }
+      G.off_xT = take((size_t)G.L * kGroup);
+      {
+        const int64_t M = fo->tree_muts[k];
+        if (2 * M + 1 + kEvChunk > INT_MAX || (int64_t)T.num_nodes + M + 64 > INT_MAX) return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "spr: tree too large");
+        G.num_muts = (int32_t)M; G.num_templates = (int32_t)(T.num_nodes + M);
+        G.num_ev_chunks = (int32_t)(2 * M / kEvChunk + 1);           // rows 0 .. 2M
+        G.num_t_chunks = (G.num_templates + 31) / 32;                // + one empty chunk, so that KB(N) always has a row
+        G.off_S = take((size_t)G.num_ev_chunks * kEvChunk * kGroup);
+        G.off_aggS = take(sizeof(int32_t) * ((size_t)G.num_ev_chunks + 1) * kGroup);
+        G.off_mask = take(sizeof(uint32_t) * ((size_t)G.num_t_chunks + 1) * kGroup);
+        G.off_aggK = take(sizeof(int32_t) * ((size_t)G.num_t_chunks + 2) * kGroup);
+        G.off_cbase = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1) * kGroup);
+        G.off_consts = take(32 * kGroup + sizeof(int32_t) * kGroup);      // G2Const [32] + root_keep [32]
+        G.off_outs = take(64 * kGroup);
+        if (g0 == 0) {
+          G.trec_owner = 1; G.off_trec = take(48 * (size_t)G.num_templates);
+          G.off_csort = take(sizeof(double) * 32 * ((size_t)G.num_t_chunks + 1));
+          G.off_cpm = take(sizeof(uint32_t) * 32 * ((size_t)G.num_t_chunks + 1));
+          G.off_cq = take(sizeof(int2) * ((size_t)G.num_t_chunks + 1));
+        } else {
+          const SprGroupDev& G0 = groups[groups.size() - g0 / kGroup];
+          G.trec_owner = 0; G.off_trec = G0.off_trec; G.off_csort = G0.off_csort; G.off_cpm = G0.off_cpm; G.off_cq = G0.off_cq;
         }
-        groups.push_back(G);
       }
+      groups.push_back(G);
     }
   }
   // (raw log-weights inside the grouped emit were measured slower than the dense weights pass over the stored heads: the two logs
   // per region then run at the emit's ~45 % lane utilisation and low occupancy, 1.26 ms vs 0.68 + 0.23 ms per 128 studies)
-  // The event-scan emit computes the raw log-weights itself (DPHY_SPR_FUSE_WEIGHTS=0: dense pass over the stored heads instead)
-  static const bool fuse_weights = [] { const char* e = getenv("DPHY_SPR_FUSE_WEIGHTS"); return !(e && atoi(e) == 0); }();
+  // The event-scan emit computes the raw log-weights itself
   for (int i = 0; i < n; ++i) {
     const dphy_spr_request& r = reqs[i];
     SprStudy& S = b->host[i];
@@ -1567,12 +1569,12 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
       if (r.x_missing_start[k] < 0 || r.x_missing_end[k] > L || r.x_missing_start[k] >= r.x_missing_end[k]) return set_error(ctx, DPHY_ERR_OUT_OF_RANGE, "spr: X missing interval out of range");
     const int N = T.num_nodes;
     const bool grouped = group_of[i] >= 0;
-    // bounded studies of a small radius walk their ball (kernels_spr_frontier.cuh; DPHY_SPR_FRONTIER=0: the per-study sweeps instead)
+    // bounded studies of a small radius walk their ball (kernels_spr_frontier.cuh), the others take the per-study sweeps.
     // Measured on a 100k-tip tree (tools/spr_bounded_timing.py): radius 1: 7.0 vs 9.7 us per study in a batch of 64, 3.4 vs 7.9 in a
     // batch of 512; radius 2: 17.4 vs 9.7 (64), 5.0 vs 7.9 (512) -- a walk lasts as long as its largest ball (mutation-free clades make
     // the ball sizes heavy-tailed) while the sweeps cost the same for every study, so larger radii only walk in large batches.
-    static const int frontier_max = [] { const char* e = getenv("DPHY_SPR_FRONTIER"); return e ? atoi(e) : 4; }();
-    const bool frontier = !grouped && r.max_muts_from_start != INT_MAX && r.max_muts_from_start <= frontier_max &&
+    constexpr int kFrontierMaxRadius = 4;
+    const bool frontier = !grouped && r.max_muts_from_start != INT_MAX && r.max_muts_from_start <= kFrontierMaxRadius &&
                           (r.max_muts_from_start <= 1 || num_bounded >= 256);
     any_frontier |= frontier;
     any_swept_limited |= !grouped && !frontier && r.max_muts_from_start != INT_MAX;
@@ -1583,7 +1585,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
       S.g2 = 1; S.g2_lane = lane_of[i]; S.g2_mut_base = G.mut_base; S.g2_num_templates = G.num_templates;
       S.off_g2S = G.off_S; S.off_g2aggS = G.off_aggS; S.off_g2mask = G.off_mask; S.off_g2aggK = G.off_aggK; S.off_g2cbase = G.off_cbase;
     }
-    S.weights_fused = (grouped && fuse_weights && r.lambda_X > 0.0) ? 1 : 0;
+    S.weights_fused = (grouped && r.lambda_X > 0.0) ? 1 : 0;
     max_tiles = std::max(max_tiles, S.num_htiles);
     if (!grouped && !frontier) max_tiles256 = std::max(max_tiles256, T.num_tiles);
     // exact upper bound on regions: every non-root node has n+1 regions, the root has 1
@@ -1681,14 +1683,13 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   b->dev.tile_flag = hdr.at<uint32_t>(d, b_flag);
   b->dev.ticket = hdr.at<uint32_t>(d, b_ticket);
   b->dev.slab = d + hdr.total;
-  b->dev.num_studies = n; b->dev.max_tiles = max_tiles; b->dev.epoch = 1;
+  b->dev.num_studies = n; b->dev.max_tiles = max_tiles;
   b->dev.g2_eopen = nullptr; b->dev.g2_tnode = nullptr; b->dev.g2_ev = nullptr; b->dev.g2_mut_off = fo->h.mut_off;
   if (!groups.empty()) {
     st = ensure_spr_tables(ctx, fo);
     if (st != DPHY_OK) return st;
     b->dev.g2_eopen = fo->d_spr_eopen; b->dev.g2_tnode = fo->d_spr_tnode; b->dev.g2_ev = fo->d_spr_ev;
   }
-  { static const bool dry = [] { const char* e = getenv("DPHY_SPR_DRY"); return e && atoi(e) != 0; }(); if (dry) b->dev.epoch = 777u; }
   b->d_groups = hdr.at<SprGroupDev>(d, b_groups); b->num_groups = (int32_t)groups.size();
   if (n == 0) { *out = b.release(); return DPHY_OK; }
   // flags + tickets start at zero; studies + X overlays uploaded through the pinned staging buffer
@@ -1719,7 +1720,6 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   for (const SprGroupDev& G : groups) group_L = std::max(group_L, G.L);
   const int ng = (int)groups.size();
   const bool any_single = max_tiles256 > 0;        // studies on the per-study path
-  static const bool use_aux = [] { const char* e = getenv("DPHY_SPR_AUX_STREAM"); return !(e && atoi(e) == 0); }();
   {
     char* sl = b->dev.slab;
     const SprPathTree* d_pt = (const SprPathTree*)(sl + off_ptrees);
@@ -1727,7 +1727,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
                                                                          (SprPathTarget*)(sl + off_tgt), (SprPathTargetAux*)(sl + off_taux));
     // fork: what depends on the tree and the studies' positions alone (constants, template records, keep masks) runs on the side stream
     // while the main stream walks the latency-bound chain paths -> X tables -> event scan
-    if (ng > 0 && use_aux) {
+    if (ng > 0) {
       if (!ctx->aux_stream) {
         if (cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
             cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
@@ -1752,7 +1752,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   }
   const dim3 grid_g2t((g2_t_chunks + kG2Warps - 1) / kG2Warps, std::max(ng, 1));
   if (ng > 0) {
-    cudaStream_t side = use_aux ? ctx->aux_stream : ctx->stream;
+    cudaStream_t side = ctx->aux_stream;
     spr_xT_kernel<<<dim3((group_L + 255) / 256, ng), 256, 0, ctx->stream>>>(b->dev, b->d_groups);
     spr_g2_consts_kernel<<<ng, kGroup, 0, side>>>(fo->h, b->dev, b->d_groups);
     spr_g2_templ_kernel<<<dim3((g2_t_chunks * 32 + 255) / 256, ng), 256, 0, side>>>(fo->h, b->dev, b->d_groups);
@@ -1761,7 +1761,8 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     spr_g2_prefix_kernel<<<dim3(kPfxCtas, ng), 1024, 0, side>>>(b->dev, b->d_groups, 1);
     spr_g2_scan_kernel<<<dim3((g2_ev_chunks + kG2Warps - 1) / kG2Warps, ng), kG2Warps * 32, 0, ctx->stream>>>(fo->h, b->dev, b->d_groups);
     spr_g2_prefix_kernel<<<dim3(kPfxCtas, ng), 1024, 0, ctx->stream>>>(b->dev, b->d_groups, 0);
-    if (use_aux) { cudaEventRecord(ctx->ev_join, ctx->aux_stream); cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0); }
+    cudaEventRecord(ctx->ev_join, ctx->aux_stream);
+    cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0);
     launched += 5;
   }
   if (any_frontier) { spr_frontier_kernel<<<(n + 3) / 4, 128, 0, ctx->stream>>>(fo->h, b->dev); ++launched; }
@@ -1773,12 +1774,8 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   spr_segments_kernel<<<n, kSetupThreads, 0, ctx->stream>>>(fo->h, b->dev);
   ++launched;
   if (any_single) {
-    // resident CTAs per SM (tuning knob DPHY_EMIT_OCC = 4 | 5 | 6; 64 / 48 / 40 registers)
-    static const int occ = [] { const char* e = getenv("DPHY_EMIT_OCC"); return e ? atoi(e) : 4; }();
     const dim3 grid_emit((max_tiles256 + kEmitSub - 1) / kEmitSub, n);
-    if (occ == 5) spr_emit_kernel<5><<<grid_emit, kTile, 0, ctx->stream>>>(fo->h, b->dev);
-    else if (occ == 6) spr_emit_kernel<6><<<grid_emit, kTile, 0, ctx->stream>>>(fo->h, b->dev);
-    else spr_emit_kernel<4><<<grid_emit, kTile, 0, ctx->stream>>>(fo->h, b->dev);
+    spr_emit_kernel<<<grid_emit, kTile, 0, ctx->stream>>>(fo->h, b->dev);
     ++launched;
   }
   bool any_weighted = false, any_unfused = false;
@@ -1793,36 +1790,29 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
   // that the set-up chain of the NEXT batch (paths, X tables, event scan, segments, bases: latency-bound kernels with small grids,
   // on the higher-priority main stream) runs next to them.  Every accessor of the batch, and every entry point that edits or frees
   // the forest, joins the tail first.
-  static const int tail_mode = [] { const char* e = getenv("DPHY_SPR_TAIL_STREAM"); return e ? atoi(e) : 2; }();   // 0 off, 1 normalize only, 2 emit too
-  const bool use_tail = tail_mode != 0 && (g2_emit || any_weighted);
-  cudaStream_t ts = ctx->stream;
-  auto fork_tail = [&]() -> int {
-    if (ts != ctx->stream) return DPHY_OK;
+  const bool use_tail = g2_emit || any_weighted;
+  if (use_tail) {
     if (!ctx->tail_stream) {
       if (cudaStreamCreateWithFlags(&ctx->tail_stream, cudaStreamNonBlocking) != cudaSuccess ||
           cudaEventCreateWithFlags(&ctx->ev_tail, cudaEventDisableTiming) != cudaSuccess)
         return set_error(ctx, DPHY_ERR_CUDA, "spr: tail stream");
     }
-    if (!b->ev_done && cudaEventCreateWithFlags(&b->ev_done, cudaEventDisableTiming) != cudaSuccess) return set_error(ctx, DPHY_ERR_CUDA, "spr: tail event");
+    if (cudaEventCreateWithFlags(&b->ev_done, cudaEventDisableTiming) != cudaSuccess) return set_error(ctx, DPHY_ERR_CUDA, "spr: tail event");
     cudaEventRecord(ctx->ev_tail, ctx->stream);
     cudaStreamWaitEvent(ctx->tail_stream, ctx->ev_tail, 0);
-    ts = ctx->tail_stream;
-    return DPHY_OK;
-  };
+  }
+  cudaStream_t ts = use_tail ? ctx->tail_stream : ctx->stream;
   if (g2_emit) {
-    if (use_tail && tail_mode >= 2) { st = fork_tail(); if (st != DPHY_OK) return st; }
-    if (fuse_weights) spr_g2_emit_kernel<2><<<grid_g2t, kG2Warps * 32, 0, ts>>>(fo->h, b->dev, b->d_groups);
-    else spr_g2_emit_kernel<1><<<grid_g2t, kG2Warps * 32, 0, ts>>>(fo->h, b->dev, b->d_groups);
+    spr_g2_emit_kernel<<<grid_g2t, kG2Warps * 32, 0, ts>>>(fo->h, b->dev, b->d_groups);
     ++launched;
   }
   if (any_weighted) {
-    if (use_tail) { st = fork_tail(); if (st != DPHY_OK) return st; }
     if (any_unfused) { spr_weights_kernel<<<dim3(kWeightBlocks, n), 256, 0, ts>>>(fo->h, b->dev); ++launched; }
     spr_normalize_kernel<<<dim3(kNormBlocks, n), 256, 0, ts>>>(b->dev);
     ++launched;
     b->weighted = true;
   }
-  if (ts != ctx->stream) { cudaEventRecord(b->ev_done, ctx->tail_stream); b->tail_pending = true; ctx->tail_dirty = true; }
+  if (use_tail) { cudaEventRecord(b->ev_done, ctx->tail_stream); b->tail_pending = true; ctx->tail_dirty = true; }
   ctx->launches += launched;
   st = check_cuda(ctx, cudaGetLastError(), "spr kernels launch");
   if (st != DPHY_OK) return st;
@@ -1862,11 +1852,12 @@ static int spr_fetch(dphy_ctx* ctx, dphy_spr_batch* b) {
   b->fetched = true;
   for (int i = 0; i < b->num; ++i) {
     const char* what = nullptr; int st = DPHY_OK;
-    if (b->host[i].error == 1) { st = DPHY_ERR_INVALID_ARGUMENT; what = "X has no parent"; }
-    else if (b->host[i].error == 2) { st = DPHY_ERR_OUT_OF_RANGE; what = "start_mut_idx out of range for the start branch"; }
-    else if (b->host[i].error == 3) { st = DPHY_ERR_INVALID_ARGUMENT; what = "start region lies inside X's subtree"; }
-    else if (b->host[i].error == 4) { st = DPHY_ERR_INTERNAL; what = "more than 2^28 mutations on the root path"; }
-    else if (b->host[i].error == 5) { st = DPHY_ERR_INTERNAL; what = "more than 65535 candidate regions on 32 consecutive branches (set DPHY_SPR_GROUPED=0)"; }
+    if (b->host[i].error == kSprErrXNoParent) { st = DPHY_ERR_INVALID_ARGUMENT; what = "X has no parent"; }
+    else if (b->host[i].error == kSprErrStartMutIdx) { st = DPHY_ERR_OUT_OF_RANGE; what = "start_mut_idx out of range for the start branch"; }
+    else if (b->host[i].error == kSprErrStartInXSubtree) { st = DPHY_ERR_INVALID_ARGUMENT; what = "start region lies inside X's subtree"; }
+    else if (b->host[i].error == kSprErrPathMuts) { st = DPHY_ERR_INTERNAL; what = "more than 2^28 mutations on the root path"; }
+    else if (b->host[i].error == kSprErrFrontierCap) { st = DPHY_ERR_INTERNAL; what = "the bounded-radius walk found more regions than the study's region capacity"; }
+    else if (b->host[i].error == kSprErrHmixCap) { st = DPHY_ERR_INTERNAL; what = "more template chunks straddle the study's path segments than the grouped emit has offset rows for"; }
     else if (b->host[i].total_regions > b->host[i].region_cap) { st = DPHY_ERR_INTERNAL; what = "region capacity exceeded"; }
     if (st != DPHY_OK) {
       // sticky: every later accessor of this batch (getters, pick, find) reports the same failure, naming the request

@@ -140,7 +140,7 @@ __global__ void __launch_bounds__(128) spr_frontier_kernel(ForestDev f, SprBatch
       next = idx + 1;
     }
   }
-  if (overflow) { if (lane == 0) S.error = 5; return; }
+  if (overflow) { if (lane == 0) S.error = kSprErrFrontierCap; return; }
   __syncwarp();
   if (lane != 0) return;
   // ---- account_for_Xs_detachment (core/spr_study.cpp:130-209) + remove_regions_in_Xs_future (:211-224), in place -----------------------------

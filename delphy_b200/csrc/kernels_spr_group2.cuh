@@ -358,7 +358,7 @@ __global__ void __launch_bounds__(kBasesThreads) spr_g2_bases_kernel(SprBatchDev
       int row0 = 0;
       if (lane == 0) row0 = (int)atomicAdd(B.ticket + sidx * 4 + 3, (unsigned)__popc(todo));
       row0 = __shfl_sync(full, row0, 0);
-      if (row0 + __popc(todo) > S.hmix_cap) { if (lane == 0) S.error = 6; todo = 0u; }
+      if (row0 + __popc(todo) > S.hmix_cap) { if (lane == 0) S.error = kSprErrHmixCap; todo = 0u; }
       for (int nrow = 0; todo; todo &= todo - 1, ++nrow) {
         const int src = __ffs(todo) - 1;
         const int tcs = tb + src * kW + wrp, lo_s = __shfl_sync(full, jlo, src), hi_s = __shfl_sync(full, jhi, src), kb_s = __shfl_sync(full, kb, src);
@@ -441,18 +441,17 @@ __global__ void __launch_bounds__(kCountWarps * 32) spr_g2_count_kernel(ForestDe
 }
 
 // ---- emit: lanes = templates, loop over the studies ------------------------------------------------------------------------------------------
-// kMode 1: the 32-byte heads;  2: heads + raw log-weights (and their per-study maximum)
-template <int kMode>
+// the 32-byte heads, and the raw log-weights (and their per-study maximum) of the studies with weights_fused
 __global__ void __launch_bounds__(kG2Warps * 32) spr_g2_emit_kernel(ForestDev f, SprBatchDev B, const SprGroupDev* __restrict__ groups) {
-  constexpr bool kFuse = kMode == 2;
   __shared__ G2Study s_st[kG2Warps][kGroup];
-  __shared__ G2Weight s_wt[kFuse ? kG2Warps : 1][kFuse ? kGroup : 1];
-  __shared__ double2 s_log[kFuse ? (1 << kLogTabBits) : 1];
+  __shared__ G2Weight s_wt[kG2Warps][kGroup];
+  __shared__ double2 s_log[1 << kLogTabBits];
   // chunk-local potentials of the lane's template for the 32 studies: one 32-byte row, kept in shared memory (36-byte pitch) because
   // the study loop is not fully unrolled -- 32 copies of its body, two logarithms each, do not fit the instruction cache: ncu showed
   // "no instruction" as the top stall -- so the byte of study s is a dynamic index
   __shared__ uint32_t s_row[kG2Warps][32][9];
-  if (kFuse) { fill_log_table(s_log); __syncthreads(); }
+  fill_log_table(s_log);
+  __syncthreads();
   const unsigned full = 0xffffffffu;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const SprGroupDev& G = groups[blockIdx.y];
@@ -468,13 +467,12 @@ __global__ void __launch_bounds__(kG2Warps * 32) spr_g2_emit_kernel(ForestDev f,
   const G2Out* op = (const G2Out*)(B.slab + G.off_outs) + lane;
   const int4 o0 = *reinterpret_cast<const int4*>(op);
   st.base = cb.x; st.mH = o0.x; st.out_lo = (unsigned)o0.z; st.out_hi = (unsigned)o0.w;
-  bool fused_lane = false;                                // (kFuse) the lane's study gets its weights here
-  unsigned long long mykey = 0ULL;                        // (kFuse) running maximum of the lane's study, as an ordered key
-  if (kFuse) {
+  unsigned long long mykey = 0ULL;                        // running maximum of the lane's study, as an ordered key
+  {
     G2Weight w; w.logfl = op->logfl; w.fa = op->fa; w.lam = op->lam; w.mu3 = op->mu3; w.lw_minus_out = op->lw_minus_out; w.fused = o0.y; w.pad = 0;
     s_wt[warp][lane] = w;
-    fused_lane = o0.y != 0;
   }
+  const bool fused_lane = o0.y != 0;                      // the lane's study gets its weights here
   // (the constants were written on the side stream, before the X-table kernel could flag its study: look at the study itself)
   if (st.c.tX == -DBL_MAX || (lane < G.num && B.studies[G.study[lane]].error)) mymask = 0u;
   // ---- the lane's template ---------------------------------------------------------------------------------------------------------------
@@ -508,8 +506,7 @@ __global__ void __launch_bounds__(kG2Warps * 32) spr_g2_emit_kernel(ForestDev f,
   __syncwarp();
   const unsigned lt = (1u << lane) - 1u;
   // log(t_max - t_min) of the unclipped region: shared by every study that does not clip it
-  double logdt = 0.0;
-  if (kFuse) logdt = fast_log(T.t_max - T.t_min, s_log);
+  const double logdt = fast_log(T.t_max - T.t_min, s_log);
   const int8_t* myrow = reinterpret_cast<const int8_t*>(s_row[warp][lane]);
 
 #pragma unroll 4
@@ -535,7 +532,7 @@ __global__ void __launch_bounds__(kG2Warps * 32) spr_g2_emit_kernel(ForestDev f,
       const unsigned long long w0 = (unsigned long long)(unsigned)T.idn | ((unsigned long long)(unsigned)T.k << 32);
       asm volatile("st.global.v4.b64 [%0], {%1, %2, %3, %4};" ::"l"(o), "l"(w0), "l"(__double_as_longlong(T.t_min)),
                    "l"(__double_as_longlong(tmx)), "l"((unsigned long long)(unsigned)m) : "memory");
-      if (kFuse && s_wt[warp][s].fused) {
+      if (s_wt[warp][s].fused) {
         // raw log-weight (core/spr_study.cpp:313-318): log(f lam dt) + f (-lam (t_X - t') + m log(mu (t_X - t') / 3)), t' = mid-point
         const G2Weight& w8 = s_wt[warp][s];
         const double x = ss.c.tX - 0.5 * (T.t_min + tmx);
@@ -545,12 +542,10 @@ __global__ void __launch_bounds__(kG2Warps * 32) spr_g2_emit_kernel(ForestDev f,
         key = f64_order_key(lw);
       }
     }
-    if (kFuse) {
-      // warp maximum of the ordered keys (two 32-bit REDUX steps), kept by the lane that owns study s
-      const unsigned hi = (unsigned)(key >> 32), mh = __reduce_max_sync(full, hi);
-      const unsigned ml = __reduce_max_sync(full, hi == mh ? (unsigned)key : 0u);
-      if (lane == s) { const unsigned long long k2 = ((unsigned long long)mh << 32) | ml; if (k2 > mykey) mykey = k2; }
-    }
+    // warp maximum of the ordered keys (two 32-bit REDUX steps), kept by the lane that owns study s
+    const unsigned hi = (unsigned)(key >> 32), mh = __reduce_max_sync(full, hi);
+    const unsigned ml = __reduce_max_sync(full, hi == mh ? (unsigned)key : 0u);
+    if (lane == s) { const unsigned long long k2 = ((unsigned long long)mh << 32) | ml; if (k2 > mykey) mykey = k2; }
   }
-  if (kFuse && fused_lane && mykey != 0ULL) atomicMax(&B.studies[G.study[lane]].max_key, mykey);
+  if (fused_lane && mykey != 0ULL) atomicMax(&B.studies[G.study[lane]].max_key, mykey);
 }

@@ -8,4 +8,3 @@ tail -15 $OUT/pytest_gpu.log
 timeout 600 python bench.py --steps 20 --warmup 3 --no-cpu-baseline "$@" > $OUT/bench.json 2> $OUT/bench.err; echo "bench exit $?"
 tail -5 $OUT/bench.err
 cat $OUT/bench.json
-timeout 300 python tools/logg_timing.py 16 4 > $OUT/logg_timing.txt 2>&1; cat $OUT/logg_timing.txt

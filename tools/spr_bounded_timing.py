@@ -1,6 +1,5 @@
 """Bounded (max_muts_from_start = limit) vs full SPR studies on a 100k-tip tree: device time per batch of 64, and the reference's
-own CPU time for the same studies (oracle/_ref, one thread per study).  usage: python tools/spr_bounded_timing.py [limit] [studies]
-(DPHY_SPR_FRONTIER=0: the O(N) per-study sweeps instead of the ball walk of kernels_spr_frontier.cuh)"""
+own CPU time for the same studies (oracle/_ref, one thread per study).  usage: python tools/spr_bounded_timing.py [limit] [studies]"""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
