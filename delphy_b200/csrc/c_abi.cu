@@ -99,8 +99,6 @@ int dphy_ctx_create(int device, dphy_ctx** out) {
     if (cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_greatest) != cudaSuccess) { delete ctx; return DPHY_ERR_CUDA; }
   }
   if (cudaEventCreateWithFlags(&ctx->pinned_ev, cudaEventDisableTiming) != cudaSuccess) { cudaStreamDestroy(ctx->stream); delete ctx; return DPHY_ERR_CUDA; }
-  cudaDeviceProp prop;
-  if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) ctx->sm_count = prop.multiProcessorCount;
   // keep freed stream-ordered allocations cached in the pool (no cudaMalloc on the hot path after warm-up)
   cudaMemPool_t pool;
   if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
@@ -232,7 +230,6 @@ static void fill_evo(dphy_sites* s, const double* mu, const double* pi_a, const 
     s->h.mu[b] = mu[b];
     for (int a = 0; a < 4; ++a) {
       s->h.pi[b * 4 + a] = pi_a[b * 4 + a];
-      s->h.log_pi[b * 4 + a] = pi_a[b * 4 + a] != 0.0 ? std::log(pi_a[b * 4 + a]) : 0.0;
       for (int c = 0; c < 4; ++c) s->h.q[b * 16 + a * 4 + c] = q_ab[b * 16 + a * 4 + c];
     }
   }
@@ -603,7 +600,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   auto tot_iv = [&](int k) -> int64_t { return totals ? totals[k].iv : trees[k].miss_off[trees[k].num_nodes]; };
   auto tot_fs = [&](int k) -> int64_t { return totals ? totals[k].fs : trees[k].fs_off[trees[k].num_nodes]; };
   auto tot_root_m = [&](int k) -> int64_t { return totals ? totals[k].root_m : trees[k].mut_off[trees[k].root + 1] - trees[k].mut_off[trees[k].root]; };
-  int64_t N = 0, M = 0, I = 0, F = 0, tiles = 0, ctiles = 0, Mnr = 0;
+  int64_t N = 0, M = 0, I = 0, F = 0, tiles = 0, ctiles = 0;
   int max_tree_nodes = 0;
   for (int k = 0; k < num_trees; ++k) {
     const auto& e = trees[k];
@@ -615,7 +612,6 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
     if (tot_m(k) < 0 || tot_iv(k) < 0 || tot_fs(k) < 0 || tot_root_m(k) < 0)
       return set_error(ctx, DPHY_ERR_INVALID_ARGUMENT, "CSR offsets are not monotone");
     N += n; M += tot_m(k); I += tot_iv(k); F += tot_fs(k);
-    Mnr += tot_m(k) - tot_root_m(k);
     tiles += (n + kTile - 1) / kTile;
     ctiles += (n + kLgTile - 1) / kLgTile;
     max_tree_nodes = std::max(max_tree_nodes, n);
@@ -632,7 +628,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
 
   std::unique_ptr<dphy_forest> fo(new (std::nothrow) dphy_forest());
   if (!fo) return DPHY_ERR_OUT_OF_MEMORY;
-  fo->total_muts = M; fo->total_ivls = I; fo->total_fs = F; fo->total_nonroot_muts = Mnr;
+  fo->total_muts = M; fo->total_ivls = I; fo->total_fs = F;
   fo->sites.assign(sites, sites + num_sites_tables);
   fo->sites_version.resize(num_sites_tables);
   fo->tree_muts.resize(num_trees); fo->tree_fs.resize(num_trees); fo->tree_max_depth.assign(num_trees, 0);
@@ -643,7 +639,6 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   const int b_trees = slab.reserve(sizeof(TreeDev) * num_trees);
   const int b_sites = slab.reserve(sizeof(SitesDev) * num_sites_tables);
   const int b_tile_tree = slab.reserve(sizeof(int32_t) * tiles);
-  const int b_ctile_tree = slab.reserve(sizeof(int32_t) * ctiles);
   const int b_ctiles = slab.reserve(sizeof(CTileDesc) * ctiles);
   const int b_corder = slab.reserve(sizeof(int32_t) * ctiles);
   const size_t header_bytes = slab.total;
@@ -659,13 +654,11 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   const int b_cnt = slab.reserve(sizeof(int32_t) * (size_t)fsw_stride * N + 64);
   // outputs + workspaces
   const int b_lambda = slab.reserve(sizeof(double) * N), b_nsmn = slab.reserve(sizeof(int32_t) * N);
-  const int b_fastl = slab.reserve(sizeof(int32_t) * ctiles), b_slowl = slab.reserve(sizeof(int32_t) * ctiles);
   const int b_strad = slab.reserve(sizeof(int32_t) * 2 * N), b_sdd = slab.reserve(sizeof(double) * N), b_sdn = slab.reserve(sizeof(int32_t) * N);
   const int b_tout = slab.reserve(sizeof(double) * 4 * num_trees), b_tiout = slab.reserve(sizeof(int32_t) * 20 * num_trees);
   const int b_tagg = slab.reserve(sizeof(double) * tiles), b_tiagg = slab.reserve(sizeof(int32_t) * tiles);
   const int b_tpart = slab.reserve(sizeof(double) * 2 * tiles), b_tipart = slab.reserve(sizeof(int32_t) * 17 * tiles);
   const int b_tflag = slab.reserve(sizeof(uint32_t) * tiles);
-  const int b_tdone = slab.reserve(sizeof(uint32_t) * num_trees), b_ticket = slab.reserve(sizeof(uint32_t) * 4);
 
   // ---- the temporary block: raw host-order arrays + flatten workspaces -------------------------------------------------------
   Slab tmp;
@@ -701,7 +694,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   const int64_t scan_tiles = (N + 1023) / 1024;
   const int w_scan = work.reserve(sizeof(int32_t) * 3 * scan_tiles);
   const int w_cnttot = work.reserve(sizeof(uint4) * 2 * (fsw_stride / 4) * scan_tiles);
-  const int w_status = work.reserve(sizeof(uint32_t) * 4 + sizeof(int32_t) * num_trees);
+  const int w_status = work.reserve(sizeof(uint32_t) * 2 + sizeof(int32_t) * num_trees);
   const int w_jobs = work.reserve(sizeof(DeviceCopyJob) * ((size_t)num_trees * 15 + 1));     // device-resident sources only (see below)
 
   DevBlock dblk(ctx->stream), tblk(ctx->stream), wblk(ctx->stream);
@@ -723,7 +716,6 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   auto* h_trees = slab.at<TreeDev>(hb, b_trees);
   auto* h_sites = slab.at<SitesDev>(hb, b_sites);
   auto* h_tile_tree = slab.at<int32_t>(hb, b_tile_tree);
-  auto* h_ctile_tree = slab.at<int32_t>(hb, b_ctile_tree);
   auto* h_ctiles = slab.at<CTileDesc>(hb, b_ctiles);
   auto* h_corder = slab.at<int32_t>(hb, b_corder);
   auto* h_raw = tmp.at<RawTreeDev>(hraw, r_raw);
@@ -742,10 +734,9 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
     for (int j = 0; j < T.num_tiles; ++j) h_tile_tree[tile_pos++] = k;
     T.first_ctile = ctile_pos; T.num_ctiles = (n + kLgTile - 1) / kLgTile;
     for (int j = 0; j < T.num_ctiles; ++j) {
-      CTileDesc& d = h_ctiles[ctile_pos];
+      CTileDesc& d = h_ctiles[ctile_pos++];
       std::memset(&d, 0, sizeof(d));
       d.tile_start = base + j * kLgTile; d.n_act = std::min(kLgTile, n - j * kLgTile); d.node_base = base; d.sites_id = T.sites_id;
-      h_ctile_tree[ctile_pos++] = k;
     }
     h_trees[k] = T;
     fo->tree_muts[k] = (int64_t)m; fo->tree_fs[k] = (int64_t)fs;
@@ -814,9 +805,8 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   ForestDev& h = fo->h;
   h.num_trees = num_trees; h.num_nodes = (int32_t)N; h.num_tiles = (int32_t)tiles; h.num_sites_tables = num_sites_tables;
   h.trees = slab.at<TreeDev>(dbase, b_trees); h.sites = slab.at<SitesDev>(dbase, b_sites);
-  h.tile_tree = slab.at<int32_t>(dbase, b_tile_tree); h.ctile_tree = slab.at<int32_t>(dbase, b_ctile_tree);
+  h.tile_tree = slab.at<int32_t>(dbase, b_tile_tree);
   h.num_ctiles = (int32_t)ctiles; h.pad0 = 0; h.ctiles = slab.at<CTileDesc>(dbase, b_ctiles);
-  h.fast_ctiles = slab.at<int32_t>(dbase, b_fastl); h.slow_ctiles = slab.at<int32_t>(dbase, b_slowl);
   h.node_id = slab.at<int32_t>(dbase, b_node_id); h.parent_pos = slab.at<int32_t>(dbase, b_parent);
   h.depth = slab.at<int32_t>(dbase, b_depth); h.subtree_size = slab.at<int32_t>(dbase, b_size);
   h.post_node = slab.at<int32_t>(dbase, b_post); h.pos_of_node = slab.at<int32_t>(dbase, b_pos);
@@ -831,8 +821,7 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   fo->d_tree_out = slab.at<double>(dbase, b_tout); fo->d_tree_iout = slab.at<int32_t>(dbase, b_tiout);
   fo->d_tile_agg = slab.at<double>(dbase, b_tagg); fo->d_tile_iagg = slab.at<int32_t>(dbase, b_tiagg);
   fo->d_tile_part = slab.at<double>(dbase, b_tpart); fo->d_tile_ipart = slab.at<int32_t>(dbase, b_tipart);
-  fo->d_tile_flag = slab.at<uint32_t>(dbase, b_tflag); fo->d_tree_done = slab.at<uint32_t>(dbase, b_tdone);
-  fo->d_ticket = slab.at<uint32_t>(dbase, b_ticket);
+  fo->d_tile_flag = slab.at<uint32_t>(dbase, b_tflag);
   fo->d_ctile_order = slab.at<int32_t>(dbase, b_corder);
   fo->d_strad_list = slab.at<int32_t>(dbase, b_strad); fo->d_sd_delta = slab.at<double>(dbase, b_sdd); fo->d_sd_n = slab.at<int32_t>(dbase, b_sdn);
 
@@ -841,10 +830,9 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
   P.trees = h.trees; P.sites = h.sites; P.tile_tree = h.tile_tree; P.raw = tmp.at<RawTreeDev>(tbase, r_raw);
   P.arcs[0] = work.at<int4>(wbase, w_arcs); P.arcs[1] = P.arcs[0] + 2 * N;
   P.scan_tiles = work.at<int32_t>(wbase, w_scan);
-  P.status = work.at<uint32_t>(wbase, w_status); P.max_depth = reinterpret_cast<int32_t*>(P.status + 4);
+  P.status = work.at<uint32_t>(wbase, w_status); P.max_depth = reinterpret_cast<int32_t*>(P.status + 2);
   P.strad_list = fo->d_strad_list;
-  P.ctiles = const_cast<CTileDesc*>(h.ctiles); P.fast_ctiles = const_cast<int32_t*>(h.fast_ctiles);
-  P.slow_ctiles = const_cast<int32_t*>(h.slow_ctiles); P.num_ctiles = (int32_t)ctiles;
+  P.ctiles = const_cast<CTileDesc*>(h.ctiles); P.num_ctiles = (int32_t)ctiles;
   P.num_nodes = (int32_t)N; P.total_muts = (int32_t)M; P.total_ivls = (int32_t)I; P.total_fs = (int32_t)F;
   P.node_id = const_cast<int32_t*>(h.node_id); P.parent_pos = const_cast<int32_t*>(h.parent_pos);
   P.depth = const_cast<int32_t*>(h.depth); P.subtree_size = const_cast<int32_t*>(h.subtree_size);
@@ -890,14 +878,14 @@ static int forest_upload_impl(dphy_ctx* ctx, int32_t num_trees, const dphy_emat_
     st = launch_flatten(ctx, P, (int)tiles, max_tree_nodes);
   }
   if (st != DPHY_OK) return st;
-  std::vector<int32_t> status(4 + num_trees, 0);
+  std::vector<int32_t> status(2 + num_trees, 0);
   ce = cudaMemcpyAsync(status.data(), P.status, sizeof(int32_t) * status.size(), cudaMemcpyDeviceToHost, ctx->stream);
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
   if (ce != cudaSuccess) return check_cuda(ctx, ce, "forest flatten");
   st = flatten_status_to_error(ctx, (uint32_t)status[0]);
   if (st != DPHY_OK) return st;
-  for (int k = 0; k < num_trees; ++k) fo->tree_max_depth[k] = status[4 + k];
-  fo->num_strad = status[1]; fo->num_fast_ctiles = status[2]; fo->num_slow_ctiles = status[3];
+  for (int k = 0; k < num_trees; ++k) fo->tree_max_depth[k] = status[2 + k];
+  fo->num_strad = status[1];
   wblk.reset();
   fo->bytes += tmp.total;
   fo->raw.assign(h_raw, h_raw + num_trees);          // device pointers of every tree's host-order arrays

@@ -16,7 +16,6 @@ __device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t* p) {
   return v;
 }
 __device__ __forceinline__ double ld_cg_f64(const double* p) { return __ldcg(p); }
-__device__ __forceinline__ int32_t ld_cg_i32(const int32_t* p) { return __ldcg(p); }
 
 // Deterministic butterfly reductions (fixed association => bit-reproducible run to run).
 __device__ __forceinline__ double warp_sum(double v) {

@@ -52,7 +52,6 @@ struct SitesDev {
   double mu[kMaxPartitions];
   double pi[kMaxPartitions * 4];
   double q[kMaxPartitions * 16];     // q_ab
-  double log_pi[kMaxPartitions * 4]; // log(pi) (or 0 where pi == 0; see pi)
   int32_t nu_uniform;        // 1 if every nu_l == nu_const (no site-rate heterogeneity): munu needs no gather
   int32_t pad;
   double nu_const;
@@ -64,14 +63,11 @@ struct SitesDev {
   double tab_logq[kMaxPartitions * 16]; // log(q_xy), 0 on the diagonal: log(mu nu_l q_xy) = munu2[l].y + tab_logq[code]
 };
 
-// Per log-G tile descriptor: everything the streaming kernel needs to issue its bulk copies without touching memory first.
+// Per log-G tile descriptor; the tile kernels load it in 16-byte pieces.
 struct alignas(16) CTileDesc {
   int32_t tile_start, n_act, node_base, sites_id;   // written by the host at upload
-  int32_t m0, m1, i0, i1;                           // event ranges of the tile (CSR offsets at its first / past-last node)
-  int32_t f0, f1, cl0, cl1;                         // cl*: the tile's slice of the tree's post-order list (closers)
-  int32_t stage_bytes, pad0, pad1, pad2;            // upper bound of the bytes staged in shared memory for this tile
+  int32_t cl0, cl1, pad0, pad1;                     // cl*: the tile's slice of the tree's post-order list (closers)
 };
-constexpr int kStageBytes = 36 * 1024;              // shared-memory stage of the streaming log-G kernel
 
 // Per-tree record.
 struct TreeDev {
@@ -99,10 +95,7 @@ struct ForestDev {
   const TreeDev* trees;
   const SitesDev* sites;
   const int32_t* tile_tree;     // [num_tiles]
-  const int32_t* ctile_tree;    // [num_ctiles]
   const CTileDesc* ctiles;      // [num_ctiles]
-  const int32_t* fast_ctiles;   // tiles whose staged bytes fit kStageBytes (streaming kernel) ...
-  const int32_t* slow_ctiles;   // ... and the others (direct-from-global kernel)
   // per device position
   const int32_t* node_id;       // host node index (within its tree)
   const int32_t* parent_pos;    // device position of the parent (-1 for a root)
@@ -162,8 +155,8 @@ struct FlattenParams {
   const TreeDev* trees; const SitesDev* sites; const int32_t* tile_tree; const RawTreeDev* raw;
   int4* arcs[2];               // ping-pong Euler-tour arcs: (succ, #enter arcs to the end, #arcs to the end, -)
   int32_t* scan_tiles;         // [ceil(num_nodes / 1024) * 3]
-  uint32_t* status;            // [0] error bits, [1] number of straddlers, [2] fast tiles, [3] slow tiles
-  CTileDesc* ctiles; int32_t* fast_ctiles; int32_t* slow_ctiles; int32_t num_ctiles;
+  uint32_t* status;            // [0] error bits, [1] number of straddlers, then max_depth
+  CTileDesc* ctiles; int32_t num_ctiles;
   int32_t* strad_list;         // (device position, sites table) of the nodes whose subtree closes in a later log-G tile than it opens
   int32_t* max_depth;          // [num_trees]
   int32_t num_nodes, total_muts, total_ivls, total_fs;
@@ -189,7 +182,6 @@ struct PlaceIndex {
   int32_t* site_off = nullptr;             // [L + 1] first record of every site
   int4* rec = nullptr;                     // [M] per mutation, by site: (first region below it, end of those regions, from << 2 | to, dref)
   int2* seg = nullptr;                     // [2 P2] (min, count) segment tree over Hr, leaves at P2 + region
-  size_t bytes = 0;                        // resident bytes
   std::vector<int32_t> h_site_off;         // host copy of site_off (scratch bounds per sample)
   // dated part (dphy_forest_place_dated_samples): a merge-sort tree over region index, keyed by the regions' t_min.  Built by the
   // first dated call that drops a region; it depends on the node and mutation times, so it is rebuilt (in the same block) once
@@ -199,7 +191,6 @@ struct PlaceIndex {
   int32_t* lc = nullptr;                   // [lg][P2] level s, entry i of node [a, a + 2^s): how many of its first i - a + 1 entries
                                            // (in t_min order) come from its left child
   int2* pre = nullptr;                     // [lg][P2] level s, entry i: (min Hr, count) over the node's first i - a + 1 entries
-  size_t dated_bytes = 0;                  // resident bytes of the dated part
   uint64_t dated_at = ~0ull;               // times version the dated part was built at (~0: not valid)
   uint64_t max_at = ~0ull;                 // times version max_key was computed at (~0: not known)
   double max_key = 0.0;                    // the largest t_min: a t_X above it drops no region
@@ -218,7 +209,6 @@ struct dphy_ctx {
   dphy::Arena arena;
   std::string last_error;
   int64_t launches = 0;
-  int sm_count = 148;
   void* pinned = nullptr;       // pinned staging buffer for host->device uploads
   size_t pinned_bytes = 0;
   cudaEvent_t pinned_ev = nullptr;   // recorded after the last async copy out of `pinned`
@@ -253,7 +243,6 @@ struct dphy_ctx {
   cudaEvent_t ev_tally[kTallyStreams] = {};
   struct DeferredCopy { void* dst; const void* src; size_t bytes; };
   std::vector<DeferredCopy> deferred_d2h;   // device->host copies of a batched getter, issued once all its kernels are enqueued
-  bool logg_attr_set = false;   // opt-in dynamic shared memory of the log-G tile kernel
   int logg_path = 0;            // DPHY_LOG_G_PATH_*: 0 auto (folded fast path when every site table has uniform nu), 1 general
 };
 
@@ -271,12 +260,11 @@ struct dphy_sites {
 
 struct dphy_forest {
   dphy::ForestDev h{};          // host mirror (device pointers)
-  dphy::ForestDev* d_self = nullptr;
   std::vector<dphy::TreeDev> trees;
   std::vector<dphy_sites*> sites;
   std::vector<void*> allocs;    // every cudaMalloc'ed block, freed on destroy
   size_t bytes = 0;
-  int64_t total_muts = 0, total_ivls = 0, total_fs = 0, total_nonroot_muts = 0;
+  int64_t total_muts = 0, total_ivls = 0, total_fs = 0;
   std::vector<int64_t> tree_muts;     // mutations per tree (incl. the root's list)
   std::vector<int64_t> tree_fs;       // from-state overrides per tree
   std::vector<int32_t> tree_max_depth;
@@ -292,7 +280,6 @@ struct dphy_forest {
   int32_t* d_tree_iout = nullptr; // [num_trees * 20]: num_muts, pad, num_muts_ab[16], ...
   // straddlers (log-G): nodes whose subtree crosses a log-G tile boundary; their deltas are precomputed per evaluation
   int32_t* d_strad_list = nullptr; int32_t num_strad = 0;
-  int32_t num_fast_ctiles = 0, num_slow_ctiles = 0;
   double* d_sd_delta = nullptr; int32_t* d_sd_n = nullptr;
   // look-back workspace
   double* d_tile_agg = nullptr;     // [num_tiles]
@@ -300,8 +287,6 @@ struct dphy_forest {
   uint32_t* d_tile_flag = nullptr;  // [num_tiles]
   double* d_tile_part = nullptr;    // [num_tiles * 2] per-tile partial sums (log G, T)
   int32_t* d_tile_ipart = nullptr;  // [num_tiles * 17]
-  uint32_t* d_tree_done = nullptr;  // [num_trees] tiles finished (for last-tile reduction)
-  uint32_t* d_ticket = nullptr;     // [1] dynamic tile ticket
   const int32_t* d_ctile_order = nullptr;   // [num_ctiles] launch order of the general log-G tile kernel (full tiles first)
   // study-independent tables of the event-scan SPR path (kernels_spr_group2.cuh), built by the first grouped batch on this forest
   int32_t* d_spr_eopen = nullptr; int32_t* d_spr_tnode = nullptr; int32_t* d_spr_ev = nullptr;

@@ -420,25 +420,15 @@ __global__ void __launch_bounds__(kTile) counts_scan_apply_kernel(FlattenParams 
   }
 }
 
-// ---- (4) log-G tile descriptors: event ranges, closer slice, staging size; fast / slow classification ---------------------------
+// ---- (4) log-G tile descriptors: the tile's slice of the tree's post-order list ----------------------------------------------
 __global__ void __launch_bounds__(256) flatten_ctiles_kernel(FlattenParams P) {
   const int j = blockIdx.x * 256 + threadIdx.x;
   if (j >= P.num_ctiles) return;
-  CTileDesc d = P.ctiles[j];
+  CTileDesc& d = P.ctiles[j];
   const int p0 = d.tile_start, p1 = d.tile_start + d.n_act;
-  d.m0 = P.mut_off[p0]; d.m1 = P.mut_off[p1];
-  d.i0 = P.miss_off[p0]; d.i1 = P.miss_off[p1];
-  d.f0 = P.fs_off[p0]; d.f1 = P.fs_off[p1];
   const int q_first = p0 - d.node_base, q_last = p1 - 1 - d.node_base;
   d.cl0 = q_first == 0 ? 0 : (q_first - 1) - P.depth[p0 - 1];
   d.cl1 = q_last - P.depth[p1 - 1];
-  const int n = d.n_act, nm = d.m1 - d.m0, ni = d.i1 - d.i0, nf = d.f1 - d.f0, nc = d.cl1 - d.cl0;
-  // every staged array may be over-fetched by < 32 bytes (16-byte alignment of both ends)
-  d.stage_bytes = (4 * n + 32) * 2 + (8 * n + 32) + (4 * (n + 1) + 32) * 2 + (2 * P.fsw_stride * n + 32) + (nm + 32) + (8 * nm + 32) +
-                  (8 * ni + 32) + (4 * nc + 32);
-  P.ctiles[j] = d;
-  if (d.stage_bytes <= kStageBytes && nm >= 0 && ni >= 0 && nf >= 0 && nc >= 0) P.fast_ctiles[atomicAdd(P.status + 2, 1u)] = j;
-  else P.slow_ctiles[atomicAdd(P.status + 3, 1u)] = j;
 }
 
 // Accepted displace moves (core/subrun.cpp:223-231,276-284): scatter new node times by host node index.

@@ -133,23 +133,120 @@ __global__ void __launch_bounds__(128) emat_log_G_straddler_kernel(const LogGPar
 // kLgTile consecutive device positions of one tree per tile; thread tid owns the two consecutive positions 2 tid and
 // 2 tid + 1.  emat_log_G_tile_kernel: one CTA per tile straight from global memory, thread-per-node list walks with batched,
 // predicated loads; any site-rate model.
-struct NodeRegs {
-  int par[2], dep[2], om[3];
-  double tN[2], tP[2];
-  double dm[2], es[2], dmi[2];
-  int nmiss[2];
-};
+constexpr int kIvlBatch = 4;   // missation intervals in flight per node per round
+constexpr int kMutBatch = 2;   // mutations in flight per node per round
 
-template <bool kPostInSmem>
-__device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm, const NodeRegs& R, int tile, int tile_start, int n_act,
-                                               int node_base, int cl0, int cl1, const int32_t* post /* post[j], j in [cl0, cl1) */,
-                                               double lambda_ref) {
+// 4 resident CTAs per SM: 64 registers, no spills (5 or 6 CTAs: 48 / 40 registers, 80 / 160 bytes of spill stores)
+__global__ void __launch_bounds__(kLgThreads, 4) emat_log_G_tile_kernel(const LogGParams P, const int32_t* __restrict__ tile_list) {
+  __shared__ LogGSmem sm;
+  const ForestDev& f = P.f;
   const int tid = threadIdx.x;
-  const int q0 = 2 * tid;
+  const int tile = tile_list[blockIdx.x];
+  const int4 ct = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile));
+  const int4 cl = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile) + 1);
+  const int tile_start = ct.x, n_act = ct.y, node_base = ct.z, cl0 = cl.x, cl1 = cl.y;
+  const SitesDev& S = f.sites[ct.w];
+  const bool uni = S.nu_uniform != 0;
+  const double* __restrict__ cumQ = S.cumQ;
+  if (tid < 64) sm.ab[tid] = 0;
+
+  // ---- node records ----------------------------------------------------------------------------------------------------------------
+  const int q0 = 2 * tid, p0 = tile_start + q0;
   const bool act0 = q0 < n_act, act1 = q0 + 1 < n_act;
+  int par[2], dep[2], nmiss[2], om[3] = {0, 0, 0}, oi[3] = {0, 0, 0}, of[3] = {0, 0, 0};
+  double tN[2], tP[2], dm[2], es[2], dmi[2];
+#pragma unroll
+  for (int k = 0; k < 2; ++k) { par[k] = -1; dep[k] = 0; tN[k] = 0.0; tP[k] = 0.0; dm[k] = 0.0; es[k] = 0.0; dmi[k] = 0.0; nmiss[k] = 0; }
+  if (act0) {
+    par[0] = f.parent_pos[p0]; dep[0] = f.depth[p0]; tN[0] = f.t[p0];
+    om[0] = f.mut_off[p0]; oi[0] = f.miss_off[p0]; of[0] = f.fs_off[p0];
+    om[1] = f.mut_off[p0 + 1]; oi[1] = f.miss_off[p0 + 1]; of[1] = f.fs_off[p0 + 1];
+    om[2] = om[1]; oi[2] = oi[1]; of[2] = of[1];
+  }
+  if (act1) {
+    par[1] = f.parent_pos[p0 + 1]; dep[1] = f.depth[p0 + 1]; tN[1] = f.t[p0 + 1];
+    om[2] = f.mut_off[p0 + 2]; oi[2] = f.miss_off[p0 + 2]; of[2] = f.fs_off[p0 + 2];
+  }
+#pragma unroll
+  for (int k = 0; k < 2; ++k) if (par[k] >= 0) tP[k] = f.t[par[k]];
+
+  // ---- per-node sums over the branch lists (list order => deterministic) -----------------------------------------------------------
+  // missation intervals: -(cumQ[end] - cumQ[start]); count of sites going missing
+  {
+    const int c0 = oi[1] - oi[0], c1 = oi[2] - oi[1];
+    const int cmax = max(c0, c1);
+    for (int j = 0; j < cmax; j += kIvlBatch) {
+      int2 se[2][kIvlBatch];
+#pragma unroll
+      for (int u = 0; u < kIvlBatch; ++u) {
+        se[0][u] = j + u < c0 ? __ldg(f.miss_se + oi[0] + j + u) : make_int2(0, 0);
+        se[1][u] = j + u < c1 ? __ldg(f.miss_se + oi[1] + j + u) : make_int2(0, 0);
+      }
+#pragma unroll
+      for (int u = 0; u < kIvlBatch; ++u) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+          // (0,0) for an absent interval: cumQ[0] - cumQ[0] == 0 exactly, so the arithmetic stays branch-free
+          dmi[k] -= __ldg(cumQ + se[k][u].y) - __ldg(cumQ + se[k][u].x);
+          nmiss[k] += se[k][u].y - se[k][u].x;
+        }
+      }
+    }
+  }
+  // mutations: d_i = mu nu (q_to - q_from);  e_i = d_i * t_i + log(mu nu q_from,to)   [g_node = sum e_i - t_P * sum d_i]
+  {
+    const int c0 = om[1] - om[0], c1 = om[2] - om[1];
+    const int cmax = max(c0, c1);
+    for (int j = 0; j < cmax; j += kMutBatch) {
+#pragma unroll
+      for (int u = 0; u < kMutBatch; ++u) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+          if (j + u < (k == 0 ? c0 : c1)) {
+            const int i = om[k] + j + u;
+            const int code = __ldg(f.mut_code + i) & 63;
+            const double tm = __ldg(f.mut_t + i);
+            double dd, lg;
+            if (uni) { dd = __ldg(S.tab_md + code); lg = __ldg(S.tab_lq + code); }
+            else {
+              // log(mu nu_l q_xy) = log(mu nu_l) [per site, tabulated with mu nu_l] + log(q_xy) [64-entry table]: one 16-byte gather
+              // instead of an fp64 log per mutation (a third of this kernel's instructions with site-rate heterogeneity on)
+              const double2 mn = __ldg(S.munu2 + __ldg(f.mut_site + i));
+              dd = mn.x * __ldg(S.tab_dq + code);
+              lg = ((code >> 2) & 3) != (code & 3) ? mn.y + __ldg(S.tab_logq + code) : 0.0;
+            }
+            dm[k] += dd;
+            if (par[k] >= 0) {     // the root's list ("mutations" above the root) is not part of log G nor of the counts
+              es[k] += dd * tm + lg;
+              atomicAdd(&sm.ab[(tid & 3) * 16 + (code & 15)], 1);
+            }
+          }
+        }
+      }
+    }
+  }
+  // from-state overrides of missing sites: folded per-branch state counts when the site rates are uniform, lists otherwise
+  if (uni) {
+    for (int k2 = 0; k2 < f.fsw_stride; ++k2) {
+      const double mq = __ldg(S.tab_muq + k2);
+      if (act0) dmi[0] += mq * (double)__ldg(f.fsw + (size_t)p0 * f.fsw_stride + k2);
+      if (act1) dmi[1] += mq * (double)__ldg(f.fsw + (size_t)(p0 + 1) * f.fsw_stride + k2);
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      for (int i = of[k]; i < of[k + 1]; ++i) {
+        const int code = __ldg(f.fs_code + i) & 63;
+        dmi[k] -= __ldg(S.munu + __ldg(f.fs_site + i)) * __ldg(S.tab_dq + code);
+      }
+    }
+  }
+
+  const double lambda_ref = __ldg(cumQ + S.L);
+  const int32_t* post = f.post_node + node_base;   // post[j], j in [cl0, cl1)
   const int q_first = tile_start - node_base;
-  const double d0 = act0 ? R.dm[0] + R.dmi[0] : 0.0, d1 = act1 ? R.dm[1] + R.dmi[1] : 0.0;
-  const int n0 = act0 ? R.nmiss[0] : 0, n1 = act1 ? R.nmiss[1] : 0;
+  const double d0 = act0 ? dm[0] + dmi[0] : 0.0, d1 = act1 ? dm[1] + dmi[1] : 0.0;
+  const int n0 = act0 ? nmiss[0] : 0, n1 = act1 ? nmiss[1] : 0;
   sm.dl[q0] = d0; sm.dl[q0 + 1] = d1;
   sm.dn[q0] = n0; sm.dn[q0 + 1] = n1;
 
@@ -166,7 +263,7 @@ __device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm
   double CL[2] = {0.0, 0.0};
   int CLn[2] = {0, 0};
   {
-    const int myc0 = act0 ? (q_first + q0) - R.dep[0] : cl0, myc1 = act1 ? (q_first + q0 + 1) - R.dep[1] : cl0;
+    const int myc0 = act0 ? (q_first + q0) - dep[0] : cl0, myc1 = act1 ? (q_first + q0 + 1) - dep[1] : cl0;
     double carry = 0.0; int icarry = 0;
     for (int c0 = cl0; c0 < cl1; c0 += kLgTile) {
       double a[2] = {0.0, 0.0}; int n[2] = {0, 0};
@@ -174,7 +271,7 @@ __device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm
       for (int u = 0; u < 2; ++u) {
         const int j = c0 + 2 * tid + u;
         if (j < cl1) {
-          const int p = kPostInSmem ? post[j] : __ldg(post + j);
+          const int p = __ldg(post + j);
           const int qa = p - tile_start;
           if (qa >= 0) { a[u] = sm.dl[qa]; n[u] = sm.dn[qa]; }
           else { a[u] = __ldg(P.sd_delta + p); n[u] = __ldg(P.sd_n + p); }     // straddler: opened in an earlier tile
@@ -206,11 +303,11 @@ __device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm
       P.lambda_out[p] = lam_local;
       P.nsmn_out[p] = iloc;
       if (q == n_act - 1) { P.tile_agg[tile] = loc; P.tile_iagg[tile] = iloc; }
-      if (R.par[k] >= 0) {
-        const double len = R.tN[k] - R.tP[k];
-        contrib += -lam_local * len + (R.es[k] - R.tP[k] * R.dm[k]);
+      if (par[k] >= 0) {
+        const double len = tN[k] - tP[k];
+        contrib += -lam_local * len + (es[k] - tP[k] * dm[k]);
         tcontrib += len;
-        nmut += R.om[k + 1] - R.om[k];
+        nmut += om[k + 1] - om[k];
       }
     }
   }
@@ -233,120 +330,6 @@ __device__ __forceinline__ void tile_back_half(const LogGParams& P, LogGSmem& sm
     }
   }
   if (tid < 16) P.tile_ipart[tile * 17 + 1 + tid] = sm.ab[tid] + sm.ab[16 + tid] + sm.ab[32 + tid] + sm.ab[48 + tid];
-}
-
-// ---- pass 1, direct-from-global variant -------------------------------------------------------------------------------------------
-constexpr int kIvlBatch = 4;   // missation intervals in flight per node per round
-constexpr int kMutBatch = 2;   // mutations in flight per node per round
-
-// 4 resident CTAs per SM: 64 registers, no spills (5 or 6 CTAs: 48 / 40 registers, 80 / 160 bytes of spill stores)
-__global__ void __launch_bounds__(kLgThreads, 4) emat_log_G_tile_kernel(const LogGParams P, const int32_t* __restrict__ tile_list) {
-  __shared__ LogGSmem sm;
-  const ForestDev& f = P.f;
-  const int tid = threadIdx.x;
-  const int tile = tile_list[blockIdx.x];
-  const int4 ct = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile));
-  const int4 cl = __ldg(reinterpret_cast<const int4*>(f.ctiles + tile) + 2);
-  const int tile_start = ct.x, n_act = ct.y, node_base = ct.z;
-  const SitesDev& S = f.sites[ct.w];
-  const bool uni = S.nu_uniform != 0;
-  const double* __restrict__ cumQ = S.cumQ;
-  if (tid < 64) sm.ab[tid] = 0;
-
-  // ---- node records ----------------------------------------------------------------------------------------------------------------
-  NodeRegs R;
-  const int q0 = 2 * tid, p0 = tile_start + q0;
-  const bool act0 = q0 < n_act, act1 = q0 + 1 < n_act;
-  int oi[3] = {0, 0, 0}, of[3] = {0, 0, 0};
-#pragma unroll
-  for (int k = 0; k < 2; ++k) { R.par[k] = -1; R.dep[k] = 0; R.tN[k] = 0.0; R.tP[k] = 0.0; R.dm[k] = 0.0; R.es[k] = 0.0; R.dmi[k] = 0.0; R.nmiss[k] = 0; }
-  R.om[0] = R.om[1] = R.om[2] = 0;
-  if (act0) {
-    R.par[0] = f.parent_pos[p0]; R.dep[0] = f.depth[p0]; R.tN[0] = f.t[p0];
-    R.om[0] = f.mut_off[p0]; oi[0] = f.miss_off[p0]; of[0] = f.fs_off[p0];
-    R.om[1] = f.mut_off[p0 + 1]; oi[1] = f.miss_off[p0 + 1]; of[1] = f.fs_off[p0 + 1];
-    R.om[2] = R.om[1]; oi[2] = oi[1]; of[2] = of[1];
-  }
-  if (act1) {
-    R.par[1] = f.parent_pos[p0 + 1]; R.dep[1] = f.depth[p0 + 1]; R.tN[1] = f.t[p0 + 1];
-    R.om[2] = f.mut_off[p0 + 2]; oi[2] = f.miss_off[p0 + 2]; of[2] = f.fs_off[p0 + 2];
-  }
-#pragma unroll
-  for (int k = 0; k < 2; ++k) if (R.par[k] >= 0) R.tP[k] = f.t[R.par[k]];
-
-  // ---- per-node sums over the branch lists (list order => deterministic) -----------------------------------------------------------
-  // missation intervals: -(cumQ[end] - cumQ[start]); count of sites going missing
-  {
-    const int c0 = oi[1] - oi[0], c1 = oi[2] - oi[1];
-    const int cmax = max(c0, c1);
-    for (int j = 0; j < cmax; j += kIvlBatch) {
-      int2 se[2][kIvlBatch];
-#pragma unroll
-      for (int u = 0; u < kIvlBatch; ++u) {
-        se[0][u] = j + u < c0 ? __ldg(f.miss_se + oi[0] + j + u) : make_int2(0, 0);
-        se[1][u] = j + u < c1 ? __ldg(f.miss_se + oi[1] + j + u) : make_int2(0, 0);
-      }
-#pragma unroll
-      for (int u = 0; u < kIvlBatch; ++u) {
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-          // (0,0) for an absent interval: cumQ[0] - cumQ[0] == 0 exactly, so the arithmetic stays branch-free
-          R.dmi[k] -= __ldg(cumQ + se[k][u].y) - __ldg(cumQ + se[k][u].x);
-          R.nmiss[k] += se[k][u].y - se[k][u].x;
-        }
-      }
-    }
-  }
-  // mutations: d_i = mu nu (q_to - q_from);  e_i = d_i * t_i + log(mu nu q_from,to)   [g_node = sum e_i - t_P * sum d_i]
-  {
-    const int c0 = R.om[1] - R.om[0], c1 = R.om[2] - R.om[1];
-    const int cmax = max(c0, c1);
-    for (int j = 0; j < cmax; j += kMutBatch) {
-#pragma unroll
-      for (int u = 0; u < kMutBatch; ++u) {
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-          if (j + u < (k == 0 ? c0 : c1)) {
-            const int i = R.om[k] + j + u;
-            const int code = __ldg(f.mut_code + i) & 63;
-            const double tm = __ldg(f.mut_t + i);
-            double dd, lg;
-            if (uni) { dd = __ldg(S.tab_md + code); lg = __ldg(S.tab_lq + code); }
-            else {
-              // log(mu nu_l q_xy) = log(mu nu_l) [per site, tabulated with mu nu_l] + log(q_xy) [64-entry table]: one 16-byte gather
-              // instead of an fp64 log per mutation (a third of this kernel's instructions with site-rate heterogeneity on)
-              const double2 mn = __ldg(S.munu2 + __ldg(f.mut_site + i));
-              dd = mn.x * __ldg(S.tab_dq + code);
-              lg = ((code >> 2) & 3) != (code & 3) ? mn.y + __ldg(S.tab_logq + code) : 0.0;
-            }
-            R.dm[k] += dd;
-            if (R.par[k] >= 0) {     // the root's list ("mutations" above the root) is not part of log G nor of the counts
-              R.es[k] += dd * tm + lg;
-              atomicAdd(&sm.ab[(tid & 3) * 16 + (code & 15)], 1);
-            }
-          }
-        }
-      }
-    }
-  }
-  // from-state overrides of missing sites: folded per-branch state counts when the site rates are uniform, lists otherwise
-  if (uni) {
-    for (int k2 = 0; k2 < f.fsw_stride; ++k2) {
-      const double mq = __ldg(S.tab_muq + k2);
-      if (act0) R.dmi[0] += mq * (double)__ldg(f.fsw + (size_t)p0 * f.fsw_stride + k2);
-      if (act1) R.dmi[1] += mq * (double)__ldg(f.fsw + (size_t)(p0 + 1) * f.fsw_stride + k2);
-    }
-  } else {
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      for (int i = of[k]; i < of[k + 1]; ++i) {
-        const int code = __ldg(f.fs_code + i) & 63;
-        R.dmi[k] -= __ldg(S.munu + __ldg(f.fs_site + i)) * __ldg(S.tab_dq + code);
-      }
-    }
-  }
-  tile_back_half<false>(P, sm, R, tile, tile_start, n_act, node_base, cl.z, cl.w,
-                        f.post_node + node_base, __ldg(cumQ + S.L));
 }
 
 // ---- pass 2: one CTA per tree -- exclusive scan of the tile aggregates (tile order), log G fold, tallies, root prior -----

@@ -554,7 +554,7 @@ int ensure_place_index(dphy_ctx* ctx, dphy_forest* fo, int tree) {
   fo->allocs.push_back(d.release());
   fo->bytes += res.total;
   X.R = (int32_t)R; X.P2 = (int32_t)P2; X.L = L;
-  X.site_off = so; X.rec = rec; X.seg = seg; X.bytes = res.total;
+  X.site_off = so; X.rec = rec; X.seg = seg;
   X.h_site_off = std::move(h_so);
   return DPHY_OK;
 }
@@ -615,7 +615,7 @@ int ensure_dated_index(dphy_ctx* ctx, dphy_forest* fo, int tree, uint64_t ver) {
     fo->allocs.push_back(d.release());
     fo->bytes += res.total;
     void* base = fo->allocs.back();
-    X.tkey = res.at<double>(base, b_tkey); X.lc = res.at<int32_t>(base, b_lc); X.pre = res.at<int2>(base, b_pre); X.dated_bytes = res.total; X.lg = lg;
+    X.tkey = res.at<double>(base, b_tkey); X.lc = res.at<int32_t>(base, b_lc); X.pre = res.at<int2>(base, b_pre); X.lg = lg;
   }
   X.dated_at = ~0ull;                       // not valid until the build below has finished
   double* key = work.at<double>(tmp.p, b_key); int32_t* idx = work.at<int32_t>(tmp.p, b_idx);

@@ -72,7 +72,7 @@ struct SprStudy {
   int32_t h_stride, tile_shift, num_htiles, weights_fused;
   // event-scan grouped path (kernels_spr_group2.cuh): lane of the study inside its group and the group's tables (0 => not used)
   int32_t g2, g2_lane, g2_mut_base, g2_num_templates;
-  int64_t off_g2S, off_g2aggS, off_g2mask, off_g2aggK, off_g2cbase, off_hang, off_hmix;
+  int64_t off_g2S, off_g2aggS, off_g2mask, off_g2aggK, off_hang, off_hmix;
   int32_t hmix_cap, pad3;
 };
 
@@ -1416,7 +1416,7 @@ struct dphy_spr_batch {
   int32_t num = 0;
   std::vector<SprStudy> host;     // filled by get_summaries
   bool fetched = false;
-  SprGroupDev* d_groups = nullptr; int32_t num_groups = 0;
+  SprGroupDev* d_groups = nullptr;
   bool weighted = false;          // spr_weights_kernel + spr_normalize_kernel have run for the current (lambda_X, f, t_max_tip)
   int status = DPHY_OK;           // sticky: the first per-study error found by spr_fetch, returned by every accessor
   std::string status_msg;
@@ -1583,7 +1583,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     if (grouped) {
       const SprGroupDev& G = groups[group_of[i]];
       S.g2 = 1; S.g2_lane = lane_of[i]; S.g2_mut_base = G.mut_base; S.g2_num_templates = G.num_templates;
-      S.off_g2S = G.off_S; S.off_g2aggS = G.off_aggS; S.off_g2mask = G.off_mask; S.off_g2aggK = G.off_aggK; S.off_g2cbase = G.off_cbase;
+      S.off_g2S = G.off_S; S.off_g2aggS = G.off_aggS; S.off_g2mask = G.off_mask; S.off_g2aggK = G.off_aggK;
     }
     S.weights_fused = (grouped && r.lambda_X > 0.0) ? 1 : 0;
     max_tiles = std::max(max_tiles, S.num_htiles);
@@ -1690,7 +1690,7 @@ int dphy_spr_study_batch(dphy_ctx* ctx, dphy_forest* fo, int32_t n, const dphy_s
     if (st != DPHY_OK) return st;
     b->dev.g2_eopen = fo->d_spr_eopen; b->dev.g2_tnode = fo->d_spr_tnode; b->dev.g2_ev = fo->d_spr_ev;
   }
-  b->d_groups = hdr.at<SprGroupDev>(d, b_groups); b->num_groups = (int32_t)groups.size();
+  b->d_groups = hdr.at<SprGroupDev>(d, b_groups);
   if (n == 0) { *out = b.release(); return DPHY_OK; }
   // flags + tickets start at zero; studies + X overlays uploaded through the pinned staging buffer
   cudaError_t ce = cudaMemsetAsync(hdr.at<char>(d, b_flag), 0, hdr.blocks[b_groups].off - hdr.blocks[b_flag].off, ctx->stream);
